@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the NAVTEX receive chain (BASELINE.json metric:
 "IQ Msamples/s through FIR cascade + FSK demod at 1-8 B200; % HBM roofline").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one pass of the whole hot path (fused FIR cascade -> demod / bit-sync -> SITOR-B state
@@ -405,6 +405,28 @@ def timed_pushes(c, eng, ptr, n, steps, warmup, s16=False, reset=False):
     return ms, st, msgs, clocks, spans
 
 
+DUMP_Y3_STREAMS = 128       # 18.9 MB of y3: the whole [1024][2][9250] complex64 block would be 152 MB
+
+
+def dump_outputs(eng, out_dir):
+    """What a caller of the timed path receives after its last step, as float32 .npy files, so that two builds can be compared
+    output for output: y3.npy [K][channel][900 Hz sample][re, im] of a fixed, seeded sample of K streams (their indices in
+    y3_streams.npy) and events.npy [stream][channel][byte] of every stream's decoded event bytes, padded with -1."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    pick = np.sort(np.random.default_rng(0).choice(eng.S, size=min(DUMP_Y3_STREAMS, eng.S), replace=False))
+    y3 = np.ascontiguousarray(eng.read_y3()[pick])
+    np.save(os.path.join(out_dir, "y3.npy"), y3.view(np.float32).reshape(*y3.shape, 2))
+    np.save(os.path.join(out_dir, "y3_streams.npy"), pick.astype(np.float32))
+    ev = [[eng.read_events(s, ch) for ch in range(eng.C)] for s in range(eng.S)]
+    out = np.full((eng.S, eng.C, max(1, max(len(e) for row in ev for e in row))), -1.0, dtype=np.float32)
+    for s, row in enumerate(ev):
+        for ch, e in enumerate(row):
+            out[s, ch, :len(e)] = np.frombuffer(e, dtype=np.uint8)
+    np.save(os.path.join(out_dir, "events.npy"), out)
+
+
 def span_stats(spans):
     if len(spans) == 0:
         return {"kernel_ms_min": None, "kernel_ms_median": None, "kernel_ms_max": None}
@@ -751,7 +773,13 @@ def main():
     ap.add_argument("--parity-streams", type=int, default=PARITY_STREAMS,
                     help="streams of the workload compared against the unmodified reference in the same run (check.oracle_parity); up to 1024")
     ap.add_argument("--pinned", default="nvx", choices=["nvx", "wc"], help="e2e host buffer: cudaHostAlloc portable (nvx) or write-combined (wc)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what their last step computed to DIR/*.npy (rank 0's streams; see dump_outputs)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "config2"):
+        ap.error("--dump-outputs applies to the default workload of --impl b200")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -823,6 +851,8 @@ def main():
     # ---- device-resident whole-job throughput ----------------------------------------------------
     eng = engine.Engine(S, BLOCK, device=local, first_stream_id=rank * S)
     max_ms, st, msgs, clocks, spans = timed_pushes(c, eng, x.data_ptr(), BLOCK, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eng, args.dump_outputs)
     # demod stage breakdown from a short extra pass (the per-stage event records would only add bubbles to the timed region)
     eng.enable_timing(2)
     eng.stats()

@@ -13,7 +13,8 @@ $NVCC $FLAGS -c capture_frontend.cpp -o ../build/capture_frontend.o
 $NVCC -shared -o ../libnavtex_b200.so ../build/fir_cascade.o ../build/fir_long.o ../build/fir_long_tc.o ../build/demod.o ../build/engine.o ../build/synth.o \
       ../build/message_assembler.o ../build/capture_frontend.o -arch=sm_100a -lcudart_static -lpthread -ldl -lrt
 g++ -O2 -std=c++17 -fPIC -shared -o ../libnavtex_compat.so navtex_compat.cpp -L.. -lnavtex_b200 -Wl,-rpath,'$ORIGIN'
-# SASS evidence for profiles/ (UTCHMMA / LDTM / STTM / UTMALDG / FFMA2 ... per kernel), regenerated with every build
-sh ../../tools/sass_counts.sh ../libnavtex_b200.so > ../../profiles/sass_r2.txt 2>/dev/null || true
+# SASS evidence (UTCHMMA / LDTM / STTM / UTMALDG / FFMA2 ... per kernel), regenerated with every build next to the objects;
+# profiles/sass_r2.txt is a committed copy and the build leaves it alone
+sh ../../tools/sass_counts.sh ../libnavtex_b200.so > ../build/sass_counts.txt 2>/dev/null || true
 grep -h "registers\|spill" ../build/*.ptxas.log | sort | uniq -c
 ls -la ../libnavtex_b200.so ../libnavtex_compat.so

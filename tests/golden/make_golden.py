@@ -13,6 +13,7 @@ import sys
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+Y3_MAX = 24000      # 900 Hz samples of y3 kept per channel (26.7 s): keeps every fixture under 1 MB
 sys.path.insert(0, os.path.dirname(HERE))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 
@@ -29,7 +30,7 @@ def main():
         out = dict(sha256=cases.digest(iq), n=iq.size // 2, y1_head=r.y1[:4096])
         for tag in oracle_lib.CHANNELS:
             out["y2_head_" + tag] = r.y2[tag][:2048]
-            out["y3_" + tag] = r.y3[tag]
+            out["y3_" + tag] = r.y3[tag][:Y3_MAX]
             out["bits_" + tag] = np.frombuffer(r.bits[tag], dtype=np.uint8)
             out["bitpos_" + tag] = r.bitpos[tag]
             out["disc_" + tag] = r.disc[tag]

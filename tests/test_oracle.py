@@ -29,7 +29,9 @@ def test_oracle_matches_golden_exactly(name):
     assert np.array_equal(r.y1[:4096], g["y1_head"])
     for tag in ol.CHANNELS:
         assert np.array_equal(r.y2[tag][:2048], g["y2_head_" + tag])
-        assert np.array_equal(r.y3[tag], g["y3_" + tag])                      # exact FP64 equality
+        y3 = g["y3_" + tag]                                                  # the first Y3_MAX samples (make_golden.py)
+        assert len(r.y3[tag]) == int(g["n"]) // 280
+        assert np.array_equal(r.y3[tag][:len(y3)], y3)                        # exact FP64 equality
         assert r.bits[tag] == g["bits_" + tag].tobytes()
         assert np.array_equal(r.bitpos[tag], g["bitpos_" + tag])
         assert np.array_equal(r.disc[tag], g["disc_" + tag])                  # float accumulators, bit-exact
