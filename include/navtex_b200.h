@@ -105,6 +105,11 @@ int nvx_engine_reset(nvx_engine *e);
  * nvx_engine_wait_ingest() or nvx_engine_sync() returns.  One engine takes one sample format between resets. */
 int nvx_engine_push_host_f32(nvx_engine *e, const float *iq, long long n);
 int nvx_engine_push_host_s16(nvx_engine *e, const int16_t *iq, long long n);   /* SDRplay / WAV sample format */
+/* RTL-SDR sample format (rtlsdr_read_async / rtl_tcp): unsigned 8-bit offset-binary I,Q bytes, block [S][n][2] stream-major.
+ * Sample value = u - 128 exactly, a float in [-128, 127].  128 rather than the converter's mid-scale 127.5 keeps the values
+ * integers: the same capture pushed as int16 (u - 128) gives bit-identical results.  The -0.5 LSB DC offset this leaves
+ * sits at -+14 kHz after the mix, where the channel filter removes it. */
+int nvx_engine_push_host_u8(nvx_engine *e, const uint8_t *iq, long long n);
 int nvx_engine_wait_ingest(nvx_engine *e);                                      /* every host buffer pushed so far has been read */
 long long nvx_engine_host_pushes(nvx_engine *e);                                /* host pushes made so far (the next one has this index) */
 int nvx_engine_wait_ingest_of(nvx_engine *e, long long push_index);             /* the buffer of that host push (0-based) has been read */
@@ -112,6 +117,7 @@ int nvx_engine_wait_ingest_of(nvx_engine *e, long long push_index);             
  * engine's stream (ordered after everything previously queued on it) */
 int nvx_engine_push_device_f32(nvx_engine *e, const void *d_iq, long long n);
 int nvx_engine_push_device_s16(nvx_engine *e, const void *d_iq, long long n);
+int nvx_engine_push_device_u8(nvx_engine *e, const void *d_iq, long long n);    /* 8-bit I,Q bytes [S][n][2], 16-byte aligned */
 /* wait for everything pushed so far and run the host-side message assembly */
 int nvx_engine_sync(nvx_engine *e);
 
@@ -141,7 +147,7 @@ typedef struct {
     double demod_ms;            /* same for the demod/bit-sync/FSM kernel */
     long long cascade_launches;
     long long demod_launches;
-    long long aux_launches;     /* tail carry, s16 -> f32 conversion */
+    long long aux_launches;     /* tail carry, second pass of five to eight channels, long-tap stages, 8-bit -> int16 widening (long-tap path) */
     long long samples;          /* IQ samples (all streams) pushed */
     double demod_stage_ms[6];   /* split of demod_ms: angle/correlation, per-offset sums + arg max, history carry | symbol clock, bit decisions, SITOR-B state machine */
     long long long_tc_fallbacks;/* long-tap stage launches that were meant for the tensor-core kernel but ran on the CUDA-core one
@@ -181,11 +187,17 @@ int nvx_debug_long_tc_band(int decimation, const double *h, int n_taps, int *geo
 typedef struct nvx_capture nvx_capture;
 /* one ring of ring_samples int16 I,Q pairs per stream (>= 2 max_block); max_block <= the engine's */
 int nvx_capture_create(nvx_engine *e, int n_streams, long long max_block, long long ring_samples, nvx_capture **out);
+/* same for RTL-SDR radios: the rings hold 8-bit I,Q pairs and the pump pushes with nvx_engine_push_host_u8 */
+int nvx_capture_create_u8(nvx_engine *e, int n_streams, long long max_block, long long ring_samples, nvx_capture **out);
 void nvx_capture_destroy(nvx_capture *c);
 /* producer (the radio callback of stream `stream`, capt_sched.c:105: separate xi[] / xq[] arrays); one producer thread per
  * stream.  NVX_ERR_OVERFLOW = the ring was full, the excess was dropped (and counted) instead of overwriting unread data */
 int nvx_capture_write(nvx_capture *c, int stream, const short *xi, const short *xq, unsigned num_samples);
-/* consumer: push what every stream has in common (multiple of 280, <= max_block) as one int16 block.
+/* producer of an 8-bit capture: num_samples interleaved I,Q byte pairs, exactly as the rtlsdr_read_async callback hands them
+ * over (len = 2 num_samples).  Writing int16 to an 8-bit capture or 8-bit pairs to an int16 capture returns NVX_ERR_ARG;
+ * overflow as for nvx_capture_write */
+int nvx_capture_write_u8(nvx_capture *c, int stream, const unsigned char *iq, unsigned num_samples);
+/* consumer: push what every stream has in common (multiple of 280, <= max_block) as one block in the capture's format.
  * Returns samples per stream pushed, 0 if there was less than 280, or a negative nvx_status */
 long long nvx_capture_pump(nvx_capture *c);
 /* or let a poller thread pump every poll_ms (<= 0: 50 ms, capt_sched.c:489); stop() drains what is left */

@@ -7,6 +7,8 @@
 //   consumer  main loop        receiver/capt_sched.c:484-528  (every 50 ms: drain the ring, sample_in_1 per I,Q pair)
 // Here every stream has its own ring of interleaved int16 I,Q; the consumer ("pump") takes what ALL streams have in
 // common, rounded down to a multiple of 280 samples, lays it out stream-major and pushes it as one int16 block.
+// nvx_capture_create_u8 makes the same front end for RTL-SDR radios: rings of interleaved 8-bit I,Q bytes (the buffer
+// rtlsdr_read_async hands its callback), pumped with nvx_engine_push_host_u8.
 //
 // nvx_store mirrors message_store.c:59-97: add = "delete from messages where bbbb = ?; insert (bbbb, message,
 // timestamp, 'NEW', freq)" with the reference's UTC "%Y-%m-%d %H:%M" stamp, keyed additionally by stream; purge drops
@@ -29,8 +31,10 @@ struct nvx_capture {
     int S = 0;
     long long ring = 0;                    // samples per stream
     long long max_block = 0;
+    bool u8 = false;                       // 8-bit I,Q pairs (nvx_capture_create_u8), else int16
+    size_t bps = 4;                        // bytes per I,Q pair in the rings and the staging buffers
     struct Ring {
-        std::vector<int16_t> buf;          // 2 * ring shorts
+        std::vector<uint8_t> buf;          // ring * bps bytes of interleaved I,Q
         long long head = 0, tail = 0;      // absolute sample counts written / consumed
         std::mutex mu;                     // in_mutex of capt_sched.c:109-112
         long long dropped = 0;
@@ -38,7 +42,7 @@ struct nvx_capture {
     std::vector<Ring> rings;
     // [S][n] staging, stream-major: two page-locked buffers (nvx_pinned_alloc), so that the engine's H2D copy of pump k is
     // asynchronous and overlaps the ring drain of pump k + 1
-    int16_t* block[2] = {nullptr, nullptr};
+    uint8_t* block[2] = {nullptr, nullptr};
     long long block_push[2] = {-1, -1};    // index of the engine host push that last read each buffer
     unsigned pumps = 0;
     std::thread poller;
@@ -58,55 +62,56 @@ long long pump_locked(nvx_capture* c) {
     n -= n % NVX_BLOCK_ALIGN;
     if (n <= 0) return 0;
     const unsigned which = c->pumps++ & 1;
-    int16_t* const blk = c->block[which];
+    uint8_t* const blk = c->block[which];
     // the copy that last read this buffer was queued two pumps ago; make sure it is over before the buffer is refilled (the copy
     // of the previous pump, out of the other buffer, keeps running meanwhile)
     if (c->block_push[which] >= 0)
         if (const int rc = nvx_engine_wait_ingest_of(c->eng, c->block_push[which])) return rc;
     for (int s = 0; s < c->S; ++s) {
         auto& r = c->rings[(size_t)s];
-        int16_t* dst = blk + (size_t)s * 2 * (size_t)n;
+        uint8_t* dst = blk + (size_t)s * c->bps * (size_t)n;
         // the producer only ever writes beyond head, so [tail, tail + n) is stable without the lock
         long long at = r.tail % c->ring;
         long long first = n < c->ring - at ? n : c->ring - at;
-        memcpy(dst, r.buf.data() + 2 * at, sizeof(int16_t) * 2 * (size_t)first);
-        if (first < n) memcpy(dst + 2 * first, r.buf.data(), sizeof(int16_t) * 2 * (size_t)(n - first));
+        memcpy(dst, r.buf.data() + c->bps * at, c->bps * (size_t)first);
+        if (first < n) memcpy(dst + c->bps * first, r.buf.data(), c->bps * (size_t)(n - first));
         std::lock_guard<std::mutex> lk(r.mu);
         r.tail += n;
     }
     c->block_push[which] = nvx_engine_host_pushes(c->eng);
-    const int rc = nvx_engine_push_host_s16(c->eng, blk, n);
+    const int rc = c->u8 ? nvx_engine_push_host_u8(c->eng, blk, n) : nvx_engine_push_host_s16(c->eng, reinterpret_cast<const int16_t*>(blk), n);
     if (rc != 0) { c->block_push[which] = -1; return rc; }
     return n;
 }
-}  // namespace
-
-extern "C" {
-
-int nvx_capture_create(nvx_engine* e, int n_streams, long long max_block, long long ring_samples, nvx_capture** out) {
+int create(nvx_engine* e, int n_streams, long long max_block, long long ring_samples, bool u8, nvx_capture** out) {
     if (!e || !out || n_streams <= 0 || max_block <= 0 || max_block % NVX_BLOCK_ALIGN != 0 || ring_samples < 2 * max_block) return NVX_ERR_ARG;
     nvx_capture* c = new nvx_capture();
     c->eng = e;
     c->S = n_streams;
     c->ring = ring_samples;
     c->max_block = max_block;
+    c->u8 = u8;
+    c->bps = u8 ? 2 : 4;
     c->rings = std::vector<nvx_capture::Ring>((size_t)n_streams);
-    for (auto& r : c->rings) r.buf.assign(2 * (size_t)ring_samples, 0);
+    for (auto& r : c->rings) r.buf.assign(c->bps * (size_t)ring_samples, 0);
     for (int k = 0; k < 2; ++k) {
         void* p = nullptr;
-        if (const int rc = nvx_pinned_alloc((size_t)n_streams * 2 * (size_t)max_block * sizeof(int16_t), 0, &p)) {
+        if (const int rc = nvx_pinned_alloc((size_t)n_streams * c->bps * (size_t)max_block, 0, &p)) {
             nvx_pinned_free(c->block[0]);
             delete c;
             return rc;
         }
-        c->block[k] = static_cast<int16_t*>(p);
+        c->block[k] = static_cast<uint8_t*>(p);
     }
     *out = c;
     return 0;
 }
 
-int nvx_capture_write(nvx_capture* c, int stream, const short* xi, const short* xq, unsigned num_samples) {
-    if (!c || stream < 0 || stream >= c->S || (!xi && num_samples) || (!xq && num_samples)) return NVX_ERR_ARG;
+// reserve room for num_samples in the ring of `stream`; put(at, i, k) stores samples i .. i + k - 1 at ring position `at`
+// (k contiguous ring slots).  Unlike the reference ring (which silently overwrites unread samples when the consumer lags,
+// capt_sched.c:120-128) an overrun is reported: the samples that do not fit are dropped and counted.
+template <typename Put>
+int write_ring(nvx_capture* c, int stream, unsigned num_samples, Put put) {
     auto& r = c->rings[(size_t)stream];
     long long head, tail;
     {
@@ -114,21 +119,45 @@ int nvx_capture_write(nvx_capture* c, int stream, const short* xi, const short* 
         head = r.head;
         tail = r.tail;
     }
-    // unlike the reference ring (which silently overwrites unread samples when the consumer lags, capt_sched.c:120-128)
-    // an overrun is reported: the samples that do not fit are dropped and counted
     long long room = c->ring - (head - tail);
     unsigned take = num_samples;
     int rc = 0;
     if ((long long)take > room) { take = (unsigned)(room > 0 ? room : 0); rc = NVX_ERR_OVERFLOW; }
-    for (unsigned i = 0; i < take; ++i) {
-        const long long at = (head + i) % c->ring;
-        r.buf[2 * (size_t)at] = xi[i];
-        r.buf[2 * (size_t)at + 1] = xq[i];
-    }
+    const long long at = head % c->ring;
+    const unsigned first = (long long)take < c->ring - at ? take : (unsigned)(c->ring - at);
+    put(r.buf.data() + c->bps * (size_t)at, 0u, first);
+    if (first < take) put(r.buf.data(), first, take - first);
     std::lock_guard<std::mutex> lk(r.mu);
     r.head = head + take;
     r.dropped += num_samples - take;
     return rc;
+}
+}  // namespace
+
+extern "C" {
+
+int nvx_capture_create(nvx_engine* e, int n_streams, long long max_block, long long ring_samples, nvx_capture** out) {
+    return create(e, n_streams, max_block, ring_samples, false, out);
+}
+
+int nvx_capture_create_u8(nvx_engine* e, int n_streams, long long max_block, long long ring_samples, nvx_capture** out) {
+    return create(e, n_streams, max_block, ring_samples, true, out);
+}
+
+int nvx_capture_write(nvx_capture* c, int stream, const short* xi, const short* xq, unsigned num_samples) {
+    if (!c || c->u8 || stream < 0 || stream >= c->S || (!xi && num_samples) || (!xq && num_samples)) return NVX_ERR_ARG;
+    return write_ring(c, stream, num_samples, [&](uint8_t* dst, unsigned i0, unsigned k) {
+        int16_t* d = reinterpret_cast<int16_t*>(dst);
+        for (unsigned i = 0; i < k; ++i) {
+            d[2 * i] = xi[i0 + i];
+            d[2 * i + 1] = xq[i0 + i];
+        }
+    });
+}
+
+int nvx_capture_write_u8(nvx_capture* c, int stream, const unsigned char* iq, unsigned num_samples) {
+    if (!c || !c->u8 || stream < 0 || stream >= c->S || (!iq && num_samples)) return NVX_ERR_ARG;
+    return write_ring(c, stream, num_samples, [&](uint8_t* dst, unsigned i0, unsigned k) { memcpy(dst, iq + 2 * (size_t)i0, 2 * (size_t)k); });
 }
 
 long long nvx_capture_pump(nvx_capture* c) {

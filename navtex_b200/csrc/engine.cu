@@ -26,12 +26,12 @@
 #include "message_assembler.h"
 
 namespace nvx {
-int cascade_box_elems(bool s16);
+int cascade_box_elems(SampleFmt f);
 int cascade_tap_class(int n1, int n2, int n3);
 int cascade_warm_super(int tap_class);
 void cascade_fill_taps(int tap_class, const double* h1, int n1, const double* h2, int n2, const double* h3, int n3, CascadeTaps* out);
-cudaError_t cascade_launch(const CascadeArgs& a, const CascadeTaps& taps, int tap_class, bool custom_taps, bool s16, int n_ch, cudaStream_t stream);
-int cascade_target_warps(int device, int reserved_sms, bool s16, int tap_class, bool heavy);
+cudaError_t cascade_launch(const CascadeArgs& a, const CascadeTaps& taps, int tap_class, bool custom_taps, SampleFmt f, int n_ch, cudaStream_t stream);
+int cascade_target_warps(int device, int reserved_sms, SampleFmt f, int tap_class, bool heavy);
 }  // namespace nvx
 
 namespace {
@@ -68,15 +68,16 @@ int load_encode() {
 }
 
 // 32-bit-element view of a stream-major sample array: [rows][2 * cols] floats for float2 samples, [rows][cols] words for
-// short2 samples (one word = one I,Q pair); box = one ring stage x 32 rows
-int encode_rows(CUtensorMap* map, const void* base, long long cols, long long rows, bool s16) {
+// short2 samples (one word = one I,Q pair), [rows][cols / 2] words for 8-bit pairs (one word = two pairs; cols is a multiple
+// of 280); box = one ring stage x 32 rows
+int encode_rows(CUtensorMap* map, const void* base, long long cols, long long rows, nvx::SampleFmt f) {
     if (int rc = load_encode()) return rc;
-    const long long el = s16 ? 1 : 2;
-    cuuint64_t dims[2] = {(cuuint64_t)(el * cols), (cuuint64_t)rows};
-    cuuint64_t strides[1] = {(cuuint64_t)(cols * el * 4)};
-    cuuint32_t box[2] = {(cuuint32_t)nvx::cascade_box_elems(s16), 32};
+    const long long row_bytes = cols * nvx::sample_bytes(f);
+    cuuint64_t dims[2] = {(cuuint64_t)(row_bytes / 4), (cuuint64_t)rows};
+    cuuint64_t strides[1] = {(cuuint64_t)row_bytes};
+    cuuint32_t box[2] = {(cuuint32_t)nvx::cascade_box_elems(f), 32};
     cuuint32_t estr[2] = {1, 1};
-    CUresult r = g_encode(map, s16 ? CU_TENSOR_MAP_DATA_TYPE_INT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(base), dims, strides, box, estr,
+    CUresult r = g_encode(map, f == nvx::SampleFmt::F32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_INT32, 2, const_cast<void*>(base), dims, strides, box, estr,
                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return fail(NVX_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) cols=%lld rows=%lld", (int)r, cols, rows);
@@ -99,6 +100,23 @@ __global__ void tail_carry_kernel(const Sample* __restrict__ old_tail, const Sam
     *reinterpret_cast<int4*>(new_tail + (size_t)s * halo + k) = *src;
 }
 
+// long-tap path, 8-bit input: out = (u - 128) as short2, 8 samples (16 bytes in, 32 out) per thread; count = S n, a multiple of 280
+__global__ void widen_u8_kernel(const uchar2* __restrict__ in, short2* __restrict__ out, long long count) {
+    const long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 8;
+    if (i >= count) return;
+    const int4 v = *reinterpret_cast<const int4*>(in + i);
+    const unsigned w[4] = {(unsigned)v.x, (unsigned)v.y, (unsigned)v.z, (unsigned)v.w};
+    int o[8];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {       // bytes I0 Q0 I1 Q1 of a word -> two short2 words
+        o[2 * k] = (int)(((w[k] & 0xFFu) - 128u) & 0xFFFFu) | (int)(((((w[k] >> 8) & 0xFFu) - 128u) & 0xFFFFu) << 16);
+        o[2 * k + 1] = (int)((((w[k] >> 16) & 0xFFu) - 128u) & 0xFFFFu) | (int)((((w[k] >> 24) - 128u) & 0xFFFFu) << 16);
+    }
+    int4* dst = reinterpret_cast<int4*>(out + i);
+    dst[0] = make_int4(o[0], o[1], o[2], o[3]);
+    dst[1] = make_int4(o[4], o[5], o[6], o[7]);
+}
+
 }  // namespace
 
 constexpr int kBuf = 3;   // blocks in flight: cascade of block i+1/i+2 overlaps demod + event download of block i
@@ -116,11 +134,12 @@ struct nvx_engine {
     int last_buf = 0;
     int tap_class = 0;                    // fused-kernel tap-length class (fir_cascade.cuh), -1 = long-tap path
     int halo = 1960;                      // carried input samples per stream: 280 x the class's warm-up superblocks
-    // carried input tail, ping-pong, in the sample format being pushed: [S][halo] float2 or short2
-    void* tail[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};     // [format][ping-pong]
-    CUtensorMap map_tail[2][2];
+    // carried input tail, ping-pong, in the sample format being pushed: [S][halo] float2, short2 or 8-bit pairs
+    void* tail[nvx::kSampleFmts][2] = {};                            // [format][ping-pong]
+    CUtensorMap map_tail[nvx::kSampleFmts][2];
     int tail_cur = 0;
-    int fmt = -1;                         // -1 = nothing pushed since create/reset, 0 = float2, 1 = short2
+    int fmt = -1;                         // -1 = nothing pushed since create/reset, else the nvx::SampleFmt of the pushes
+    short2* u8_wide = nullptr;            // long-tap path, 8-bit input: [S][max_block] short2 (u - 128), allocated on first use
     nvx::DemodBuffers db = {};
     double* corrbuf[2] = {nullptr, nullptr};   // |mask correlation| rows, alternating per block (each block reads its history from the other)
     uint8_t* d_events[kBuf] = {}; int* d_ev_count[kBuf] = {}; int ev_cap = 0;
@@ -152,7 +171,7 @@ struct nvx_engine {
     std::vector<int> stream_tag;          // optional [S][2] message tags
     bool serial = false;                  // NVX_PIPELINE=serial: the next cascade waits for this block's whole demod
     bool ff_on_main = true;               // feed-forward demod kernels follow the cascade on the main stream
-    int target_warps[2] = {576, 576};     // resident cascade warps per sample format
+    int target_warps[nvx::kSampleFmts] = {576, 576, 576};   // resident cascade warps per sample format
     nvx::MessageAssembler assembler;
     std::vector<nvx::AssembledMessage> ready, handed;
     std::vector<nvx_message> view;
@@ -191,7 +210,8 @@ int free_engine(nvx_engine* e) {
         e->worker.join();
     }
     for (cudaEvent_t ev : e->ev_pool) cudaEventDestroy(ev);
-    for (int f = 0; f < 2; ++f) { cudaFree(e->tail[f][0]); cudaFree(e->tail[f][1]); }
+    for (int f = 0; f < nvx::kSampleFmts; ++f) { cudaFree(e->tail[f][0]); cudaFree(e->tail[f][1]); }
+    cudaFree(e->u8_wide);
     cudaFree(e->corrbuf[0]); cudaFree(e->corrbuf[1]); cudaFree(e->db.clock); cudaFree(e->db.fsm);
     cudaFree(e->db.bitpos); cudaFree(e->db.bitval); cudaFree(e->db.nbits);
     cudaFree(e->d_bits); cudaFree(e->d_disc); cudaFree(e->d_bit_count);
@@ -222,9 +242,11 @@ int free_engine(nvx_engine* e) {
 }
 
 int reset_state(nvx_engine* e) {
-    for (int f = 0; f < 2; ++f)
+    // the warm-up before the first block sees silence: the value 0, which is the byte 128 in 8-bit offset binary
+    for (int f = 0; f < nvx::kSampleFmts; ++f)
         for (int k = 0; k < 2; ++k)
-            CU_TRY(cudaMemsetAsync(e->tail[f][k], 0, (size_t)e->S * e->halo * (f ? sizeof(short2) : sizeof(float2)), e->stream));
+            CU_TRY(cudaMemsetAsync(e->tail[f][k], (nvx::SampleFmt)f == nvx::SampleFmt::U8 ? 128 : 0,
+                                   (size_t)e->S * e->halo * nvx::sample_bytes((nvx::SampleFmt)f), e->stream));
     e->fmt = -1;
     if (e->long_taps)
         for (int k = 0; k < 3; ++k)
@@ -384,11 +406,11 @@ void note_tc_fallback(nvx_engine* e, int stage, const char* why) {
     fail(0, "note: long-tap stage %d ran on the CUDA-core kernel: %s", stage, why);
 }
 
-int process_block(nvx_engine* e, const void* d_x, long long n, bool s16) {
+int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fmt) {
     using namespace nvx;
-    if (e->fmt >= 0 && e->fmt != (int)s16)
-        return fail(NVX_ERR_ARG, "sample format changed between pushes (float and int16 blocks cannot be mixed without a reset)");
-    e->fmt = (int)s16;
+    if (e->fmt >= 0 && e->fmt != (int)fmt)
+        return fail(NVX_ERR_ARG, "sample format changed between pushes (float, int16 and 8-bit blocks cannot be mixed without a reset)");
+    e->fmt = (int)fmt;
     if (n <= 0 || n % kSuper != 0) return fail(NVX_ERR_ARG, "block length %lld is not a positive multiple of %d", n, kSuper);
     if (n > e->cfg.max_block) return fail(NVX_ERR_ARG, "block length %lld exceeds max_block %lld", n, e->cfg.max_block);
     if (((uintptr_t)d_x & 15) != 0) return fail(NVX_ERR_ARG, "device block is not 16-byte aligned");
@@ -400,12 +422,12 @@ int process_block(nvx_engine* e, const void* d_x, long long n, bool s16) {
         collect_spans(e);
     }
     CascadeArgs ca;
-    if (int rc = encode_rows(&ca.map_x, d_x, n, e->S, s16)) return rc;
-    ca.map_tail = e->map_tail[s16][e->tail_cur];
+    if (int rc = encode_rows(&ca.map_x, d_x, n, e->S, fmt)) return rc;
+    ca.map_tail = e->map_tail[(int)fmt][e->tail_cur];
     const int n_super = (int)(n / kSuper);
     const int groups = (e->S + 31) / 32;
     // time segments: enough warps to fill the machine once, but keep the 7-superblock warm-up small
-    int segs = e->target_warps[s16] / groups;            // never more warps than are resident at once (no second wave)
+    int segs = e->target_warps[(int)fmt] / groups;            // never more warps than are resident at once (no second wave)
     const int min_seg = 63;
     if (segs > n_super / min_seg) segs = n_super / min_seg;
     if (segs < 1) segs = 1;
@@ -443,6 +465,16 @@ int process_block(nvx_engine* e, const void* d_x, long long n, bool s16) {
         CU_TRY(cudaEventRecord(t0, e->stream));
     }
     if (e->long_taps) {
+        // 8-bit input: widened to the int16 values u - 128 in front of the unchanged int16 long path (same results bit for bit)
+        if (fmt == SampleFmt::U8) {
+            if (!e->u8_wide) CU_TRY(cudaMalloc(&e->u8_wide, (size_t)e->S * e->cfg.max_block * sizeof(short2)));
+            const long long count = (long long)e->S * n;
+            widen_u8_kernel<<<(unsigned)((count / 8 + 255) / 256), 256, 0, e->stream>>>(static_cast<const uchar2*>(d_x), e->u8_wide, count);
+            CU_TRY(cudaGetLastError());
+            e->stats.aux_launches++;
+            d_x = e->u8_wide;
+        }
+        const int s16 = fmt != SampleFmt::F32;
         const int cur = e->lcur, nx = cur ^ 1;
         const long long p1 = e->cfg.max_block / NVX_D1, p2 = e->cfg.max_block / (NVX_D1 * NVX_D2);
         LongArgs la = {};
@@ -483,7 +515,7 @@ int process_block(nvx_engine* e, const void* d_x, long long n, bool s16) {
             const int left = e->C - c0;
             const int n_ch = left <= nvx::kMaxFusedCh ? left : (left + 1) / 2;      // 5 = 3 + 2, 6 = 3 + 3, 7 = 4 + 3, 8 = 4 + 4
             ca.ch0 = c0;
-            CU_TRY(cascade_launch(ca, e->taps, e->tap_class, e->custom_taps, s16, n_ch, e->stream));
+            CU_TRY(cascade_launch(ca, e->taps, e->tap_class, e->custom_taps, fmt, n_ch, e->stream));
             if (c0) e->stats.aux_launches++;
             c0 += n_ch;
         }
@@ -492,14 +524,19 @@ int process_block(nvx_engine* e, const void* d_x, long long n, bool s16) {
 
     const int nxt = e->tail_cur ^ 1;
     if (!e->long_taps) {
-        const long long work = (long long)e->S * (e->halo / (s16 ? 4 : 2));
+        const long long work = (long long)e->S * (e->halo / (16 / sample_bytes(fmt)));
         const unsigned grid = (unsigned)((work + 255) / 256);
-        if (s16)
-            tail_carry_kernel<short2><<<grid, 256, 0, e->stream>>>(static_cast<const short2*>(e->tail[1][e->tail_cur]), static_cast<const short2*>(d_x),
-                                                                   static_cast<short2*>(e->tail[1][nxt]), e->S, n, e->halo);
+        const void* old_tail = e->tail[(int)fmt][e->tail_cur];
+        void* new_tail = e->tail[(int)fmt][nxt];
+        if (fmt == SampleFmt::U8)
+            tail_carry_kernel<uchar2><<<grid, 256, 0, e->stream>>>(static_cast<const uchar2*>(old_tail), static_cast<const uchar2*>(d_x),
+                                                                   static_cast<uchar2*>(new_tail), e->S, n, e->halo);
+        else if (fmt == SampleFmt::S16)
+            tail_carry_kernel<short2><<<grid, 256, 0, e->stream>>>(static_cast<const short2*>(old_tail), static_cast<const short2*>(d_x),
+                                                                   static_cast<short2*>(new_tail), e->S, n, e->halo);
         else
-            tail_carry_kernel<float2><<<grid, 256, 0, e->stream>>>(static_cast<const float2*>(e->tail[0][e->tail_cur]), static_cast<const float2*>(d_x),
-                                                                   static_cast<float2*>(e->tail[0][nxt]), e->S, n, e->halo);
+            tail_carry_kernel<float2><<<grid, 256, 0, e->stream>>>(static_cast<const float2*>(old_tail), static_cast<const float2*>(d_x),
+                                                                   static_cast<float2*>(new_tail), e->S, n, e->halo);
         CU_TRY(cudaGetLastError());
     }
     e->tail_cur = nxt;
@@ -549,10 +586,10 @@ int process_block(nvx_engine* e, const void* d_x, long long n, bool s16) {
 }
 
 // H2D on the copy stream into staging slot k % 2, then the block's kernels on the main stream
-int push_host(nvx_engine* e, const void* iq, long long n, bool s16) {
+int push_host(nvx_engine* e, const void* iq, long long n, nvx::SampleFmt fmt) {
     if (n <= 0 || n % nvx::kSuper != 0 || n > e->cfg.max_block) return fail(NVX_ERR_ARG, "bad block length %lld", n);
     CU_TRY(cudaSetDevice(e->cfg.device));
-    const size_t bytes = (size_t)e->S * (size_t)n * (s16 ? sizeof(short2) : sizeof(float2));
+    const size_t bytes = (size_t)e->S * (size_t)n * nvx::sample_bytes(fmt);
     const int slot = (int)(e->host_pushes % 2);
     if (e->stage_bytes[slot] < bytes) {
         CU_TRY(cudaStreamSynchronize(e->stream_copy));
@@ -566,7 +603,7 @@ int push_host(nvx_engine* e, const void* iq, long long n, bool s16) {
     CU_TRY(cudaMemcpyAsync(e->stage[slot], iq, bytes, cudaMemcpyHostToDevice, e->stream_copy));
     CU_TRY(cudaEventRecord(e->copy_done[slot], e->stream_copy));
     CU_TRY(cudaStreamWaitEvent(e->stream, e->copy_done[slot], 0));
-    if (int rc = process_block(e, e->stage[slot], n, s16)) return rc;
+    if (int rc = process_block(e, e->stage[slot], n, fmt)) return rc;
     CU_TRY(cudaEventRecord(e->stage_free[slot], e->stream));
     e->host_pushes++;
     return 0;
@@ -690,9 +727,9 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
         CREATE_TRY(cudaEventCreateWithFlags(&e->demod_done[k], cudaEventDisableTiming));
         CREATE_TRY(cudaEventCreateWithFlags(&e->ff_done[k], cudaEventDisableTiming));
     }
-    for (int f = 0; f < 2; ++f)
+    for (int f = 0; f < nvx::kSampleFmts; ++f)
         for (int k = 0; k < 2; ++k)
-            CREATE_TRY(cudaMalloc(&e->tail[f][k], (size_t)e->S * e->halo * (f ? sizeof(short2) : sizeof(float2))));
+            CREATE_TRY(cudaMalloc(&e->tail[f][k], (size_t)e->S * e->halo * nvx::sample_bytes((nvx::SampleFmt)f)));
     e->db.p_max = e->P_max;
     for (int k = 0; k < kBuf; ++k) CREATE_TRY(cudaMalloc(&e->y3buf[k], (size_t)e->channels * (nvx::kHistY + e->P_max) * sizeof(float2)));
     for (int k = 0; k < 2; ++k) CREATE_TRY(cudaMalloc(&e->corrbuf[k], (size_t)e->channels * (nvx::kHistC + e->P_max + nvx::kPadC) * sizeof(double)));
@@ -757,10 +794,11 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
         CREATE_TRY(cudaMemcpy(e->d_nco_ch, nco_ch.data(), nco_ch.size() * sizeof(nvx::NcoChan), cudaMemcpyHostToDevice));
     }
 #undef CREATE_TRY
-    for (int f = 0; f < 2; ++f)
+    for (int f = 0; f < nvx::kSampleFmts; ++f)
         for (int k = 0; k < 2; ++k)
-            if (int rc = encode_rows(&e->map_tail[f][k], e->tail[f][k], e->halo, e->S, f != 0)) { free_engine(e); return rc; }
-    for (int f = 0; f < 2; ++f) e->target_warps[f] = nvx::cascade_target_warps(cfg->device, nvx::demod_reserved_sms(e->channels), f != 0, e->tap_class, C > 2);
+            if (int rc = encode_rows(&e->map_tail[f][k], e->tail[f][k], e->halo, e->S, (nvx::SampleFmt)f)) { free_engine(e); return rc; }
+    for (int f = 0; f < nvx::kSampleFmts; ++f)
+        e->target_warps[f] = nvx::cascade_target_warps(cfg->device, nvx::demod_reserved_sms(e->channels), (nvx::SampleFmt)f, e->tap_class, C > 2);
     e->assembler.resize(e->channels);
     if (int rc = reset_state(e)) { free_engine(e); return rc; }
     e->worker = std::thread(worker_main, e);
@@ -785,24 +823,36 @@ int nvx_engine_reset(nvx_engine* e) {
 int nvx_engine_push_device_f32(nvx_engine* e, const void* d_iq, long long n) {
     if (!e || !d_iq) return fail(NVX_ERR_ARG, "null argument");
     CU_TRY(cudaSetDevice(e->cfg.device));
-    return process_block(e, d_iq, n, false);
+    return process_block(e, d_iq, n, nvx::SampleFmt::F32);
 }
 
 int nvx_engine_push_device_s16(nvx_engine* e, const void* d_iq, long long n) {
     if (!e || !d_iq) return fail(NVX_ERR_ARG, "null argument");
     if (((uintptr_t)d_iq & 15) != 0) return fail(NVX_ERR_ARG, "device block is not 16-byte aligned");
     CU_TRY(cudaSetDevice(e->cfg.device));
-    return process_block(e, d_iq, n, true);
+    return process_block(e, d_iq, n, nvx::SampleFmt::S16);
+}
+
+int nvx_engine_push_device_u8(nvx_engine* e, const void* d_iq, long long n) {
+    if (!e || !d_iq) return fail(NVX_ERR_ARG, "null argument");
+    if (((uintptr_t)d_iq & 15) != 0) return fail(NVX_ERR_ARG, "device block is not 16-byte aligned");
+    CU_TRY(cudaSetDevice(e->cfg.device));
+    return process_block(e, d_iq, n, nvx::SampleFmt::U8);
 }
 
 int nvx_engine_push_host_f32(nvx_engine* e, const float* iq, long long n) {
     if (!e || !iq) return fail(NVX_ERR_ARG, "null argument");
-    return push_host(e, iq, n, false);
+    return push_host(e, iq, n, nvx::SampleFmt::F32);
 }
 
 int nvx_engine_push_host_s16(nvx_engine* e, const int16_t* iq, long long n) {
     if (!e || !iq) return fail(NVX_ERR_ARG, "null argument");
-    return push_host(e, iq, n, true);
+    return push_host(e, iq, n, nvx::SampleFmt::S16);
+}
+
+int nvx_engine_push_host_u8(nvx_engine* e, const uint8_t* iq, long long n) {
+    if (!e || !iq) return fail(NVX_ERR_ARG, "null argument");
+    return push_host(e, iq, n, nvx::SampleFmt::U8);
 }
 
 int nvx_engine_wait_ingest(nvx_engine* e) {

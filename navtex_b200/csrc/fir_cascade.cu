@@ -7,15 +7,15 @@
 
 namespace nvx {
 
-template <bool kImm, bool kGenNco, bool kS16, int kClass, int kCh>
-__global__ void __launch_bounds__(InFmt<kS16, kClass, kCh>::kWarps * 32, kCtasPerSm) fir_cascade_kernel(const __grid_constant__ CascadeParams<kClass> prm) {
+template <bool kImm, bool kGenNco, SampleFmt kFmt, int kClass, int kCh>
+__global__ void __launch_bounds__(InFmt<kFmt, kClass, kCh>::kWarps * 32, kCtasPerSm) fir_cascade_kernel(const __grid_constant__ CascadeParams<kClass> prm) {
     const CascadeArgs& a = prm.a;
-    using F = InFmt<kS16, kClass, kCh>;
+    using F = InFmt<kFmt, kClass, kCh>;
     using G = Geo<kClass>;
     constexpr int kWarmSuper = G::kWarm, kHalo = G::kWarm * kSuper, kLive1 = G::kLive1, kLive2 = G::kLive2, kLive3 = G::kLive3;
     constexpr int kWarpsPerCta = F::kWarps;
     constexpr int kStages = F::kStages, kStageBytes = F::kStageBytes, kStepsPerStage = F::kSteps, kStageIn = F::kStageIn;
-    constexpr int kRowBytes = F::kRowBytes, kStepBytes = F::kStepBytes, kEl = F::kElemsPerSample;
+    constexpr int kRowBytes = F::kRowBytes;
     extern __shared__ __align__(128) uint8_t smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     uint8_t* const wbase = smem + (size_t)warp * (kStages * kStageBytes);
@@ -45,13 +45,16 @@ __global__ void __launch_bounds__(InFmt<kS16, kClass, kCh>::kWarps * 32, kCtasPe
     // first input sample of this segment's warm-up, relative to the chunk start (negative = carried tail)
     const long long pos0 = ((long long)first_sb - kWarmSuper) * kSuper;
 
+    // sample position -> 32-bit element of the tensor map (8-bit pairs: two samples per element; stage positions and the halo
+    // are multiples of 56, so the division is exact)
+    auto elem = [](long long p) { return (int)(p * F::kSampleBytes / 4); };
     auto issue = [&](int t, int stage) {
         if (lane == 0) {
             const uint32_t bar = bar0 + 8 * stage;
             const long long p = pos0 + (long long)t * kStageIn;
             mbar_arrive_expect_tx(bar, kStageBytes);
-            if (p < 0) tma_load_2d(wbase_s + stage * kStageBytes, &a.map_tail, (int)(kEl * (p + kHalo)), strm0, bar);
-            else       tma_load_2d(wbase_s + stage * kStageBytes, &a.map_x, (int)(kEl * p), strm0, bar);
+            if (p < 0) tma_load_2d(wbase_s + stage * kStageBytes, &a.map_tail, elem(p + kHalo), strm0, bar);
+            else       tma_load_2d(wbase_s + stage * kStageBytes, &a.map_x, elem(p), strm0, bar);
         }
     };
 
@@ -117,7 +120,7 @@ __global__ void __launch_bounds__(InFmt<kS16, kClass, kCh>::kWarps * 32, kCtasPe
                     if (nco_idx[c] >= kNcoDen) nco_idx[c] -= kNcoDen;
                 }
             }
-            cascade_step<kImm, kGenNco, kS16, kClass, kCh>(prm.taps, prm.nco, st, reinterpret_cast<const float4*>(rowb + u * kStepBytes), phase, r10 + u, y3, nl);
+            cascade_step<kImm, kGenNco, kFmt, kClass, kCh>(prm.taps, prm.nco, st, rowb, u, phase, r10 + u, y3, nl);
             phase += 7;
             if (phase >= kNcoPeriod) phase -= kNcoPeriod;
         }
@@ -136,7 +139,9 @@ __global__ void __launch_bounds__(InFmt<kS16, kClass, kCh>::kWarps * 32, kCtasPe
     }
 }
 
-int cascade_box_elems(bool s16) { return s16 ? InFmt<true>::kBoxElems : InFmt<false>::kBoxElems; }
+int cascade_box_elems(SampleFmt f) {
+    return f == SampleFmt::F32 ? InFmt<SampleFmt::F32>::kBoxElems : f == SampleFmt::S16 ? InFmt<SampleFmt::S16>::kBoxElems : InFmt<SampleFmt::U8>::kBoxElems;
+}
 
 // pad a tap set with zeros at the old end up to the class length (a shorter FIR is the same FIR with zero taps)
 template <int kClass>
@@ -180,42 +185,50 @@ void cascade_fill_taps(int tap_class, const double* h1, int n1, const double* h2
 
 // warps that are resident at once across the device, leaving `reserved_sms` SMs to the sequential demod kernels:
 // the host sizes the grid to at most one full wave
-template <bool kS16, int kClass, int kCh>
+template <SampleFmt kFmt, int kClass, int kCh>
 static int target_warps_fmt(int device, int reserved_sms) {
-    using F = InFmt<kS16, kClass, kCh>;
+    using F = InFmt<kFmt, kClass, kCh>;
     int sms = 148, per_sm = kCtasPerSm;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-    auto kern = fir_cascade_kernel<false, true, kS16, kClass, kCh>;
+    auto kern = fir_cascade_kernel<false, true, kFmt, kClass, kCh>;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, F::kSmemBytes);
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, F::kWarps * 32, F::kSmemBytes) != cudaSuccess || per_sm < 1)
         per_sm = kCtasPerSm;
     if (sms - reserved_sms >= 8) sms -= reserved_sms;
     return sms * per_sm * F::kWarps;
 }
-// heavy = a launch carries three or four channels (different CTA shape for int16 input)
-int cascade_target_warps(int device, int reserved_sms, bool s16, int tap_class, bool heavy) {
-    if (tap_class == 1) return s16 ? target_warps_fmt<true, 1, 2>(device, reserved_sms) : target_warps_fmt<false, 1, 2>(device, reserved_sms);
-    if (heavy) return s16 ? target_warps_fmt<true, 0, 4>(device, reserved_sms) : target_warps_fmt<false, 0, 4>(device, reserved_sms);
-    return s16 ? target_warps_fmt<true, 0, 2>(device, reserved_sms) : target_warps_fmt<false, 0, 2>(device, reserved_sms);
+template <int kClass, int kCh>
+static int target_warps_cls(int device, int reserved_sms, SampleFmt f) {
+    switch (f) {
+        case SampleFmt::F32: return target_warps_fmt<SampleFmt::F32, kClass, kCh>(device, reserved_sms);
+        case SampleFmt::S16: return target_warps_fmt<SampleFmt::S16, kClass, kCh>(device, reserved_sms);
+        default: return target_warps_fmt<SampleFmt::U8, kClass, kCh>(device, reserved_sms);
+    }
+}
+// heavy = a launch carries three or four channels (different CTA shape for integer input)
+int cascade_target_warps(int device, int reserved_sms, SampleFmt f, int tap_class, bool heavy) {
+    if (tap_class == 1) return target_warps_cls<1, 2>(device, reserved_sms, f);
+    if (heavy) return target_warps_cls<0, 4>(device, reserved_sms, f);
+    return target_warps_cls<0, 2>(device, reserved_sms, f);
 }
 
-template <bool kS16, int kClass, int kCh>
+template <SampleFmt kFmt, int kClass, int kCh>
 static cudaError_t launch_fmt(const CascadeArgs& a, const CascadeTaps& taps, bool custom_taps, cudaStream_t stream) {
-    const size_t smem = InFmt<kS16, kClass, kCh>::kSmemBytes;
+    const size_t smem = InFmt<kFmt, kClass, kCh>::kSmemBytes;
     // more than two channels always run the general (per-channel) NCO; two channels use the reference's table unless offsets were given
     const bool gen = a.nco != nullptr;
     // immediates only for the reference taps themselves; every other set (class 0 or 1) reads the constant bank
     constexpr bool kCanImm = kClass == 0;
     constexpr bool kTable = kCh == 2;          // the table variants exist for exactly two channels
     auto kern = (gen || !kTable)
-                    ? ((custom_taps || !kCanImm) ? fir_cascade_kernel<false, true, kS16, kClass, kCh> : fir_cascade_kernel<kCanImm, true, kS16, kClass, kCh>)
-                    : ((custom_taps || !kCanImm) ? fir_cascade_kernel<false, !kTable, kS16, kClass, kCh> : fir_cascade_kernel<kCanImm, !kTable, kS16, kClass, kCh>);
+                    ? ((custom_taps || !kCanImm) ? fir_cascade_kernel<false, true, kFmt, kClass, kCh> : fir_cascade_kernel<kCanImm, true, kFmt, kClass, kCh>)
+                    : ((custom_taps || !kCanImm) ? fir_cascade_kernel<false, !kTable, kFmt, kClass, kCh> : fir_cascade_kernel<kCanImm, !kTable, kFmt, kClass, kCh>);
     if (!gen && !kTable) return cudaErrorInvalidValue;
     {   // function attributes are per device: set on every launch (cheap) rather than cached process-wide
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
-    constexpr int kWarpsPerCta = InFmt<kS16, kClass, kCh>::kWarps;
+    constexpr int kWarpsPerCta = InFmt<kFmt, kClass, kCh>::kWarps;
     const long long warps = (long long)((a.streams + 31) / 32) * a.segs;
     const unsigned grid = (unsigned)((warps + kWarpsPerCta - 1) / kWarpsPerCta);
     CascadeParams<kClass> prm;
@@ -226,17 +239,26 @@ static cudaError_t launch_fmt(const CascadeArgs& a, const CascadeTaps& taps, boo
     return cudaGetLastError();
 }
 
+template <int kClass, int kCh>
+static cudaError_t launch_cls(SampleFmt f, const CascadeArgs& a, const CascadeTaps& taps, bool custom_taps, cudaStream_t stream) {
+    switch (f) {
+        case SampleFmt::F32: return launch_fmt<SampleFmt::F32, kClass, kCh>(a, taps, custom_taps, stream);
+        case SampleFmt::S16: return launch_fmt<SampleFmt::S16, kClass, kCh>(a, taps, custom_taps, stream);
+        default: return launch_fmt<SampleFmt::U8, kClass, kCh>(a, taps, custom_taps, stream);
+    }
+}
+
 // n_ch = channels of this launch (a.ch0 .. a.ch0 + n_ch - 1): 2 in either tap class, 1 / 3 / 4 in the reference class
-cudaError_t cascade_launch(const CascadeArgs& a, const CascadeTaps& taps, int tap_class, bool custom_taps, bool s16, int n_ch, cudaStream_t stream) {
+cudaError_t cascade_launch(const CascadeArgs& a, const CascadeTaps& taps, int tap_class, bool custom_taps, SampleFmt f, int n_ch, cudaStream_t stream) {
     if (tap_class == 1) {
         if (n_ch != 2) return cudaErrorInvalidValue;
-        return s16 ? launch_fmt<true, 1, 2>(a, taps, true, stream) : launch_fmt<false, 1, 2>(a, taps, true, stream);
+        return launch_cls<1, 2>(f, a, taps, true, stream);
     }
     switch (n_ch) {
-        case 1: return s16 ? launch_fmt<true, 0, 1>(a, taps, custom_taps, stream) : launch_fmt<false, 0, 1>(a, taps, custom_taps, stream);
-        case 2: return s16 ? launch_fmt<true, 0, 2>(a, taps, custom_taps, stream) : launch_fmt<false, 0, 2>(a, taps, custom_taps, stream);
-        case 3: return s16 ? launch_fmt<true, 0, 3>(a, taps, custom_taps, stream) : launch_fmt<false, 0, 3>(a, taps, custom_taps, stream);
-        case 4: return s16 ? launch_fmt<true, 0, 4>(a, taps, custom_taps, stream) : launch_fmt<false, 0, 4>(a, taps, custom_taps, stream);
+        case 1: return launch_cls<0, 1>(f, a, taps, custom_taps, stream);
+        case 2: return launch_cls<0, 2>(f, a, taps, custom_taps, stream);
+        case 3: return launch_cls<0, 3>(f, a, taps, custom_taps, stream);
+        case 4: return launch_cls<0, 4>(f, a, taps, custom_taps, stream);
         default: return cudaErrorInvalidValue;
     }
 }

@@ -18,11 +18,11 @@
 //     the tap as a 32-bit immediate / uniform operand: 2 FMAs per lane per issue slot.
 //   * a warp's 32 rows are 32 consecutive streams at the same time segment, so the samples they
 //     need for two 28-sample steps form a [32 streams x 448 B] box of the stream-major input
-//     (224 B when the input is int16 pairs): ONE TMA tensor copy (cp.async.bulk.tensor.2d ->
+//     (224 B when the input is int16 pairs, 112 B for 8-bit pairs): ONE TMA tensor copy (cp.async.bulk.tensor.2d ->
 //     UTMALDG) per warp per stage into a per-warp ring of shared-memory stages, completion
 //     tracked by one mbarrier per stage.  Each lane then reads its own row with LDS.128.
 //   * variants (template flags): taps as immediates or from the constant bank (replacement tap
-//     sets), the reference's 9-entry NCO table or an exact per-stream NCO, float2 or short2 input.
+//     sets), the reference's 9-entry NCO table or an exact per-stream NCO, float2, short2 or 8-bit input (SampleFmt).
 //   * time segments are made independent by recomputing a 7-superblock (1960-sample) warm-up
 //     from the raw input that precedes the segment (previous segment, or the carried tail of
 //     the previous chunk); since every 900 Hz output depends on exactly 2181 inputs
@@ -75,32 +75,58 @@ constexpr int kNcoPeriod = 9;                      // fir2cpp.C:12-14
 #ifndef NVX_S16_WARPS_PER_CTA
 #define NVX_S16_WARPS_PER_CTA 12
 #endif
+#ifndef NVX_U8_ROW_PAD_BYTES
+#define NVX_U8_ROW_PAD_BYTES 32
+#endif
+#ifndef NVX_U8_STAGES
+#define NVX_U8_STAGES 2
+#endif
+#ifndef NVX_U8_WARPS_PER_CTA
+#define NVX_U8_WARPS_PER_CTA 12
+#endif
 constexpr int kCtasPerSm = NVX_CTAS_PER_SM;
+
+// The sample formats an engine accepts (one between resets).  Every layer -- the fused kernel's staging geometry and
+// conversion, the tensor maps, the tail buffers, the host staging -- takes its decision from this one enum.
+//   F32: float2 I,Q
+//   S16: int16 I,Q pairs (the SDRplay's / WAV's own samples, capt_sched.c:120-128), value = the int16
+//   U8:  unsigned 8-bit offset-binary I,Q pairs (the RTL-SDR's rtlsdr_read_async / rtl_tcp format), value = u - 128 exactly.
+//        128 rather than the converter's mid-scale 127.5 keeps the values integers, so the same capture pushed as int16 (or
+//        fed to the reference) gives bit-identical results; the -0.5 LSB DC offset this leaves sits at -+14 kHz after the
+//        mix, where the channel filter removes it.
+enum class SampleFmt : int { F32 = 0, S16 = 1, U8 = 2 };
+constexpr int kSampleFmts = 3;
+__host__ __device__ constexpr int sample_bytes(SampleFmt f) { return f == SampleFmt::F32 ? 8 : f == SampleFmt::S16 ? 4 : 2; }
+
 // Staging geometry per input sample format.  float2 input: 8 B / sample, 2 steps = 448 B (+16 B pad) per row.
-// short2 input (the radio's / WAV's own int16 I,Q pairs, capt_sched.c:120-128): 4 B / sample, 2 steps = 224 B (+16 B pad)
-// per row; both pads make the per-lane LDS.128 row reads bank-conflict free (row pitch = 4 or 28 words mod 32).  The
-// int16 variant is FP32-issue-bound, not HBM-bound (4.06 B / sample), so short rows cost it nothing, while a loop body
-// of more than two steps would outgrow the 32 KB L1.5 instruction cache -- with one warp per SM sub-partition an
+// short2 input: 4 B / sample, 2 steps = 224 B (+16 B pad) per row.  8-bit input: 2 B / sample, 2 steps = 112 B (+32 B pad)
+// per row; a 28-sample step is 56 B, not a whole number of 16-byte reads, so the 8-bit rows are read per 2-step stage
+// (7 x LDS.128).  All three pads make the per-lane LDS.128 row reads bank-conflict free (row pitch = 4 or 28 words mod
+// 32).  The int16 variant is FP32-issue-bound, not HBM-bound (4.06 B / sample), so short rows cost it nothing, while a loop
+// body of more than two steps would outgrow the 32 KB L1.5 instruction cache -- with one warp per SM sub-partition an
 // instruction fetch from L2 is not hidden (measured: 5 steps per stage = 5.3 ms, 2 steps = 3.3 ms per block).  Being
 // issue-bound it also wants more warps per sub-partition: 12 warps x 2 stages = 2.77 ms, 8 x 3 = 2.90 ms, 16 x 1 = 2.81 ms,
-// 4 warps x 6 stages = 3.27 ms.
-template <bool kS16, int kClass = 0, int kCh = 2>
+// 4 warps x 6 stages = 3.27 ms.  The 8-bit variant runs the same arithmetic on half the bytes; its CTA shapes are the int16
+// ones (DESIGN.md 3.1 has the sweep).
+template <SampleFmt kFmt, int kClass = 0, int kCh = 2>
 struct InFmt {
-    static constexpr int kSteps = kS16 ? NVX_S16_STEPS_PER_STAGE : NVX_STEPS_PER_STAGE;   // 28-sample steps per TMA box row
-    static constexpr int kSampleBytes = kS16 ? 4 : 8;
+    static constexpr bool kF32 = kFmt == SampleFmt::F32;
+    static constexpr int kSteps = kF32 ? NVX_STEPS_PER_STAGE : NVX_S16_STEPS_PER_STAGE;   // 28-sample steps per TMA box row
+    static constexpr int kSampleBytes = sample_bytes(kFmt);
     static constexpr int kStepBytes = kStepIn * kSampleBytes;
     static constexpr int kStageIn = kSteps * kStepIn;                                     // input samples per stream per stage
-    static constexpr int kRowBytes = kSteps * kStepBytes + (kS16 ? NVX_S16_ROW_PAD_BYTES : NVX_ROW_PAD_FLOATS * 4);
+    static constexpr int kPadBytes = kF32 ? NVX_ROW_PAD_FLOATS * 4 : kFmt == SampleFmt::S16 ? NVX_S16_ROW_PAD_BYTES : NVX_U8_ROW_PAD_BYTES;
+    static constexpr int kRowBytes = kSteps * kStepBytes + kPadBytes;
     static constexpr int kBoxElems = kRowBytes / 4;                                       // TMA box width in 32-bit elements (pad over-fetched)
-    static constexpr int kElemsPerSample = kSampleBytes / 4;
     static constexpr int kStageBytes = 32 * kRowBytes;                                    // per warp per stage
     // the medium tap class needs ~250 registers per thread: 4 warps per CTA for either format; three or four channels sharing
     // stage 1 need ~200: at most 8 warps per CTA
-    static constexpr int kStages = kS16 ? (kClass != 0 ? 6 : kCh > 2 ? 3 : NVX_S16_STAGES) : NVX_STAGES;
-    static constexpr int kWarps = kS16 ? (kClass != 0 ? 4 : kCh > 2 ? 8 : NVX_S16_WARPS_PER_CTA) : NVX_WARPS_PER_CTA;      // per CTA
+    static constexpr int kStages = kF32 ? NVX_STAGES : (kClass != 0 ? 6 : kCh > 2 ? 3 : kFmt == SampleFmt::S16 ? NVX_S16_STAGES : NVX_U8_STAGES);
+    static constexpr int kWarps = kF32 ? NVX_WARPS_PER_CTA : (kClass != 0 ? 4 : kCh > 2 ? 8 : kFmt == SampleFmt::S16 ? NVX_S16_WARPS_PER_CTA : NVX_U8_WARPS_PER_CTA);      // per CTA
     static constexpr int kSmemBytes = kWarps * kStages * kStageBytes + kWarps * kStages * 8;
     static_assert(kStepsPerSuper % kSteps == 0, "a stage must not straddle superblocks");
     static_assert(kRowBytes % 16 == 0 && kStageBytes % 128 == 0 && kBoxElems <= 256, "TMA box alignment");
+    static_assert((kSteps * kStepBytes) % 16 == 0, "a stage row is read in whole 16-byte loads");
     static_assert(kSmemBytes <= 227 * 1024, "shared memory per CTA");
 };
 // Tap-length classes of the fused kernel.  Class 0 = the reference lengths 37 / 47 / 71 (taps may be immediates); class 1 =
@@ -155,7 +181,7 @@ constexpr int kMaxFusedCh = 4;   // channels one pass of the fused kernel carrie
 constexpr int kMaxChannels = 8;  // per capture: more than four take two passes over the input
 
 struct CascadeArgs {
-    CUtensorMap map_x;    // 32-bit view [S][2 n] (float2 input) or [S][n] (short2 input) of this chunk, box InFmt::kBoxElems x 32
+    CUtensorMap map_x;    // 32-bit view [S][2 n] (float2 input), [S][n] (short2) or [S][n / 2] (8-bit pairs) of this chunk, box InFmt::kBoxElems x 32
     CUtensorMap map_tail; // same view of [S][halo]: the halo = 280 kWarm samples that preceded the chunk (zeros at start)
     float2* y3;           // [S][2][y3_pitch] 900 Hz output; this chunk's samples start at y3_off
     long long n;          // samples per stream in this chunk (multiple of kSuper)
@@ -247,9 +273,38 @@ __device__ __forceinline__ float2 iq_of(int packed) {
     return __fadd2_rn(biased, make_float2(-8421376.0f, -8421376.0f));
 }
 
-template <bool kImm, bool kGenNco, bool kS16, int kClass, int kCh>
+// 8-bit offset binary u -> u - 128, exact, also without I2F: PRMT puts u in the low mantissa byte of 2^23 (2^23 + u), one
+// packed add of -(2^23 + 128) per I,Q pair finishes it.  No sign flip: the data is offset binary already.
+__device__ __forceinline__ float2 iq_of_u8(unsigned w, unsigned sel_i, unsigned sel_q) {
+    const float2 biased = make_float2(__uint_as_float(__byte_perm(w, 0x4B000000u, sel_i)), __uint_as_float(__byte_perm(w, 0x4B000000u, sel_q)));
+    return __fadd2_rn(biased, make_float2(-8388736.0f, -8388736.0f));
+}
+
+// the four input samples that complete stage-1 output q of step u, read from this lane's row of the ring stage
+template <SampleFmt kFmt>
+__device__ __forceinline__ void load_quad(const uint8_t* stage_row, int u, int q, float2 (&xs)[4]) {
+    if constexpr (kFmt == SampleFmt::F32) {
+        const float4* row = reinterpret_cast<const float4*>(stage_row + u * InFmt<kFmt>::kStepBytes);
+        const float4 v0 = row[2 * q], v1 = row[2 * q + 1];
+        xs[0] = make_float2(v0.x, v0.y); xs[1] = make_float2(v0.z, v0.w);
+        xs[2] = make_float2(v1.x, v1.y); xs[3] = make_float2(v1.z, v1.w);
+    } else if constexpr (kFmt == SampleFmt::S16) {
+        const int4 v = reinterpret_cast<const int4*>(stage_row + u * InFmt<kFmt>::kStepBytes)[q];
+        xs[0] = iq_of(v.x); xs[1] = iq_of(v.y); xs[2] = iq_of(v.z); xs[3] = iq_of(v.w);
+    } else {
+        // 8 B per quad: quad c = 7 u + q of the stage is one half of the stage row's 16-byte word c / 2 (u and q are
+        // compile-time constants, so the two halves of a word come from the same LDS.128)
+        const int c = 7 * u + q;
+        const int4 v = reinterpret_cast<const int4*>(stage_row)[c >> 1];
+        const unsigned w0 = (unsigned)((c & 1) ? v.z : v.x), w1 = (unsigned)((c & 1) ? v.w : v.y);
+        xs[0] = iq_of_u8(w0, 0x7440, 0x7441); xs[1] = iq_of_u8(w0, 0x7442, 0x7443);
+        xs[2] = iq_of_u8(w1, 0x7440, 0x7441); xs[3] = iq_of_u8(w1, 0x7442, 0x7443);
+    }
+}
+
+template <bool kImm, bool kGenNco, SampleFmt kFmt, int kClass, int kCh>
 __device__ __forceinline__ void cascade_step(const TapSet<kClass>& ts, const NcoTable& nco, CascadeState<kClass, kCh>& st,
-                                             const float4* __restrict__ row, int nco_phase, const int r10, float2 (&y3)[kCh], NcoLane<kCh>& nl) {
+                                             const uint8_t* __restrict__ stage_row, const int u, int nco_phase, const int r10, float2 (&y3)[kCh], NcoLane<kCh>& nl) {
     using G = Geo<kClass>;
     constexpr int kLive1 = G::kLive1, kLive2 = G::kLive2, kLive3 = G::kLive3;
     static_assert(!kImm || kClass == 0, "immediate taps are the reference set");
@@ -272,14 +327,7 @@ __device__ __forceinline__ void cascade_step(const TapSet<kClass>& ts, const Nco
     for (int q = 0; q < NVX_D2; ++q) {
         // four inputs complete stage-1 output q of this step
         float2 xs[4];
-        if (kS16) {
-            const int4 v = reinterpret_cast<const int4*>(row)[q];
-            xs[0] = iq_of(v.x); xs[1] = iq_of(v.y); xs[2] = iq_of(v.z); xs[3] = iq_of(v.w);
-        } else {
-            const float4 v0 = row[2 * q], v1 = row[2 * q + 1];
-            xs[0] = make_float2(v0.x, v0.y); xs[1] = make_float2(v0.z, v0.w);
-            xs[2] = make_float2(v1.x, v1.y); xs[3] = make_float2(v1.z, v1.w);
-        }
+        load_quad<kFmt>(stage_row, u, q, xs);
 #pragma unroll
         for (int r = 0; r < NVX_D1; ++r) {
 #pragma unroll

@@ -49,11 +49,13 @@ class SynthDesc(C.Structure):
 
 EXPORTS = (
     "nvx_default_config", "nvx_last_error", "nvx_engine_create", "nvx_engine_destroy", "nvx_engine_reset",
-    "nvx_engine_push_host_f32", "nvx_engine_push_host_s16", "nvx_engine_push_device_f32", "nvx_engine_push_device_s16",
+    "nvx_engine_push_host_f32", "nvx_engine_push_host_s16", "nvx_engine_push_host_u8", "nvx_engine_push_device_f32",
+    "nvx_engine_push_device_s16", "nvx_engine_push_device_u8",
     "nvx_engine_sync", "nvx_engine_wait_ingest", "nvx_engine_host_pushes", "nvx_engine_wait_ingest_of", "nvx_engine_poll_messages", "nvx_engine_try_poll_messages", "nvx_engine_set_message_callback", "nvx_engine_read_y3",
     "nvx_engine_read_bits", "nvx_engine_read_events", "nvx_engine_enable_timing", "nvx_engine_get_stats",
     "nvx_engine_stream", "nvx_engine_get_cascade_spans", "nvx_engine_fence", "nvx_pinned_alloc", "nvx_pinned_free", "nvx_synth_fill_device", "nvx_host_assemble", "nvx_debug_long_tc_band",
-    "nvx_capture_create", "nvx_capture_destroy", "nvx_capture_write", "nvx_capture_pump", "nvx_capture_start", "nvx_capture_stop",
+    "nvx_capture_create", "nvx_capture_create_u8", "nvx_capture_destroy", "nvx_capture_write", "nvx_capture_write_u8", "nvx_capture_pump",
+    "nvx_capture_start", "nvx_capture_stop",
     "nvx_capture_dropped", "nvx_store_create", "nvx_store_destroy", "nvx_store_add", "nvx_store_add_at", "nvx_store_sink",
     "nvx_store_count", "nvx_store_get", "nvx_store_purge", "nvx_store_dump_csv",
 )
@@ -77,7 +79,8 @@ def load_library():
     L.nvx_engine_destroy.argtypes = [C.c_void_p]
     L.nvx_engine_destroy.restype = None
     L.nvx_engine_reset.argtypes = [C.c_void_p]
-    for name in ("nvx_engine_push_host_f32", "nvx_engine_push_host_s16", "nvx_engine_push_device_f32", "nvx_engine_push_device_s16"):
+    for name in ("nvx_engine_push_host_f32", "nvx_engine_push_host_s16", "nvx_engine_push_host_u8", "nvx_engine_push_device_f32",
+                 "nvx_engine_push_device_s16", "nvx_engine_push_device_u8"):
         getattr(L, name).argtypes = [C.c_void_p, C.c_void_p, C.c_longlong]
     L.nvx_engine_sync.argtypes = [C.c_void_p]
     L.nvx_engine_poll_messages.argtypes = [C.c_void_p, C.POINTER(C.POINTER(Message)), C.POINTER(C.c_size_t)]
@@ -101,9 +104,11 @@ def load_library():
     L.nvx_host_assemble.argtypes = [C.c_char_p, C.c_size_t, C.c_int, C.c_int, MESSAGE_CB, C.c_void_p]
     L.nvx_engine_set_message_callback.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     L.nvx_capture_create.argtypes = [C.c_void_p, C.c_int, C.c_longlong, C.c_longlong, C.POINTER(C.c_void_p)]
+    L.nvx_capture_create_u8.argtypes = [C.c_void_p, C.c_int, C.c_longlong, C.c_longlong, C.POINTER(C.c_void_p)]
     L.nvx_capture_destroy.argtypes = [C.c_void_p]
     L.nvx_capture_destroy.restype = None
     L.nvx_capture_write.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_uint]
+    L.nvx_capture_write_u8.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_uint]
     for name in ("nvx_capture_pump", "nvx_capture_dropped"):
         getattr(L, name).restype = C.c_longlong
     L.nvx_capture_pump.argtypes = [C.c_void_p]
@@ -202,20 +207,21 @@ class Engine:
         _check(self.L.nvx_engine_reset(self._h))
 
     def push_host(self, iq: np.ndarray):
-        """iq: [S, n, 2] (or [S, 2n]) float32 or int16, C-contiguous."""
+        """iq: [S, n, 2] (or [S, 2n]) float32, int16 or uint8 (8-bit offset binary, value u - 128), C-contiguous."""
         iq = np.ascontiguousarray(iq)
         n = iq.size // (2 * self.S)
-        fn = {np.dtype(np.float32): self.L.nvx_engine_push_host_f32, np.dtype(np.int16): self.L.nvx_engine_push_host_s16}[iq.dtype]
+        fn = {np.dtype(np.float32): self.L.nvx_engine_push_host_f32, np.dtype(np.int16): self.L.nvx_engine_push_host_s16,
+              np.dtype(np.uint8): self.L.nvx_engine_push_host_u8}[iq.dtype]
         _check(fn(self._h, iq.ctypes.data_as(C.c_void_p), n))
         self.last_n = n
 
-    def push_host_ptr(self, ptr: int, n: int, s16: bool):
-        fn = self.L.nvx_engine_push_host_s16 if s16 else self.L.nvx_engine_push_host_f32
+    def push_host_ptr(self, ptr: int, n: int, s16: bool, u8: bool = False):
+        fn = self.L.nvx_engine_push_host_u8 if u8 else self.L.nvx_engine_push_host_s16 if s16 else self.L.nvx_engine_push_host_f32
         _check(fn(self._h, C.c_void_p(ptr), n))
         self.last_n = n
 
-    def push_device(self, ptr: int, n: int, s16: bool = False):
-        fn = self.L.nvx_engine_push_device_s16 if s16 else self.L.nvx_engine_push_device_f32
+    def push_device(self, ptr: int, n: int, s16: bool = False, u8: bool = False):
+        fn = self.L.nvx_engine_push_device_u8 if u8 else self.L.nvx_engine_push_device_s16 if s16 else self.L.nvx_engine_push_device_f32
         _check(fn(self._h, C.c_void_p(ptr), n))
         self.last_n = n
 
@@ -352,22 +358,31 @@ class Store:
 
 
 class Capture:
-    """SDRplay-format front end: per-stream int16 rings fed by radio callbacks, pumped into the engine in blocks."""
+    """Radio front end: per-stream rings fed by radio callbacks, pumped into the engine in blocks.  fmt="s16": SDRplay-format
+    int16 rings (write); fmt="u8": RTL-SDR 8-bit rings (write_u8)."""
 
-    def __init__(self, eng: "Engine", max_block: int, ring_samples: int):
+    def __init__(self, eng: "Engine", max_block: int, ring_samples: int, fmt: str = "s16"):
         self.L, self.eng = eng.L, eng
         self._h = C.c_void_p()
-        _check(self.L.nvx_capture_create(eng._h, eng.S, max_block, ring_samples, C.byref(self._h)))
+        create = {"s16": self.L.nvx_capture_create, "u8": self.L.nvx_capture_create_u8}[fmt]
+        _check(create(eng._h, eng.S, max_block, ring_samples, C.byref(self._h)))
 
     def write(self, stream: int, xi: np.ndarray, xq: np.ndarray) -> int:
         xi = np.ascontiguousarray(xi, dtype=np.int16)
         xq = np.ascontiguousarray(xq, dtype=np.int16)
         return self.L.nvx_capture_write(self._h, stream, xi.ctypes.data_as(C.c_void_p), xq.ctypes.data_as(C.c_void_p), len(xi))
 
+    def write_u8(self, stream: int, iq: np.ndarray) -> int:
+        """iq: interleaved I,Q bytes ([n, 2] or [2n] uint8), as the rtlsdr_read_async callback hands them over."""
+        iq = np.ascontiguousarray(iq, dtype=np.uint8)
+        return self.L.nvx_capture_write_u8(self._h, stream, iq.ctypes.data_as(C.c_void_p), iq.size // 2)
+
     def pump(self) -> int:
         n = self.L.nvx_capture_pump(self._h)
         if n < 0:
             _check(int(n))
+        if n > 0:
+            self.eng.last_n = int(n)             # read_y3 / read_events of the engine see this block
         return int(n)
 
     def start(self, poll_ms: int = 50):

@@ -157,6 +157,15 @@ def quantise_s16(x: np.ndarray) -> np.ndarray:
     return iq
 
 
+def quantise_u8(x: np.ndarray) -> np.ndarray:
+    """Complex capture -> interleaved unsigned 8-bit offset-binary I,Q (the RTL-SDR's format): rint, + 128, clipped to
+    [0, 255].  The engine reads a byte u as u - 128."""
+    iq = np.empty(2 * len(x), dtype=np.uint8)
+    iq[0::2] = np.clip(np.rint(x.real) + 128, 0, 255).astype(np.uint8)
+    iq[1::2] = np.clip(np.rint(x.imag) + 128, 0, 255).astype(np.uint8)
+    return iq
+
+
 def write_wav(path: str, iq_s16: np.ndarray) -> None:
     """Stereo s16 252 kHz WAV, I = left, Q = right: the format PrepWav would write (capt_sched.c:87-96)."""
     with wave.open(path, "wb") as w:
