@@ -129,7 +129,7 @@ struct nvx_engine {
     cudaStream_t stream_demod = nullptr;  // demod kernels + event download, one block behind
     float2* y3buf[kBuf] = {};
     uint8_t* pickbuf[kBuf] = {};
-    cudaEvent_t casc_done[kBuf] = {}, demod_done[kBuf] = {}, ff_done[kBuf] = {};
+    cudaEvent_t demod_done[kBuf] = {}, ff_done[kBuf] = {};
     long long blocks = 0;
     int last_buf = 0;
     int tap_class = 0;                    // fused-kernel tap-length class (fir_cascade.cuh), -1 = long-tap path
@@ -169,8 +169,6 @@ struct nvx_engine {
     bool ltc_wanted[2] = {false, false};  // the tensor-core kernel was asked for (NVX_LONG_TC mask) for that stage
     nvx::LongStageTaps ltaps[3];          // this engine's long-path taps: passed in the parameter block of every stage launch
     std::vector<int> stream_tag;          // optional [S][2] message tags
-    bool serial = false;                  // NVX_PIPELINE=serial: the next cascade waits for this block's whole demod
-    bool ff_on_main = true;               // feed-forward demod kernels follow the cascade on the main stream
     int target_warps[nvx::kSampleFmts] = {576, 576, 576};   // resident cascade warps per sample format
     nvx::MessageAssembler assembler;
     std::vector<nvx::AssembledMessage> ready, handed;
@@ -230,7 +228,6 @@ int free_engine(nvx_engine* e) {
     for (int k = 0; k < kBuf; ++k) {
         cudaFree(e->y3buf[k]); cudaFree(e->d_events[k]); cudaFree(e->d_ev_count[k]);
         cudaFreeHost(e->h_events[k]); cudaFreeHost(e->h_ev_count[k]);
-        if (e->casc_done[k]) cudaEventDestroy(e->casc_done[k]);
         if (e->demod_done[k]) cudaEventDestroy(e->demod_done[k]);
         if (e->ff_done[k]) cudaEventDestroy(e->ff_done[k]);
         cudaFree(e->pickbuf[k]);
@@ -447,10 +444,6 @@ int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fm
     ca.ch_total = e->C;
     ca.ch0 = 0;
 
-    // this block's FIR output goes into the y3 buffer block (blocks - 3) used -- long drained, see wait_drained above -- whose
-    // last samples the feed-forward kernels of block (blocks - 2) read as their history: when those run on the demod stream
-    // nothing else orders them before this launch
-    if (!e->ff_on_main && e->blocks >= 2) CU_TRY(cudaStreamWaitEvent(e->stream, e->ff_done[(b + 1) % kBuf], 0));
     cudaEvent_t t0 = nullptr, t1 = nullptr, marks[8] = {};
     if (e->timing) {
         const int base = (int)e->ev_used;
@@ -541,8 +534,6 @@ int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fm
     }
     e->tail_cur = nxt;
 
-    CU_TRY(cudaEventRecord(e->casc_done[b], e->stream));
-
     // demod of this block runs on its own stream, overlapping the next block's cascade
     DemodArgs da;
     da.b = e->db;
@@ -556,16 +547,15 @@ int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fm
     da.events = e->d_events[b]; da.ev_count = e->d_ev_count[b]; da.ev_cap = e->ev_cap;
     da.bits = e->d_bits; da.disc = e->d_disc; da.bit_count = e->d_bit_count; da.bit_cap = e->bit_cap;
     // The feed-forward demod kernels are short whole-GPU kernels (0.25 ms of FP64 work per 10 s block of 2048 channels); beside
-    // the cascade (one warp per SM sub-partition, little latency slack) they cost it about what they take alone, so by default
-    // they follow it on the main stream and only the sequential symbol-clock / state-machine kernels (64 warps on the SMs the
-    // cascade grid leaves free) overlap the next block's cascade.  NVX_PIPELINE=overlap moves them to the demod stream too.
-    cudaStream_t s_ff = e->ff_on_main ? e->stream : e->stream_demod;
-    if (!e->ff_on_main) CU_TRY(cudaStreamWaitEvent(e->stream_demod, e->casc_done[b], 0));
-    CU_TRY(demod_launch(da, s_ff, e->stream_demod, e->ff_done[b], e->timing > 1 ? marks : nullptr));
+    // the cascade (one warp per SM sub-partition, little latency slack) they cost it about what they take alone, so they follow
+    // it on the main stream and only the sequential symbol-clock / state-machine kernels (64 warps on the SMs the cascade grid
+    // leaves free) overlap the next block's cascade (the whole chain beside it measured no faster: DESIGN.md §3.3).  The main
+    // stream also orders their look-back into the previous block's y3 buffer before the cascade two blocks on, which
+    // overwrites it.
+    CU_TRY(demod_launch(da, e->stream, e->stream_demod, e->ff_done[b], e->timing > 1 ? marks : nullptr));
     CU_TRY(cudaMemcpyAsync(e->h_ev_count[b], e->d_ev_count[b], sizeof(int) * e->channels, cudaMemcpyDeviceToHost, e->stream_demod));
     CU_TRY(cudaMemcpyAsync(e->h_events[b], e->d_events[b], (size_t)e->channels * e->ev_cap, cudaMemcpyDeviceToHost, e->stream_demod));
     CU_TRY(cudaEventRecord(e->demod_done[b], e->stream_demod));
-    if (e->serial) CU_TRY(cudaStreamWaitEvent(e->stream, e->demod_done[b], 0));
     // the next block's cascade may overwrite neither this block's input staging nor (two blocks on) its y3
     // buffer before the demod has consumed them: the staging buffers are only touched on e->stream (ordered),
     // the y3 buffer is protected by the demod_done wait above
@@ -713,17 +703,8 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
             CREATE_TRY(cudaEventCreateWithFlags(&e->stage_free[k], cudaEventDisableTiming));
         }
         CREATE_TRY(cudaStreamCreateWithPriority(&e->stream_demod, cudaStreamNonBlocking, hi));
-        // tuning knob NVX_PIPELINE: default "main" = the feed-forward demod kernels follow the cascade on the main stream and only
-        // the sequential kernels run beside the next cascade; "overlap" = the whole demod chain of block i runs on the demod
-        // stream beside the cascade of block i + 1 (A/B on one box, 30 steps each, twice: 3.81 / 3.84 ms per step against 3.86 /
-        // 3.81 -- no difference beyond the noise, while the cascade itself slows from 3.48 to 3.71 ms); "serial" = the next
-        // cascade waits for the whole demod
-        const char* mode = getenv("NVX_PIPELINE");
-        e->serial = mode && !strcmp(mode, "serial");
-        e->ff_on_main = !(mode && !strcmp(mode, "overlap"));
     }
     for (int k = 0; k < kBuf; ++k) {
-        CREATE_TRY(cudaEventCreateWithFlags(&e->casc_done[k], cudaEventDisableTiming));
         CREATE_TRY(cudaEventCreateWithFlags(&e->demod_done[k], cudaEventDisableTiming));
         CREATE_TRY(cudaEventCreateWithFlags(&e->ff_done[k], cudaEventDisableTiming));
     }

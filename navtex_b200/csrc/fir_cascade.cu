@@ -102,11 +102,7 @@ __global__ void __launch_bounds__(InFmt<kFmt, kClass, kCh>::kWarps * 32, kCtasPe
     for (int t = 0; t < warp_stages; ++t) {
         mbar_wait(bar0 + 8 * stage, parity);
         const uint8_t* rowb = wbase + stage * kStageBytes + lane * kRowBytes;
-#ifdef NVX_ROLL_STEPS
-#pragma unroll 1
-#else
 #pragma unroll
-#endif
         for (int u = 0; u < kStepsPerStage; ++u) {
             if (kGenNco) {
 #pragma unroll

@@ -54,8 +54,6 @@
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
-#include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <vector>
@@ -76,8 +74,6 @@ constexpr int kLoaderWarp0 = kConvWarps + 2;
 constexpr int kLoaderWarps = 2;
 constexpr int kEpiWarp0 = kLoaderWarp0 + kLoaderWarps;
 constexpr int kTcThreads = 32 * (kConvWarps + 2 + kLoaderWarps + 4);
-// streaming kernel: 4 kCW converter warps (kCW per TMEM lane quarter) + issuer + TMA + loaders + 4 epilogue warps
-__host__ __device__ constexpr int tcs_threads(int kCW) { return 32 * (4 * kCW + 2 + kLoaderWarps + 4); }
 constexpr int kSlotBytes = kRows * 128;    // one raw-input slot: [128 rows x 128 B]
 constexpr int kMaxSlots = 8;
 constexpr int kDumpPad = 4;                // epilogue dump: [128 rows][2 NP + 4] floats (row pitch = 4 words mod 32: conflict-free)
@@ -105,8 +101,6 @@ struct TcArgs {
     int rows, s16, T, H, chunks, J, slots, box_rows, mix;
     int rows_src;                          // rows of the input: rows, or rows / 2 stream rows when the stage mixes on load
     int cpt, lead;                         // streaming kernel: chunks per tile advance (D N / chunk samples), chunks a window leads its tile by
-    long long* trace;                      // development aid (NVX_TC_TRACE): clock64 stamps of CTA 0's first chunks, else null
-    int dbg;                               // development aid (NVX_TC_DBG bit mask): leave parts of the pipeline out to find the limiter (results are garbage)
     long long tiles_per_block;             // output tiles per row block
     long long work;                        // row blocks * tiles_per_block
     float2 nco_tab[kNcoPeriod + 16];       // (cos, -sin)(2 pi k 14000 / 63000), fir2cpp.C:104-107, continued periodically (mix on load)
@@ -144,12 +138,6 @@ __device__ __forceinline__ void tmem_st16(uint32_t taddr, const float (&v)[16]) 
     asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
                  ::"r"(taddr), "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7]), "f"(v[8]), "f"(v[9]),
                    "f"(v[10]), "f"(v[11]), "f"(v[12]), "f"(v[13]), "f"(v[14]), "f"(v[15]) : "memory");
-}
-
-__device__ __forceinline__ void tmem_st(uint32_t taddr, const float (&v)[16]) { tmem_st16(taddr, v); }
-__device__ __forceinline__ void tmem_st(uint32_t taddr, const float (&v)[8]) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};"
-                 ::"r"(taddr), "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7]) : "memory");
 }
 
 // general loader for tiles that touch the carried history
@@ -377,7 +365,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) fir_tc_kernel(const __grid_cons
                 const int n_lo = num <= 0 ? 0 : (num + D - 1) / D;
                 int n_hi = (kCS * c + kCS - 1) / D;
                 n_hi = n_hi > N - 1 ? N - 1 : n_hi;
-                const bool trim = !(a.dbg & 16) && n_lo <= n_hi;
+                const bool trim = n_lo <= n_hi;
                 const uint32_t c_off = trim ? ((uint32_t)n_lo & ~15u) : 0u;
                 const uint32_t np = trim ? (((uint32_t)n_hi | 15u) + 1u) - c_off : (uint32_t)N;
                 const uint32_t idesc_np = (idesc & ~(0x3Fu << 17)) | ((np >> 3) << 17);
@@ -573,11 +561,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) fir_tc_kernel(const __grid_cons
 // converters refill the other A set, so two A sets are enough.  Everything else -- band matrix, descriptors, 3xTF32 split, slot
 // ring, TMA / cp.async alternation, epilogue phases -- is as in fir_tc_kernel.
 constexpr int kSN = 64;                    // outputs per tile of the streaming kernel
-constexpr int kTraceChunks = 96, kTraceCols = 8;
-#define NVX_TRACE(col, idx)                                                                                   \
-    do {                                                                                                      \
-        if (a.trace && blockIdx.x == 0 && (idx) < kTraceChunks && lane == 0) a.trace[(idx) * kTraceCols + (col)] = clock64(); \
-    } while (0)
 
 // L = live tiles = accumulator slots: 2 while a window spans at most two tiles (lead <= cpt: two A sets), 3 up to three tiles
 // (cpt < lead <= 2 cpt, i.e. up to 516 taps at D = 4: the third slot takes the place of the second A set, so conversion and MMAs
@@ -587,7 +570,7 @@ constexpr int kTraceChunks = 96, kTraceCols = 8;
 // rotate every sample by its channel's NCO phase (fir2cpp.C:112-128: "518" by (cos, -sin), "490" by the conjugate) before the
 // TF32 split -- the same two FP32 operations per component as the stage-1 epilogue's mix, so the products are bit-identical,
 // while y1 crosses HBM once per stream instead of once per channel on both sides.
-// kCW: converter warps per TMEM lane quarter, each converting 32 / kCW samples of a chunk per row.  Two is what ships.  The
+// Converters: two warps per TMEM lane quarter, each converting 16 samples of a chunk per row, as in fir_tc_kernel.  The
 // converters are a latency-bound chain of ~300 instructions per chunk and warp and set the chunk period of stage 2 (in-kernel
 // trace, 65 taps: 1 470 cycles per chunk against 963 with conversion, loads and epilogue knocked out), so four per quarter were
 // built and measured: 24 warps per CTA cap the kernel at 80 registers per thread, every role spills, and the whole chain is
@@ -601,11 +584,10 @@ constexpr int kTraceChunks = 96, kTraceCols = 8;
 // hand-overs has two chunk periods to complete) -- correct only with two A sets and an even number of chunks in the ring (a parity
 // wait cannot tell phase k from phase k + 2), and slower where it applies (65 taps: 328 -> 319 Gsamples/s): the converters are
 // bound by their instruction throughput, not by the latency of the hand-overs.
-template <int D, int L, bool kMixIn = false, int kCW = 2>
-__global__ void __launch_bounds__(tcs_threads(kCW), 1) fir_tcs_kernel(const __grid_constant__ TcArgs a) {
+template <int D, int L, bool kMixIn = false>
+__global__ void __launch_bounds__(kTcThreads, 1) fir_tcs_kernel(const __grid_constant__ TcArgs a) {
     constexpr int N = kSN;
-    constexpr int kConvWarps = 4 * kCW, kIssuerWarp = kConvWarps, kTmaWarp = kConvWarps + 1, kLoaderWarp0 = kConvWarps + 2;
-    constexpr int kPer = kKB / kCW;                          // samples (A columns) per converter thread and chunk
+    constexpr int kPer = kKB / 2;                            // samples (A columns) per converter thread and chunk
     constexpr int kInRows = kMixIn ? kRows / 2 : kRows;      // input rows per row block
     static_assert(!kMixIn || chunk_samples(D) % kNcoPeriod == 1, "mix on load: a chunk advances the NCO phase index by one");
     constexpr int kCS = chunk_samples(D);
@@ -685,7 +667,7 @@ __global__ void __launch_bounds__(tcs_threads(kCW), 1) fir_tcs_kernel(const __gr
                     odd ^= 1;
                     if (++ring_at == ring_chunks) { ring_at = 0; ring_ph ^= 1; }
                     if (!mine) continue;
-                    const bool fast = G >= 0 && !(a.dbg & 1);   // chunks before the block come from the carried history
+                    const bool fast = G >= 0;       // chunks before the block come from the carried history
                     if (kMixIn) {
                         const uint32_t full = bar0 + 8 * (kBarRawFull + slot);
                         bar_wait(bar0 + 8 * (kBarRawEmpty + slot), ph ^ 1);
@@ -739,7 +721,7 @@ __global__ void __launch_bounds__(tcs_threads(kCW), 1) fir_tcs_kernel(const __gr
                 if (!mine) continue;
                 bar_wait(bar0 + 8 * (kBarRawEmpty + slot), ph ^ 1);
                 if (slots_per_chunk == 2) bar_wait(bar0 + 8 * (kBarRawEmpty + slot + 1), ph ^ 1);
-                if (G >= 0 && !(a.dbg & 1)) {
+                if (G >= 0) {
                     const long long t = G * kCS + u16 * per_piece;
                     const bool t_ok = t + per_piece <= a.n_in && u16 * per_piece < kCS;
                     const uint8_t* src = static_cast<const uint8_t*>(a.in) + ((size_t)(rb * kInRows + r0) * a.in_pitch + t) * esz;
@@ -774,7 +756,6 @@ __global__ void __launch_bounds__(tcs_threads(kCW), 1) fir_tcs_kernel(const __gr
         const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(kRows >> 4) << 24);
         bar_wait(bar0 + 8 * kBarG, 0);
         uint32_t s = 0, ph = 0;
-        int gi = 0;
         int q0 = 0;                                         // tiles of the segments already done (32-bit: a CTA walks < 2^31 tiles)
         uint64_t dh0[kKB / kUmmaK], dl0[kKB / kUmmaK];      // band descriptors at offset 0, one per k-step
 #pragma unroll
@@ -791,7 +772,6 @@ __global__ void __launch_bounds__(tcs_threads(kCW), 1) fir_tcs_kernel(const __gr
         // instructions instead of 64: 37 % less tensor work at 255 taps, more for shorter filters.  The first MMA of a tile still
         // spans all 64 columns: it is the one that clears them (its chunk has column offset 0 anyway).
         struct Plan { uint32_t valid, c, slot, wait_par, d_off, idesc_np; uint64_t dadd; };
-        const bool trim = !(a.dbg & 16);
         auto plan = [&](int r, int t1, int which, int q0_, int n_tiles) {
             Plan p;
             const int t = t1 + which;
@@ -808,8 +788,8 @@ __global__ void __launch_bounds__(tcs_threads(kCW), 1) fir_tcs_kernel(const __gr
             int n_lo = kOpc * (c - lead), n_hi = kOpc * c + kOpc - 1;
             n_lo = n_lo < 0 ? 0 : n_lo;
             n_hi = n_hi > N - 1 ? N - 1 : n_hi;
-            const uint32_t off = trim ? ((uint32_t)n_lo & ~15u) : 0u;
-            const uint32_t np = trim ? (((uint32_t)n_hi | 15u) + 1u) - off : (uint32_t)N;
+            const uint32_t off = (uint32_t)n_lo & ~15u;
+            const uint32_t np = (((uint32_t)n_hi | 15u) + 1u) - off;
             p.d_off = p.slot * kSlotCols + off;
             p.idesc_np = (idesc & ~(0x3Fu << 17)) | ((np >> 3) << 17);
             p.dadd = (goff >> 4) + (uint64_t)off * 8;           // 16 rows of the band = two 1024-byte atoms
@@ -848,9 +828,8 @@ __global__ void __launch_bounds__(tcs_threads(kCW), 1) fir_tcs_kernel(const __gr
             Plan pl[L];
 #pragma unroll
             for (int w = 0; w < L; ++w) pl[w] = plan(r, t1, w, q0, n_tiles);
-            for (int j = 0; j < n_chunks; ++j, ++gi) {
+            for (int j = 0; j < n_chunks; ++j) {
                 bar_wait(bar0 + 8 * (kBarAFull + s), ph);
-                NVX_TRACE(0, gi);
                 asm volatile("tcgen05.fence::after_thread_sync;");
                 const uint32_t at = tmem + kACol0 + s * kSetCols;
                 if (pl[0].valid) issue(pl[0], at);
@@ -863,7 +842,6 @@ __global__ void __launch_bounds__(tcs_threads(kCW), 1) fir_tcs_kernel(const __gr
                 for (int w = 1; w < L; ++w)
                     if (pl[w].valid) issue(pl[w], at);
                 if (leader) umma_commit(bar0 + 8 * (kBarAEmpty + s));
-                NVX_TRACE(1, gi);
                 if (++s == kSets) { s = 0; ph ^= 1; }
                 r = r2; t1 = t2;
 #pragma unroll
@@ -875,13 +853,12 @@ __global__ void __launch_bounds__(tcs_threads(kCW), 1) fir_tcs_kernel(const __gr
         const int q = warp & 3, kh = warp >> 2;              // TMEM lane quarter, column group of the chunk
         const int r = q * 32 + lane;
         const uint32_t lane_base = tmem + ((uint32_t)(q * 32) << 16) + kACol0 + kh * kPer;
-        // where this thread's kPer samples sit: float2 input = two 128-byte pieces of 16 samples per row (two slots, or -- mix on
-        // load -- two halves of one slot), int16 input = one piece of 32 samples
-        const int piece = a.s16 ? 0 : (kh * kPer) / 16;
-        const int in_piece = a.s16 ? kh * kPer : (kh * kPer) % 16;     // first sample inside the piece
+        // where this thread's kPer samples sit: float2 input = piece kh of two 128-byte pieces of 16 samples per row (two slots,
+        // or -- mix on load -- two halves of one slot), int16 input = half kh of one piece of 32 samples
+        const int piece = a.s16 ? 0 : kh;
+        const int in_piece = a.s16 ? kh * kPer : 0;         // first sample inside the piece
         int slot = kMixIn ? 0 : piece;
         uint32_t sph = 0, s = 0, ph = 0;
-        int gi = 0;
         const int r_in = r & (kInRows - 1);                  // this thread's input row inside the row block
         const bool conj = kMixIn && q >= 2;                  // mix on load: rows 64..127 are the "490" channel (conjugate rotation)
         NVX_FOR_SEGMENTS({
@@ -892,15 +869,11 @@ __global__ void __launch_bounds__(tcs_threads(kCW), 1) fir_tcs_kernel(const __gr
                 const long long t0 = (a.k_abs + (cpt * ta - lead) * kCS + kh * kPer) % kNcoPeriod;
                 p9 = (int)(t0 < 0 ? t0 + kNcoPeriod : t0);
             }
-            for (long long G = cpt * ta - lead; G < cpt * tb; ++G, ++gi) {
+            for (long long G = cpt * ta - lead; G < cpt * tb; ++G) {
                 bar_wait(bar0 + 8 * (kBarRawFull + slot), sph);
-                if (warp == 0) NVX_TRACE(2, gi);
                 const uint8_t* row = s_raw + slot * kSlotBytes + (kMixIn ? piece * kHalfBytes : 0) + r_in * 128;
                 float ih[kPer], il[kPer], qh[kPer], ql[kPer];
-                if (a.dbg & 2) {
-#pragma unroll
-                    for (int j = 0; j < kPer; ++j) ih[j] = il[j] = qh[j] = ql[j] = (float)gi;
-                } else if (G >= 0) {
+                if (G >= 0) {
                     if (a.s16) {
 #pragma unroll
                         for (int u = 0; u < kPer / 4; ++u) {
@@ -941,22 +914,17 @@ __global__ void __launch_bounds__(tcs_threads(kCW), 1) fir_tcs_kernel(const __gr
                 if (kMixIn && ++p9 == kNcoPeriod) p9 = 0;
                 __syncwarp();
                 if (lane == 0) bar_arrive(bar0 + 8 * (kBarRawEmpty + slot));
-                if (warp == 0) NVX_TRACE(3, gi);
                 bar_wait(bar0 + 8 * (kBarAEmpty + s), ph ^ 1);
-                if (warp == 0) NVX_TRACE(4, gi);
                 asm volatile("tcgen05.fence::after_thread_sync;");
                 const uint32_t col = lane_base + s * kSetCols;
-                if (!(a.dbg & 4)) {
-                    tmem_st(col + 0 * 32, ih);
-                    tmem_st(col + 1 * 32, il);
-                    tmem_st(col + 2 * 32, qh);
-                    tmem_st(col + 3 * 32, ql);
-                    asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-                }
+                tmem_st16(col + 0 * 32, ih);
+                tmem_st16(col + 1 * 32, il);
+                tmem_st16(col + 2 * 32, qh);
+                tmem_st16(col + 3 * 32, ql);
+                asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
                 asm volatile("tcgen05.fence::before_thread_sync;");
                 __syncwarp();
                 if (lane == 0) bar_arrive(bar0 + 8 * (kBarAFull + s));
-                if (warp == 0) NVX_TRACE(5, gi);
                 if (++s == kSets) { s = 0; ph ^= 1; }
                 slot += slots_per_chunk;
                 if (slot >= a.slots) { slot -= a.slots; sph ^= 1; }
@@ -975,19 +943,12 @@ __global__ void __launch_bounds__(tcs_threads(kCW), 1) fir_tcs_kernel(const __gr
                 const long long n0 = t * N;
                 const uint32_t taddr = tmem + ((uint32_t)(q * 32) << 16) + slot * kSlotCols;
                 bar_wait(bar0 + 8 * (kBarTile + slot), (uint32_t)((tq / L) & 1));
-                if (q == 0) NVX_TRACE(6, tq);
                 asm volatile("tcgen05.fence::after_thread_sync;");
                 // mix on load: this warp's 32 rows are the streams rb 64 + (q & 1) 32 .. of channel q >> 1; output rows are
                 // channel rows, 2 stream + channel
                 const int row0 = kMixIn ? rb * kInRows + (q & 1) * 32 : rb * kRows + q * 32;
                 const int rows_left = (kMixIn ? a.rows_src : a.rows) - row0;
                 const int r_max = rows_left < 32 ? rows_left : 32;
-                if (a.dbg & 8) {
-                    asm volatile("tcgen05.fence::before_thread_sync;");
-                    __syncwarp();
-                    if (lane == 0) bar_arrive(bar0 + 8 * (kBarTmemFree + slot));
-                    continue;
-                }
 #pragma unroll 1
                 for (int pass = 0; pass < N / NP; ++pass) {
                     if (pass) __syncwarp();
@@ -1003,7 +964,6 @@ __global__ void __launch_bounds__(tcs_threads(kCW), 1) fir_tcs_kernel(const __gr
                     if (pass == N / NP - 1) asm volatile("tcgen05.fence::before_thread_sync;");
                     __syncwarp();
                     if (pass == N / NP - 1 && lane == 0) bar_arrive(bar0 + 8 * (kBarTmemFree + slot));
-                    if (pass == N / NP - 1 && q == 0) NVX_TRACE(7, tq);
 #pragma unroll 1
                     for (int h = 0; h < NP / 32; ++h) {
                         const int m = h * 32 + lane;
@@ -1093,20 +1053,15 @@ int tc_slots(int D, int N, int T, int L = 2) {        // raw-input slots that fi
     return 0;
 }
 
-template <int D, int L, bool kMixIn, int kCW>
-cudaError_t launch_tcs_w(TcArgs& a, int sms, cudaStream_t stream) {
-    a.slots = tc_slots(D, kSN, a.T, L);
-    const size_t smem = tc_smem(D, kSN, a.T, a.slots, L);
-    cudaError_t e = cudaFuncSetAttribute(fir_tcs_kernel<D, L, kMixIn, kCW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    const long long grid = a.work < sms ? a.work : sms;
-    fir_tcs_kernel<D, L, kMixIn, kCW><<<(unsigned)grid, tcs_threads(kCW), smem, stream>>>(a);
-    return cudaGetLastError();
-}
-
 template <int D, int L, bool kMixIn = false>
 cudaError_t launch_tcs(TcArgs& a, int sms, cudaStream_t stream) {
-    return launch_tcs_w<D, L, kMixIn, 2>(a, sms, stream);
+    a.slots = tc_slots(D, kSN, a.T, L);
+    const size_t smem = tc_smem(D, kSN, a.T, a.slots, L);
+    cudaError_t e = cudaFuncSetAttribute(fir_tcs_kernel<D, L, kMixIn>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    const long long grid = a.work < sms ? a.work : sms;
+    fir_tcs_kernel<D, L, kMixIn><<<(unsigned)grid, kTcThreads, smem, stream>>>(a);
+    return cudaGetLastError();
 }
 
 template <int D, int N>
@@ -1128,22 +1083,17 @@ int long_tc_tile(int D, int T) {
     // measured with the data operand in tensor memory (tools/probes/umma_ts_probe.cu): 23 / 36 / 64 cycles per tcgen05.mma at
     // N = 32 / 64 / 128, i.e. 211 / 218 / 288 cycles per output column at 255 taps; N = 64 halves the re-read of N = 32.  N = 128
     // (stage 1 only: 1.5x instead of 2x re-read, but two A sets and a two-pass epilogue) wins from ~400 taps on: 511 taps 131
-    // against 122 Gsamples/s, 255 taps 183 against 190
-    int want = getenv("NVX_TC_N") ? atoi(getenv("NVX_TC_N")) : (D == NVX_D1 && T >= 384 ? 128 : 64);
-    for (int N : {128, 64, 32})
-        // stage 2 only with N = 64 (fits up to 959 taps): with N = 32 tiles the CUDA-core kernel is faster
-        if (N <= want && (D == NVX_D1 || N == 64) && tc_slots(D, N, T)) return N;
-    return 0;
+    // against 122 Gsamples/s, 255 taps 183 against 190.  No N = 32 kernel: at stage 1, N = 64 fits every tap count up to
+    // kLongMaxTaps; stage 2 takes N = 64 only (fits up to 959 taps): with N = 32 tiles the CUDA-core kernel is faster
+    if (D == NVX_D1 && T >= 384 && tc_slots(D, 128, T)) return 128;
+    return tc_slots(D, 64, T) ? 64 : 0;
 }
 
-// the streaming kernel serves a stage when a window spans at most three tiles (lead <= 2 x chunks per tile) and its band fits;
-// NVX_TC_STREAM=0 keeps the tile-at-a-time kernel (A/B measurements)
+// the streaming kernel serves a stage when a window spans at most three tiles (lead <= 2 x chunks per tile) and its band fits
 bool tcs_applies(int D, int T_taps) {
     if (D != NVX_D1 && D != NVX_D2) return false;
-    if (getenv("NVX_TC_STREAM") && atoi(getenv("NVX_TC_STREAM")) == 0) return false;
     const int lead = tcs_lead(D, T_taps);
-    const int max_lead = (getenv("NVX_TC_LIVE") && atoi(getenv("NVX_TC_LIVE")) == 2 ? 1 : 2) * tcs_cpt(D);      // two or three live tiles
-    return lead <= max_lead && tc_slots(D, kSN, D + lead * chunk_samples(D), lead > tcs_cpt(D) ? 3 : 2) > 0;
+    return lead <= 2 * tcs_cpt(D) && tc_slots(D, kSN, D + lead * chunk_samples(D), lead > tcs_cpt(D) ? 3 : 2) > 0;
 }
 
 struct LongTcStage {
@@ -1278,39 +1228,16 @@ cudaError_t long_tc_launch(const LongTcStage* s, const LongArgs& la, const LongS
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     if (s->streaming) {
-        static long long* d_trace = nullptr;
-        static int traced = 0;
-        const char* tr = getenv("NVX_TC_TRACE");       // development aid: NVX_TC_TRACE=<decimation> dumps CTA 0's timeline of one launch to stderr
-        const bool want = tr && atoi(tr) == s->D && traced < 3;
-        if (want && !d_trace) cudaMalloc(&d_trace, sizeof(long long) * kTraceChunks * kTraceCols);
-        if (want) { cudaMemsetAsync(d_trace, 0, sizeof(long long) * kTraceChunks * kTraceCols, stream); a.trace = d_trace; }
-        a.dbg = (tr && getenv("NVX_TC_DBG")) ? atoi(getenv("NVX_TC_DBG")) : 0;      // knock-out experiments: only together with the trace
-        if (getenv("NVX_TC_TRIM") && atoi(getenv("NVX_TC_TRIM")) == 0) a.dbg |= 16;  // A/B: full-width MMAs for every chunk (same results)
         const bool three = a.lead > a.cpt;
-        const cudaError_t e = s->D == NVX_D1 ? (three ? launch_tcs<NVX_D1, 3>(a, sms, stream) : launch_tcs<NVX_D1, 2>(a, sms, stream))
-                              : la.mix_in    ? (three ? launch_tcs<NVX_D2, 3, true>(a, sms, stream) : launch_tcs<NVX_D2, 2, true>(a, sms, stream))
-                                             : (three ? launch_tcs<NVX_D2, 3>(a, sms, stream) : launch_tcs<NVX_D2, 2>(a, sms, stream));
-        if (want && e == cudaSuccess && ++traced == 3) {
-            static long long h[kTraceChunks * kTraceCols];
-            cudaStreamSynchronize(stream);
-            cudaMemcpy(h, d_trace, sizeof h, cudaMemcpyDeviceToHost);
-            fprintf(stderr, "# tcs trace D=%d: chunk  AFull_seen issued | raw_full converted AEmpty_seen AFull_arrived | tile_done tmem_freed (cycles since first stamp)\n", s->D);
-            long long t0 = h[2];
-            fprintf(stderr, "# dbg=%d: cycles per chunk over chunks 24..88 = %.0f\n", a.dbg, (double)(h[88 * kTraceCols + 1] - h[24 * kTraceCols + 1]) / 64.0);
-            if (!getenv("NVX_TC_TRACE_FULL")) return e;
-            for (int k = 0; k < kTraceChunks; ++k) {
-                fprintf(stderr, "%3d", k);
-                for (int c = 0; c < kTraceCols; ++c) fprintf(stderr, " %8lld", h[k * kTraceCols + c] ? h[k * kTraceCols + c] - t0 : -1);
-                fprintf(stderr, "\n");
-            }
-        }
-        return e;
+        return s->D == NVX_D1 ? (three ? launch_tcs<NVX_D1, 3>(a, sms, stream) : launch_tcs<NVX_D1, 2>(a, sms, stream))
+               : la.mix_in    ? (three ? launch_tcs<NVX_D2, 3, true>(a, sms, stream) : launch_tcs<NVX_D2, 2, true>(a, sms, stream))
+                              : (three ? launch_tcs<NVX_D2, 3>(a, sms, stream) : launch_tcs<NVX_D2, 2>(a, sms, stream));
     }
-    if (getenv("NVX_TC_TRIM") && atoi(getenv("NVX_TC_TRIM")) == 0) a.dbg |= 16;
-    if (s->D == NVX_D1)
-        return s->N == 128 ? launch_tc<NVX_D1, 128>(a, sms, stream)
-                           : s->N == 64 ? launch_tc<NVX_D1, 64>(a, sms, stream) : launch_tc<NVX_D1, 32>(a, sms, stream);
-    return s->N == 64 ? launch_tc<NVX_D2, 64>(a, sms, stream) : launch_tc<NVX_D2, 32>(a, sms, stream);
+    // the tile widths long_tc_tile picks
+    if (s->D == NVX_D1 && s->N == 128) return launch_tc<NVX_D1, 128>(a, sms, stream);
+    if (s->D == NVX_D1 && s->N == 64) return launch_tc<NVX_D1, 64>(a, sms, stream);
+    if (s->D == NVX_D2 && s->N == 64) return launch_tc<NVX_D2, 64>(a, sms, stream);
+    return cudaErrorInvalidValue;
 }
 
 }  // namespace nvx

@@ -67,3 +67,18 @@ def test_band_is_refused_where_the_kernel_does_not_apply():
     assert geo["n_tile"] == 64 and geo["taps_padded"] == 259 and geo["chunks"] == 25      # streaming: 16 + 9 chunks of 28 samples
     geo, _, _ = engine.long_tc_band(7, np.ones(959))
     assert geo["n_tile"] == 64 and geo["copies"] == 2
+
+
+def test_every_tap_count_lands_on_a_built_tile_width():
+    # the tile-at-a-time kernel is only instantiated for N = 128 and 64 at D = 4 and N = 64 at D = 7 (the streaming kernel's
+    # N is 64 too): every tap count the engine accepts, 1 .. 1024 per stage, must map to one of those or be refused
+    for T in range(1, 1025):
+        h = np.ones(T)
+        geo, _, _ = engine.long_tc_band(4, h)
+        assert geo["n_tile"] == (128 if 517 <= T <= 548 else 64), (T, geo)
+        if T >= 960:
+            with pytest.raises(engine.NvxError):
+                engine.long_tc_band(7, h)
+        else:
+            geo, _, _ = engine.long_tc_band(7, h)
+            assert geo["n_tile"] == 64, (T, geo)

@@ -2,8 +2,3 @@
 python -m pytest tests -m gpu -x -q 2>&1 | tail -3
 python bench.py --steps 30 --warmup 3 > gpurun_out/bench8.json 2> gpurun_out/bench8.err; tail -3 gpurun_out/bench8.err
 python bench.py --workload config4 --seconds 60 > gpurun_out/bench8_config4.json 2> gpurun_out/bench8_config4.err; tail -3 gpurun_out/bench8_config4.err
-for v in "" roll "" roll; do
-  if [ -z "$v" ]; then unset NVX_LIB; else export NVX_LIB=$PWD/navtex_b200/variants/libnavtex_b200_$v.so; fi
-  echo "== variant '$v' f32"
-  python tools/quick_perf.py --steps 30 --timing 1 2>&1 | tail -3 | grep -v stages
-done
