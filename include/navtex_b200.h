@@ -57,7 +57,9 @@ typedef struct {
      * 1024 per stage, e.g. the 255-tap stress designs) take the long-tap path: one register-tiled FIR kernel per stage,
      * intermediates in HBM.
      * Tap sets are per engine (they travel in the kernel parameter block of every launch): engines with different
-     * filters can be alive on one device at the same time */
+     * filters can be alive on one device at the same time.
+     * Tap order: h[0] weighs the newest sample: y[k] = sum_i h[i] x[D (k + 1) - 1 - i] (D = 4, 7, 10 for h1, h2, h3; the
+     * order matters for asymmetric filters, e.g. minimum-phase designs) */
     const double *h1, *h2, *h3;
     int keep_bits;              /* record 'B'/'Y' decisions and discriminator sums for nvx_engine_read_bits */
     int first_stream_id;        /* global id of stream 0 (multi-GPU sharding; only used to label messages) */
