@@ -10,7 +10,6 @@
 #include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <condition_variable>
@@ -24,15 +23,6 @@
 #include "fir_cascade.cuh"
 #include "fir_long.cuh"
 #include "message_assembler.h"
-
-namespace nvx {
-int cascade_box_elems(SampleFmt f);
-int cascade_tap_class(int n1, int n2, int n3);
-int cascade_warm_super(int tap_class);
-void cascade_fill_taps(int tap_class, const double* h1, int n1, const double* h2, int n2, const double* h3, int n3, CascadeTaps* out);
-cudaError_t cascade_launch(const CascadeArgs& a, const CascadeTaps& taps, int tap_class, bool custom_taps, SampleFmt f, int n_ch, cudaStream_t stream);
-int cascade_target_warps(int device, int reserved_sms, SampleFmt f, int tap_class, bool heavy);
-}  // namespace nvx
 
 namespace {
 
@@ -100,23 +90,6 @@ __global__ void tail_carry_kernel(const Sample* __restrict__ old_tail, const Sam
     *reinterpret_cast<int4*>(new_tail + (size_t)s * halo + k) = *src;
 }
 
-// long-tap path, 8-bit input: out = (u - 128) as short2, 8 samples (16 bytes in, 32 out) per thread; count = S n, a multiple of 280
-__global__ void widen_u8_kernel(const uchar2* __restrict__ in, short2* __restrict__ out, long long count) {
-    const long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 8;
-    if (i >= count) return;
-    const int4 v = *reinterpret_cast<const int4*>(in + i);
-    const unsigned w[4] = {(unsigned)v.x, (unsigned)v.y, (unsigned)v.z, (unsigned)v.w};
-    int o[8];
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {       // bytes I0 Q0 I1 Q1 of a word -> two short2 words
-        o[2 * k] = (int)(((w[k] & 0xFFu) - 128u) & 0xFFFFu) | (int)(((((w[k] >> 8) & 0xFFu) - 128u) & 0xFFFFu) << 16);
-        o[2 * k + 1] = (int)((((w[k] >> 16) & 0xFFu) - 128u) & 0xFFFFu) | (int)((((w[k] >> 24) - 128u) & 0xFFFFu) << 16);
-    }
-    int4* dst = reinterpret_cast<int4*>(out + i);
-    dst[0] = make_int4(o[0], o[1], o[2], o[3]);
-    dst[1] = make_int4(o[4], o[5], o[6], o[7]);
-}
-
 }  // namespace
 
 constexpr int kBuf = 3;   // blocks in flight: cascade of block i+1/i+2 overlaps demod + event download of block i
@@ -134,12 +107,12 @@ struct nvx_engine {
     int last_buf = 0;
     int tap_class = 0;                    // fused-kernel tap-length class (fir_cascade.cuh), -1 = long-tap path
     int halo = 1960;                      // carried input samples per stream: 280 x the class's warm-up superblocks
-    // carried input tail, ping-pong, in the sample format being pushed: [S][halo] float2, short2 or 8-bit pairs
-    void* tail[nvx::kSampleFmts][2] = {};                            // [format][ping-pong]
-    CUtensorMap map_tail[nvx::kSampleFmts][2];
+    // fused path: carried input tail, ping-pong, in the sample format being pushed: [S][halo] float2, short2 or 8-bit pairs
+    // (each buffer sized for float2); filled with silence and described to the TMA unit when the first push fixes the format
+    void* tail[2] = {};
+    CUtensorMap map_tail[2];
     int tail_cur = 0;
     int fmt = -1;                         // -1 = nothing pushed since create/reset, else the nvx::SampleFmt of the pushes
-    short2* u8_wide = nullptr;            // long-tap path, 8-bit input: [S][max_block] short2 (u - 128), allocated on first use
     nvx::DemodBuffers db = {};
     double* corrbuf[2] = {nullptr, nullptr};   // |mask correlation| rows, alternating per block (each block reads its history from the other)
     uint8_t* d_events[kBuf] = {}; int* d_ev_count[kBuf] = {}; int ev_cap = 0;
@@ -156,18 +129,8 @@ struct nvx_engine {
     int last_P = 0;
     bool custom_taps = false;
     nvx::CascadeTaps taps;                // this engine's filter constants: passed in the parameter block of every cascade launch
-    nvx::NcoParam* d_nco = nullptr;       // per-stream NCO parameters, two-channel layout of the long-tap path, else null
-    nvx::NcoChan* d_nco_ch = nullptr;     // per (stream, channel) NCO parameters of the fused kernel's general-NCO variants, else null
-    // long-tap path (tap counts other than 37 / 47 / 71): per-stage kernels, intermediates and histories in HBM
-    bool long_taps = false;
-    nvx::LongStage lst[3];
-    float2* lhist[3][2] = {};             // [stage][ping-pong]: [rows][H]
-    float2 *y1buf = nullptr, *y2buf = nullptr;
-    int lcur = 0;
-    nvx::LongTcStage* ltc[2] = {nullptr, nullptr};   // tensor-core variants of stages 1 and 2 (null: CUDA-core kernel)
-    bool mix_on_load = false;             // long path, reference NCO table, streaming tensor-core stage 2: stage 1 writes ONE un-mixed row per stream
-    bool ltc_wanted[2] = {false, false};  // the tensor-core kernel was asked for (NVX_LONG_TC mask) for that stage
-    nvx::LongStageTaps ltaps[3];          // this engine's long-path taps: passed in the parameter block of every stage launch
+    nvx::NcoChan* d_nco_ch = nullptr;     // [S][C] per-stream NCO parameters (nvx_config.nco_hz), else null: the reference table
+    nvx::LongPath* lp = nullptr;          // tap sets too long for the fused kernel: the three stage kernels (fir_long.cuh), else null
     std::vector<int> stream_tag;          // optional [S][2] message tags
     int target_warps[nvx::kSampleFmts] = {576, 576, 576};   // resident cascade warps per sample format
     nvx::MessageAssembler assembler;
@@ -208,8 +171,7 @@ int free_engine(nvx_engine* e) {
         e->worker.join();
     }
     for (cudaEvent_t ev : e->ev_pool) cudaEventDestroy(ev);
-    for (int f = 0; f < nvx::kSampleFmts; ++f) { cudaFree(e->tail[f][0]); cudaFree(e->tail[f][1]); }
-    cudaFree(e->u8_wide);
+    cudaFree(e->tail[0]); cudaFree(e->tail[1]);
     cudaFree(e->corrbuf[0]); cudaFree(e->corrbuf[1]); cudaFree(e->db.clock); cudaFree(e->db.fsm);
     cudaFree(e->db.bitpos); cudaFree(e->db.bitval); cudaFree(e->db.nbits);
     cudaFree(e->d_bits); cudaFree(e->d_disc); cudaFree(e->d_bit_count);
@@ -220,11 +182,8 @@ int free_engine(nvx_engine* e) {
         if (e->stage_free[k]) cudaEventDestroy(e->stage_free[k]);
     }
     if (e->stream_copy) cudaStreamDestroy(e->stream_copy);
-    cudaFree(e->d_nco);
     cudaFree(e->d_nco_ch);
-    for (int k = 0; k < 3; ++k) { cudaFree(e->lhist[k][0]); cudaFree(e->lhist[k][1]); }
-    cudaFree(e->y1buf); cudaFree(e->y2buf);
-    nvx::long_tc_free(e->ltc[0]); nvx::long_tc_free(e->ltc[1]);
+    nvx::long_path_free(e->lp);
     for (int k = 0; k < kBuf; ++k) {
         cudaFree(e->y3buf[k]); cudaFree(e->d_events[k]); cudaFree(e->d_ev_count[k]);
         cudaFreeHost(e->h_events[k]); cudaFreeHost(e->h_ev_count[k]);
@@ -239,17 +198,8 @@ int free_engine(nvx_engine* e) {
 }
 
 int reset_state(nvx_engine* e) {
-    // the warm-up before the first block sees silence: the value 0, which is the byte 128 in 8-bit offset binary
-    for (int f = 0; f < nvx::kSampleFmts; ++f)
-        for (int k = 0; k < 2; ++k)
-            CU_TRY(cudaMemsetAsync(e->tail[f][k], (nvx::SampleFmt)f == nvx::SampleFmt::U8 ? 128 : 0,
-                                   (size_t)e->S * e->halo * nvx::sample_bytes((nvx::SampleFmt)f), e->stream));
-    e->fmt = -1;
-    if (e->long_taps)
-        for (int k = 0; k < 3; ++k)
-            for (int q = 0; q < 2; ++q)
-                CU_TRY(cudaMemsetAsync(e->lhist[k][q], 0, (size_t)(k == 0 ? e->S : e->channels) * e->lst[k].H * sizeof(float2), e->stream));
-    e->lcur = 0;
+    e->fmt = -1;                                    // the next push fixes the format and fills the fused path's tail
+    if (e->lp) CU_TRY(nvx::long_path_reset(e->lp, e->stream));
     for (int k = 0; k < kBuf; ++k) {
         e->db.y3 = e->y3buf[k];
         e->db.picks = e->pickbuf[k];
@@ -397,16 +347,25 @@ int sync_engine(nvx_engine* e) {
     return 0;
 }
 
-// a long-tap stage that was meant for the tensor cores ran on the CUDA-core kernel: counted, and explained in nvx_last_error()
-void note_tc_fallback(nvx_engine* e, int stage, const char* why) {
-    e->stats.long_tc_fallbacks++;
-    fail(0, "note: long-tap stage %d ran on the CUDA-core kernel: %s", stage, why);
+// what the long-tap path reports goes into this engine's nvx_stats and nvx_last_error()
+int long_report(nvx_engine* e, int rc, const nvx::LongReport& rep) {
+    e->stats.aux_launches += rep.launches;
+    e->stats.long_tc_fallbacks += rep.fallbacks;
+    if (rep.msg[0]) fail(rc, "%s", rep.msg);
+    return rc;
 }
 
 int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fmt) {
     using namespace nvx;
     if (e->fmt >= 0 && e->fmt != (int)fmt)
         return fail(NVX_ERR_ARG, "sample format changed between pushes (float, int16 and 8-bit blocks cannot be mixed without a reset)");
+    if (e->fmt < 0 && !e->lp) {
+        // the warm-up before the first block sees silence: the value 0, which is the byte 128 in 8-bit offset binary
+        for (int k = 0; k < 2; ++k) {
+            CU_TRY(cudaMemsetAsync(e->tail[k], fmt == SampleFmt::U8 ? 128 : 0, (size_t)e->S * e->halo * sample_bytes(fmt), e->stream));
+            if (int rc = encode_rows(&e->map_tail[k], e->tail[k], e->halo, e->S, fmt)) return rc;
+        }
+    }
     e->fmt = (int)fmt;
     if (n <= 0 || n % kSuper != 0) return fail(NVX_ERR_ARG, "block length %lld is not a positive multiple of %d", n, kSuper);
     if (n > e->cfg.max_block) return fail(NVX_ERR_ARG, "block length %lld exceeds max_block %lld", n, e->cfg.max_block);
@@ -420,7 +379,7 @@ int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fm
     }
     CascadeArgs ca;
     if (int rc = encode_rows(&ca.map_x, d_x, n, e->S, fmt)) return rc;
-    ca.map_tail = e->map_tail[(int)fmt][e->tail_cur];
+    ca.map_tail = e->map_tail[e->tail_cur];
     const int n_super = (int)(n / kSuper);
     const int groups = (e->S + 31) / 32;
     // time segments: enough warps to fill the machine once, but keep the 7-superblock warm-up small
@@ -457,51 +416,10 @@ int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fm
         }
         CU_TRY(cudaEventRecord(t0, e->stream));
     }
-    if (e->long_taps) {
-        // 8-bit input: widened to the int16 values u - 128 in front of the unchanged int16 long path (same results bit for bit)
-        if (fmt == SampleFmt::U8) {
-            if (!e->u8_wide) CU_TRY(cudaMalloc(&e->u8_wide, (size_t)e->S * e->cfg.max_block * sizeof(short2)));
-            const long long count = (long long)e->S * n;
-            widen_u8_kernel<<<(unsigned)((count / 8 + 255) / 256), 256, 0, e->stream>>>(static_cast<const uchar2*>(d_x), e->u8_wide, count);
-            CU_TRY(cudaGetLastError());
-            e->stats.aux_launches++;
-            d_x = e->u8_wide;
-        }
-        const int s16 = fmt != SampleFmt::F32;
-        const int cur = e->lcur, nx = cur ^ 1;
-        const long long p1 = e->cfg.max_block / NVX_D1, p2 = e->cfg.max_block / (NVX_D1 * NVX_D2);
-        LongArgs la = {};
-        la.in = d_x; la.hist = e->lhist[0][cur]; la.out = e->y1buf; la.n_in = n; la.out_pitch = p1; la.out_off = 0;
-        la.rows_in = e->S; la.stage = 0; la.s16 = s16; la.k_abs = e->sb_abs * (kSuper / NVX_D1); la.nco = e->d_nco;
-        la.plain = e->mix_on_load;                 // stage 2 mixes while it loads: one un-mixed 63 kHz row per stream
-        cudaError_t tc = e->ltc[0] ? long_tc_launch(e->ltc[0], la, e->lst[0], n, e->stream) : cudaErrorNotSupported;
-        if (tc == cudaErrorNotSupported) {         // 252 k -> 63 k, mixed: one row per channel
-            if (e->ltc_wanted[0]) note_tc_fallback(e, 1, e->ltc[0] ? "this block cannot be described to the TMA unit (pointer or pitch not 16-byte aligned)"
-                                                                    : "the tap set does not fit the tensor-core tile");
-            tc = long_launch(la, e->lst[0], e->ltaps[0], n, e->stream);
-        }
-        CU_TRY(tc);
-        CU_TRY(long_carry(e->lhist[0][cur], d_x, n, e->lhist[0][nx], e->S, e->lst[0].H, n, s16, e->stream));
-        la.in = e->y1buf; la.hist = e->lhist[1][cur]; la.out = e->y2buf; la.n_in = n / NVX_D1; la.out_pitch = p2;
-        la.rows_in = e->channels; la.stage = 1; la.s16 = 0; la.nco = nullptr;
-        la.plain = 0; la.mix_in = e->mix_on_load;   // (k_abs: the block's first stage-2 INPUT sample sits at that 63 kHz tick)
-        tc = e->ltc[1] ? long_tc_launch(e->ltc[1], la, e->lst[1], p1, e->stream) : cudaErrorNotSupported;
-        if (tc == cudaErrorNotSupported && e->mix_on_load)      // (cannot happen: y1buf and its pitch are 16-byte aligned)
-            return fail(NVX_ERR_CUDA, "long-tap stage 2: the tensor-core kernel refused the block and the stage-1 output is un-mixed");
-        if (tc == cudaErrorNotSupported) {         // 63 k -> 9 k
-            if (e->ltc_wanted[1]) note_tc_fallback(e, 2, e->ltc[1] ? "this block cannot be described to the TMA unit (pointer or pitch not 16-byte aligned)"
-                                                                    : "the tap set does not fit the tensor-core tile");
-            tc = long_launch(la, e->lst[1], e->ltaps[1], p1, e->stream);
-        }
-        CU_TRY(tc);
-        CU_TRY(long_carry(e->lhist[1][cur], e->y1buf, p1, e->lhist[1][nx], e->mix_on_load ? e->S : e->channels, e->lst[1].H, n / NVX_D1, 0, e->stream));
-        la.mix_in = 0;
-        la.in = e->y2buf; la.hist = e->lhist[2][cur]; la.out = e->y3buf[b]; la.n_in = n / (NVX_D1 * NVX_D2);
-        la.out_pitch = ca.y3_pitch; la.out_off = ca.y3_off; la.stage = 2;
-        CU_TRY(long_launch(la, e->lst[2], e->ltaps[2], p2, e->stream));                // 9 k -> 900
-        CU_TRY(long_carry(e->lhist[2][cur], e->y2buf, p2, e->lhist[2][nx], e->channels, e->lst[2].H, la.n_in, 0, e->stream));
-        e->lcur = nx;
-        e->stats.aux_launches += 5;
+    if (e->lp) {
+        LongReport rep;
+        const int rc = long_path_run(e->lp, d_x, n, fmt, e->sb_abs * (kSuper / NVX_D1), e->y3buf[b], ca.y3_pitch, ca.y3_off, e->stream, &rep);
+        if (long_report(e, rc, rep)) return rc;
     } else {
         // up to four channels share one pass over the input (stage 1 computed once for all of them); five to eight take two
         for (int c0 = 0; c0 < e->C;) {
@@ -515,12 +433,12 @@ int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fm
     }
     if (e->timing) CU_TRY(cudaEventRecord(t1, e->stream));
 
-    const int nxt = e->tail_cur ^ 1;
-    if (!e->long_taps) {
+    if (!e->lp) {
+        const int nxt = e->tail_cur ^ 1;
         const long long work = (long long)e->S * (e->halo / (16 / sample_bytes(fmt)));
         const unsigned grid = (unsigned)((work + 255) / 256);
-        const void* old_tail = e->tail[(int)fmt][e->tail_cur];
-        void* new_tail = e->tail[(int)fmt][nxt];
+        const void* old_tail = e->tail[e->tail_cur];
+        void* new_tail = e->tail[nxt];
         if (fmt == SampleFmt::U8)
             tail_carry_kernel<uchar2><<<grid, 256, 0, e->stream>>>(static_cast<const uchar2*>(old_tail), static_cast<const uchar2*>(d_x),
                                                                    static_cast<uchar2*>(new_tail), e->S, n, e->halo);
@@ -531,8 +449,8 @@ int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fm
             tail_carry_kernel<float2><<<grid, 256, 0, e->stream>>>(static_cast<const float2*>(old_tail), static_cast<const float2*>(d_x),
                                                                    static_cast<float2*>(new_tail), e->S, n, e->halo);
         CU_TRY(cudaGetLastError());
+        e->tail_cur = nxt;
     }
-    e->tail_cur = nxt;
 
     // demod of this block runs on its own stream, overlapping the next block's cascade
     DemodArgs da;
@@ -637,11 +555,9 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
     if ((long long)C * cfg->n_streams > 65535) { delete e; return fail(NVX_ERR_ARG, "n_streams x n_channels = %lld exceeds 65535 channel rows per engine", (long long)C * cfg->n_streams); }
     e->C = C;
     if (cfg->stream_freq_tag) e->stream_tag.assign(cfg->stream_freq_tag, cfg->stream_freq_tag + (size_t)C * (size_t)cfg->n_streams);
-    std::vector<nvx::NcoParam> nco;
-    std::vector<nvx::NcoChan> nco_ch;
+    std::vector<nvx::NcoChan> nco;
     if (cfg->nco_hz) {
-        nco_ch.resize((size_t)cfg->n_streams * C);
-        if (C == 2) nco.resize((size_t)cfg->n_streams);
+        nco.resize((size_t)cfg->n_streams * C);
         for (int k = 0; k < C * cfg->n_streams; ++k) {
             const double f = cfg->nco_hz[k], twice = 2.0 * f;
             if (!(fabs(f) < 31500.0) || twice != nearbyint(twice)) {
@@ -651,10 +567,8 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
             long long num = (long long)twice % nvx::kNcoDen;
             if (num < 0) num += nvx::kNcoDen;
             // same expression as fir2cpp.C:105-106 for table entry 1, rounded once to float
-            const float2 step = make_float2((float)cos((2 * M_PI * 1 * f) / 63000), (float)-sin((2 * M_PI * 1 * f) / 63000));
-            nco_ch[(size_t)k].num = (int)num;
-            nco_ch[(size_t)k].step = step;
-            if (C == 2) { nco[(size_t)k / 2].num[k & 1] = (int)num; nco[(size_t)k / 2].step[k & 1] = step; }
+            nco[(size_t)k].num = (int)num;
+            nco[(size_t)k].step = make_float2((float)cos((2 * M_PI * 1 * f) / 63000), (float)-sin((2 * M_PI * 1 * f) / 63000));
         }
     }
     e->S = cfg->n_streams;
@@ -671,16 +585,11 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
     for (int k = 0; k < 3; ++k)
         if (n[k] < 1 || n[k] > nvx::kLongMaxTaps) { delete e; return fail(NVX_ERR_ARG, "tap count %d outside 1..%d", n[k], nvx::kLongMaxTaps); }
     e->tap_class = nvx::cascade_tap_class(n[0], n[1], n[2]);
-    e->long_taps = e->tap_class < 0;
     if (C != 2 && e->tap_class != 0) {
         delete e;
         return fail(NVX_ERR_ARG, "n_channels = %d is served by the fused kernel's reference tap class only (up to %d / %d / %d taps)", C, NVX_T1, NVX_T2, NVX_T3);
     }
     e->halo = nvx::kSuper * nvx::cascade_warm_super(e->tap_class);
-    if (e->long_taps) {
-        const int D[3] = {NVX_D1, NVX_D2, NVX_D3};
-        for (int k = 0; k < 3; ++k) e->lst[k] = nvx::long_stage(D[k], n[k]);
-    }
     // per block and channel: at most one character plus one abort per 14 bits ... generous bound
     e->ev_cap = 2 * (e->P_max / 63 + 2) + 8;
     e->bit_cap = cfg->keep_bits ? e->P_max / 8 + 2 : 0;      // the symbol clock may run one sample per bit fast while it slews
@@ -708,9 +617,8 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
         CREATE_TRY(cudaEventCreateWithFlags(&e->demod_done[k], cudaEventDisableTiming));
         CREATE_TRY(cudaEventCreateWithFlags(&e->ff_done[k], cudaEventDisableTiming));
     }
-    for (int f = 0; f < nvx::kSampleFmts; ++f)
-        for (int k = 0; k < 2; ++k)
-            CREATE_TRY(cudaMalloc(&e->tail[f][k], (size_t)e->S * e->halo * nvx::sample_bytes((nvx::SampleFmt)f)));
+    if (e->tap_class >= 0)
+        for (int k = 0; k < 2; ++k) CREATE_TRY(cudaMalloc(&e->tail[k], (size_t)e->S * e->halo * nvx::sample_bytes(nvx::SampleFmt::F32)));
     e->db.p_max = e->P_max;
     for (int k = 0; k < kBuf; ++k) CREATE_TRY(cudaMalloc(&e->y3buf[k], (size_t)e->channels * (nvx::kHistY + e->P_max) * sizeof(float2)));
     for (int k = 0; k < 2; ++k) CREATE_TRY(cudaMalloc(&e->corrbuf[k], (size_t)e->channels * (nvx::kHistC + e->P_max + nvx::kPadC) * sizeof(double)));
@@ -735,49 +643,19 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
         CREATE_TRY(cudaMalloc(&e->d_bit_count, sizeof(int) * e->channels));
         CREATE_TRY(cudaMemset(e->d_bit_count, 0, sizeof(int) * e->channels));
     }
-    if (e->long_taps) {
-        static const double d1[NVX_T1] = {NVX_H1_VALUES}, d2[NVX_T2] = {NVX_H2_VALUES}, d3[NVX_T3] = {NVX_H3_VALUES};
-        const double* hh[3] = {cfg->h1 ? cfg->h1 : d1, cfg->h2 ? cfg->h2 : d2, cfg->h3 ? cfg->h3 : d3};
-        for (int k = 0; k < 3; ++k)
-            if (!nvx::long_fill_taps(e->lst[k], hh[k], &e->ltaps[k])) { free_engine(e); return fail(NVX_ERR_ARG, "stage %d: %d taps do not fit the long-tap kernel", k + 1, e->lst[k].T); }
-        for (int k = 0; k < 3; ++k)
-            for (int q = 0; q < 2; ++q)
-                CREATE_TRY(cudaMalloc(&e->lhist[k][q], (size_t)(k == 0 ? e->S : e->channels) * e->lst[k].H * sizeof(float2)));
-        // stages 1 and 2 on the tensor cores where the band matrix fits (fir_long_tc.cu); NVX_LONG_TC is a mask (bit 0: stage
-        // 1, bit 1: stage 2; 0 keeps the CUDA-core kernels, whose output is bit-identical across blockings)
-        const int tc_mask = getenv("NVX_LONG_TC") ? atoi(getenv("NVX_LONG_TC")) : 3;
-        e->ltc_wanted[0] = (tc_mask & 1) != 0;
-        e->ltc_wanted[1] = (tc_mask & 2) != 0;
-        if (tc_mask & 1) e->ltc[0] = nvx::long_tc_prepare(NVX_D1, e->lst[0].T, hh[0], e->stream);
-        if (tc_mask & 2) e->ltc[1] = nvx::long_tc_prepare(NVX_D2, e->lst[1].T, hh[1], e->stream);
-        // a stage the tensor-core kernel does not serve (e.g. stage 2 beyond 959 taps) runs on the CUDA-core kernel: same
-        // results to rounding, about half the speed.  Not an error, but never silent: nvx_last_error() says so after create
-        // and nvx_stats.long_tc_fallbacks counts every such stage launch.
-        for (int k = 0; k < 2; ++k)
-            if (e->ltc_wanted[k] && !e->ltc[k])
-                fail(0, "note: long-tap stage %d (%d taps) is not served by the tensor-core kernel and runs on the CUDA-core kernel", k + 1, e->lst[k].T);
-        CREATE_TRY(cudaMalloc(&e->y1buf, (size_t)e->channels * (cfg->max_block / NVX_D1) * sizeof(float2)));
-        // "mix on load": with the reference offsets (no per-stream NCO) and stage 2 on the streaming tensor-core kernel, stage 1
-        // writes one un-mixed 63 kHz row per stream and stage 2 rotates while it converts: y1 crosses HBM once per stream instead
-        // of once per channel, in both directions.  NVX_LONG_MIX=stage1 keeps the rotation in the stage-1 epilogue (A/B measurements).
-        e->mix_on_load = nco.empty() && nvx::long_tc_mixes_on_load(e->ltc[1]) && (cfg->max_block / NVX_D1) % 2 == 0 &&
-                         !(getenv("NVX_LONG_MIX") && !strcmp(getenv("NVX_LONG_MIX"), "stage1"));
-        CREATE_TRY(cudaMalloc(&e->y2buf, (size_t)e->channels * (cfg->max_block / (NVX_D1 * NVX_D2)) * sizeof(float2)));
+    if (!nco.empty()) {
+        CREATE_TRY(cudaMalloc(&e->d_nco_ch, nco.size() * sizeof(nvx::NcoChan)));
+        CREATE_TRY(cudaMemcpy(e->d_nco_ch, nco.data(), nco.size() * sizeof(nvx::NcoChan), cudaMemcpyHostToDevice));
+    }
+    if (e->tap_class < 0) {
+        const double* const h[3] = {cfg->h1, cfg->h2, cfg->h3};
+        nvx::LongReport rep;
+        const int rc = nvx::long_path_create(e->S, cfg->max_block, n, h, e->d_nco_ch, e->stream, &e->lp, &rep);
+        if (long_report(e, rc, rep)) { free_engine(e); return rc; }
     } else {
         nvx::cascade_fill_taps(e->tap_class, cfg->h1, n[0], cfg->h2, n[1], cfg->h3, n[2], &e->taps);
     }
-    if (!nco.empty()) {
-        CREATE_TRY(cudaMalloc(&e->d_nco, nco.size() * sizeof(nvx::NcoParam)));
-        CREATE_TRY(cudaMemcpy(e->d_nco, nco.data(), nco.size() * sizeof(nvx::NcoParam), cudaMemcpyHostToDevice));
-    }
-    if (!nco_ch.empty()) {
-        CREATE_TRY(cudaMalloc(&e->d_nco_ch, nco_ch.size() * sizeof(nvx::NcoChan)));
-        CREATE_TRY(cudaMemcpy(e->d_nco_ch, nco_ch.data(), nco_ch.size() * sizeof(nvx::NcoChan), cudaMemcpyHostToDevice));
-    }
 #undef CREATE_TRY
-    for (int f = 0; f < nvx::kSampleFmts; ++f)
-        for (int k = 0; k < 2; ++k)
-            if (int rc = encode_rows(&e->map_tail[f][k], e->tail[f][k], e->halo, e->S, (nvx::SampleFmt)f)) { free_engine(e); return rc; }
     for (int f = 0; f < nvx::kSampleFmts; ++f)
         e->target_warps[f] = nvx::cascade_target_warps(cfg->device, nvx::demod_reserved_sms(e->channels), (nvx::SampleFmt)f, e->tap_class, C > 2);
     e->assembler.resize(e->channels);

@@ -168,11 +168,8 @@ struct NcoTable { float2 w[kNcoPeriod + NVX_D2]; };
 // output k is k * f / 63000 turns, tracked exactly as an integer numerator over 126000 (f on a 0.5 Hz grid); every
 // 28-sample step re-seeds the phasor from that exact phase (sincospif) and advances it by six complex multiplies.
 constexpr int kNcoDen = 126000;
-struct NcoParam {      // two-channel layout of the long-tap path
-    int num[2];        // (2 f) mod 126000, per channel
-    float2 step[2];    // (cos, -sin)(2 pi f / 63000): rotation per stage-1 output
-};
-// fused kernel: one entry per (stream, channel), [S][channels]: any number of channels can share stage 1 (SURVEY.md 8f.4)
+// one entry per (stream, channel), [S][channels]: any number of channels can share stage 1 (SURVEY.md 8f.4); the fused kernel's
+// general-NCO variants and the long-tap path's stage 1 (two channels: entries 2 row + c) read the same array
 struct NcoChan {
     int num;           // (2 f) mod 126000
     float2 step;       // (cos, -sin)(2 pi f / 63000)
@@ -214,6 +211,14 @@ struct CascadeTaps {
     TapSet<1> t1;
     NcoTable nco;
 };
+
+// host side (fir_cascade.cu)
+int cascade_box_elems(SampleFmt f);
+int cascade_tap_class(int n1, int n2, int n3);
+int cascade_warm_super(int tap_class);
+void cascade_fill_taps(int tap_class, const double* h1, int n1, const double* h2, int n2, const double* h3, int n3, CascadeTaps* out);
+cudaError_t cascade_launch(const CascadeArgs& a, const CascadeTaps& taps, int tap_class, bool custom_taps, SampleFmt f, int n_ch, cudaStream_t stream);
+int cascade_target_warps(int device, int reserved_sms, SampleFmt f, int tap_class, bool heavy);
 
 #ifdef NVX_CASCADE_DEVICE_CODE
 

@@ -1,11 +1,25 @@
-// fir_long.cu -- register-tiled polyphase decimating FIR kernels for long tap sets (see fir_long.cuh).
+// fir_long.cu -- register-tiled polyphase decimating FIR kernels for long tap sets, and the long-tap path of an engine that
+// runs them (see fir_long.cuh).
 #include "fir_long.cuh"
 
 #include <math.h>
+#include <stdarg.h>
+#include <stdio.h>
+#include <stdlib.h>
+#include <string.h>
+
+#include "../../include/navtex_b200.h"
 
 namespace nvx {
 
 namespace {
+
+// taps of one stage regrouped per decimation phase + the reference NCO table: passed by value in the kernel parameter block
+constexpr int kLongTapSlots = 1152;             // D * J <= 1024 + D * kLongR
+struct LongStageTaps {
+    float h[kLongTapSlots];
+    float2 nco[kNcoPeriod];
+};
 
 // The taps of the launched stage and the reference NCO table travel in the kernel parameter block (constant bank 0,
 // __grid_constant__): per engine, so engines with different tap sets can be alive on one device, and still warp-uniform
@@ -132,8 +146,8 @@ __global__ void __launch_bounds__(long_threads(D)) fir_long_kernel(const LongArg
         // NCO mix: output k sits at 63 kHz clock tick k_abs + k; channel c gets y1 * (cos - j sin)(2 pi tick f_c / 63000)
         float2* out0 = a.out + (size_t)(2 * row_in) * a.out_pitch + a.out_off + k0 + (long long)kLongR * t;
         float2* out1 = out0 + a.out_pitch;
-        NcoParam np = {};
-        if (a.nco) np = a.nco[row_in];
+        int num[2] = {0, 0};
+        if (a.nco) { num[0] = a.nco[2 * row_in].num; num[1] = a.nco[2 * row_in + 1].num; }
         const long long tick0 = a.k_abs + k0 + (long long)kLongR * t;
         long long r9 = tick0 % kNcoPeriod, rden = tick0 % kNcoDen;
         int k9 = (int)(r9 < 0 ? r9 + kNcoPeriod : r9), kden = (int)(rden < 0 ? rden + kNcoDen : rden);
@@ -143,7 +157,7 @@ __global__ void __launch_bounds__(long_threads(D)) fir_long_kernel(const LongArg
             if (a.nco) {
 #pragma unroll
                 for (int c = 0; c < 2; ++c) {
-                    const int ph = (int)(((long long)kden * np.num[c]) % kNcoDen);
+                    const int ph = (int)(((long long)kden * num[c]) % kNcoDen);
                     float tt = (float)ph * (2.0f / kNcoDen);
                     if (tt > 1.0f) tt -= 2.0f;
                     float sn, cs;
@@ -202,7 +216,30 @@ cudaError_t launch_one(const LongArgs& a, const LongStage& st, const LongStageTa
     return cudaGetLastError();
 }
 
-}  // namespace
+// 8-bit input: out = (u - 128) as short2, 8 samples (16 bytes in, 32 out) per thread; count = S n, a multiple of 280
+__global__ void widen_u8_kernel(const uchar2* __restrict__ in, short2* __restrict__ out, long long count) {
+    const long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 8;
+    if (i >= count) return;
+    const int4 v = *reinterpret_cast<const int4*>(in + i);
+    const unsigned w[4] = {(unsigned)v.x, (unsigned)v.y, (unsigned)v.z, (unsigned)v.w};
+    int o[8];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {       // bytes I0 Q0 I1 Q1 of a word -> two short2 words
+        o[2 * k] = (int)(((w[k] & 0xFFu) - 128u) & 0xFFFFu) | (int)(((((w[k] >> 8) & 0xFFu) - 128u) & 0xFFFFu) << 16);
+        o[2 * k + 1] = (int)((((w[k] >> 16) & 0xFFu) - 128u) & 0xFFFFu) | (int)((((w[k] >> 24) - 128u) & 0xFFFFu) << 16);
+    }
+    int4* dst = reinterpret_cast<int4*>(out + i);
+    dst[0] = make_int4(o[0], o[1], o[2], o[3]);
+    dst[1] = make_int4(o[4], o[5], o[6], o[7]);
+}
+
+int say(LongReport* rep, int code, const char* fmt, ...) {
+    va_list ap;
+    va_start(ap, fmt);
+    vsnprintf(rep->msg, sizeof rep->msg, fmt, ap);
+    va_end(ap);
+    return code;
+}
 
 LongStage long_stage(int D, int T) {
     LongStage s;
@@ -236,6 +273,7 @@ cudaError_t long_launch(const LongArgs& a, const LongStage& st, const LongStageT
     }
 }
 
+// new_hist = last H samples of (old_hist ++ block[.][0..n)) per row; block rows are `pitch` samples apart, short2 if s16
 cudaError_t long_carry(const float2* old_hist, const void* block, long long pitch, float2* new_hist, int rows, int H, long long n,
                        int s16, cudaStream_t stream) {
     const long long work = (long long)rows * H;
@@ -245,6 +283,138 @@ cudaError_t long_carry(const float2* old_hist, const void* block, long long pitc
     else
         long_carry_kernel<float2><<<grid, 256, 0, stream>>>(old_hist, static_cast<const float2*>(block), pitch, new_hist, rows, H, n);
     return cudaGetLastError();
+}
+
+}  // namespace
+
+// ---- the long-tap path of one engine ----
+
+struct LongPath {
+    int S = 0;                            // streams; stages 2 and 3 run over the 2 S channel rows
+    long long max_block = 0;
+    const NcoChan* nco = nullptr;         // the engine's [S][2] per-stream offsets, or null: the reference table
+    LongStage st[3];
+    LongStageTaps taps[3];                // passed in the parameter block of every stage launch
+    float2* hist[3][2] = {};              // [stage][ping-pong]: [rows][H]
+    int cur = 0;
+    float2 *y1 = nullptr, *y2 = nullptr;  // 63 kHz and 9 kHz intermediates, [2 S][max_block / 4] and [2 S][max_block / 28]
+    LongTcStage* tc[3] = {};              // tensor-core variants of stages 1 and 2 (null: CUDA-core kernel; stage 3 has none)
+    bool tc_wanted[3] = {};               // the tensor-core kernel was asked for (NVX_LONG_TC mask) for that stage
+    bool mix_on_load = false;             // stage 1 writes ONE un-mixed row per stream, stage 2 rotates while it loads
+    short2* u8_wide = nullptr;            // 8-bit input: [S][max_block] short2 (u - 128), allocated on first use
+};
+
+namespace {
+
+size_t hist_bytes(const LongPath* lp, int k) { return (size_t)(k == 0 ? lp->S : 2 * lp->S) * lp->st[k].H * sizeof(float2); }
+
+// stage k + 1: on the tensor cores where they serve it, else on the CUDA-core kernel (counted and explained when the tensor cores
+// were asked for); then its history carry, the last H inputs of each of `rows` rows (S stream rows of y1 when stage 2 mixes on load)
+int run_stage(LongPath* lp, int k, const LongArgs& a, long long in_pitch, int rows, cudaStream_t stream, LongReport* rep) {
+    cudaError_t e = lp->tc[k] ? long_tc_launch(lp->tc[k], a, lp->st[k], in_pitch, stream) : cudaErrorNotSupported;
+    if (e == cudaErrorNotSupported && a.mix_in)      // (cannot happen: y1 and its pitch are 16-byte aligned)
+        return say(rep, NVX_ERR_CUDA, "long-tap stage 2: the tensor-core kernel refused the block and the stage-1 output is un-mixed");
+    if (e == cudaErrorNotSupported) {
+        if (lp->tc_wanted[k]) {
+            rep->fallbacks++;
+            say(rep, 0, "note: long-tap stage %d ran on the CUDA-core kernel: %s", k + 1, lp->tc[k] ? "this block cannot be described to the TMA unit (pointer or pitch not 16-byte aligned)"
+                                                                                         : "the tap set does not fit the tensor-core tile");
+        }
+        e = long_launch(a, lp->st[k], lp->taps[k], in_pitch, stream);
+    }
+    if (e == cudaSuccess) e = long_carry(a.hist, a.in, in_pitch, lp->hist[k][lp->cur ^ 1], rows, lp->st[k].H, a.n_in, a.s16, stream);
+    return e == cudaSuccess ? 0 : say(rep, NVX_ERR_CUDA, "long-tap stage %d failed: %s", k + 1, cudaGetErrorString(e));
+}
+
+}  // namespace
+
+int long_path_create(int S, long long max_block, const int n[3], const double* const h[3], const NcoChan* nco, cudaStream_t stream,
+                     LongPath** out, LongReport* rep) {
+    static const double ref1[NVX_T1] = {NVX_H1_VALUES}, ref2[NVX_T2] = {NVX_H2_VALUES}, ref3[NVX_T3] = {NVX_H3_VALUES};
+    const double* hh[3] = {h[0] ? h[0] : ref1, h[1] ? h[1] : ref2, h[2] ? h[2] : ref3};
+    const int D[3] = {NVX_D1, NVX_D2, NVX_D3};
+    LongPath* lp = new LongPath();
+    lp->S = S; lp->max_block = max_block; lp->nco = nco;
+    for (int k = 0; k < 3; ++k) {
+        lp->st[k] = long_stage(D[k], n[k]);
+        if (!long_fill_taps(lp->st[k], hh[k], &lp->taps[k])) { long_path_free(lp); return say(rep, NVX_ERR_ARG, "stage %d: %d taps do not fit the long-tap kernel", k + 1, n[k]); }
+    }
+    cudaError_t e = cudaSuccess;
+    for (int k = 0; k < 3; ++k)
+        for (int q = 0; q < 2 && e == cudaSuccess; ++q) e = cudaMalloc(&lp->hist[k][q], hist_bytes(lp, k));
+    if (e == cudaSuccess) e = cudaMalloc(&lp->y1, (size_t)2 * S * (max_block / NVX_D1) * sizeof(float2));
+    if (e == cudaSuccess) e = cudaMalloc(&lp->y2, (size_t)2 * S * (max_block / (NVX_D1 * NVX_D2)) * sizeof(float2));
+    if (e != cudaSuccess) {
+        long_path_free(lp);
+        return say(rep, e == cudaErrorMemoryAllocation ? NVX_ERR_NOMEM : NVX_ERR_CUDA, "long-tap path: cudaMalloc failed: %s", cudaGetErrorString(e));
+    }
+    // stages 1 and 2 on the tensor cores where the band matrix fits (fir_long_tc.cu); NVX_LONG_TC is a mask (bit 0: stage
+    // 1, bit 1: stage 2; 0 keeps the CUDA-core kernels, whose output is bit-identical across blockings)
+    const int tc_mask = getenv("NVX_LONG_TC") ? atoi(getenv("NVX_LONG_TC")) : 3;
+    for (int k = 0; k < 2; ++k) {
+        lp->tc_wanted[k] = (tc_mask >> k & 1) != 0;
+        if (lp->tc_wanted[k]) lp->tc[k] = long_tc_prepare(D[k], n[k], hh[k], stream);
+        // a stage the tensor-core kernel does not serve (e.g. stage 2 beyond 959 taps) runs on the CUDA-core kernel: same
+        // results to rounding, about half the speed.  Not an error, but never silent: nvx_last_error() says so after create
+        // and nvx_stats.long_tc_fallbacks counts every such stage launch.
+        if (lp->tc_wanted[k] && !lp->tc[k])
+            say(rep, 0, "note: long-tap stage %d (%d taps) is not served by the tensor-core kernel and runs on the CUDA-core kernel", k + 1, n[k]);
+    }
+    // "mix on load": with the reference offsets (no per-stream NCO) and stage 2 on the streaming tensor-core kernel, stage 1
+    // writes one un-mixed 63 kHz row per stream and stage 2 rotates while it converts: y1 crosses HBM once per stream instead
+    // of once per channel, in both directions.  NVX_LONG_MIX=stage1 keeps the rotation in the stage-1 epilogue (A/B measurements).
+    const char* mix = getenv("NVX_LONG_MIX");
+    lp->mix_on_load = !nco && long_tc_mixes_on_load(lp->tc[1]) && (max_block / NVX_D1) % 2 == 0 && !(mix && !strcmp(mix, "stage1"));
+    *out = lp;
+    return 0;
+}
+
+cudaError_t long_path_reset(LongPath* lp, cudaStream_t stream) {
+    lp->cur = 0;
+    cudaError_t e = cudaSuccess;
+    for (int k = 0; k < 3; ++k)
+        for (int q = 0; q < 2 && e == cudaSuccess; ++q) e = cudaMemsetAsync(lp->hist[k][q], 0, hist_bytes(lp, k), stream);
+    return e;
+}
+
+// 3 stage launches and 3 history carries: 5 in nvx_stats.aux_launches, where the engine counts one per block for every path
+int long_path_run(LongPath* lp, const void* x, long long n, SampleFmt fmt, long long tick, float2* y3, long long y3_pitch,
+                  long long y3_off, cudaStream_t stream, LongReport* rep) {
+    const int S = lp->S;
+    // 8-bit input: widened to the int16 values u - 128 in front of the unchanged int16 path (same results bit for bit)
+    if (fmt == SampleFmt::U8) {
+        const long long count = (long long)S * n;
+        cudaError_t e = lp->u8_wide ? cudaSuccess : cudaMalloc(&lp->u8_wide, (size_t)S * lp->max_block * sizeof(short2));
+        if (e == cudaSuccess) widen_u8_kernel<<<(unsigned)((count / 8 + 255) / 256), 256, 0, stream>>>(static_cast<const uchar2*>(x), lp->u8_wide, count);
+        if (e == cudaSuccess) e = cudaGetLastError();
+        if (e != cudaSuccess) return say(rep, NVX_ERR_CUDA, "long-tap path, 8-bit input: %s", cudaGetErrorString(e));
+        rep->launches++;
+        x = lp->u8_wide;
+    }
+    const long long p1 = lp->max_block / NVX_D1, p2 = lp->max_block / (NVX_D1 * NVX_D2);     // row pitches of y1 and y2
+    LongArgs a1 = {};         // 252 k -> 63 k: mixed, one row per channel, or un-mixed, one row per stream (mix on load)
+    a1.in = x; a1.hist = lp->hist[0][lp->cur]; a1.out = lp->y1; a1.n_in = n; a1.out_pitch = p1;
+    a1.rows_in = S; a1.stage = 0; a1.s16 = fmt != SampleFmt::F32; a1.k_abs = tick; a1.nco = lp->nco; a1.plain = lp->mix_on_load;
+    if (int rc = run_stage(lp, 0, a1, n, S, stream, rep)) return rc;
+    LongArgs a2 = {};         // 63 k -> 9 k (k_abs: the block's first stage-2 INPUT sample sits at that 63 kHz tick)
+    a2.in = lp->y1; a2.hist = lp->hist[1][lp->cur]; a2.out = lp->y2; a2.n_in = n / NVX_D1; a2.out_pitch = p2;
+    a2.rows_in = 2 * S; a2.stage = 1; a2.k_abs = tick; a2.mix_in = lp->mix_on_load;
+    if (int rc = run_stage(lp, 1, a2, p1, lp->mix_on_load ? S : 2 * S, stream, rep)) return rc;
+    LongArgs a3 = {};         // 9 k -> 900
+    a3.in = lp->y2; a3.hist = lp->hist[2][lp->cur]; a3.out = y3; a3.n_in = n / (NVX_D1 * NVX_D2); a3.out_pitch = y3_pitch; a3.out_off = y3_off;
+    a3.rows_in = 2 * S; a3.stage = 2;
+    if (int rc = run_stage(lp, 2, a3, p2, 2 * S, stream, rep)) return rc;
+    lp->cur ^= 1;
+    rep->launches += 5;
+    return 0;
+}
+
+void long_path_free(LongPath* lp) {
+    if (!lp) return;
+    for (auto& h : lp->hist) { cudaFree(h[0]); cudaFree(h[1]); }
+    cudaFree(lp->y1); cudaFree(lp->y2); cudaFree(lp->u8_wide);
+    long_tc_free(lp->tc[0]); long_tc_free(lp->tc[1]);
+    delete lp;
 }
 
 }  // namespace nvx

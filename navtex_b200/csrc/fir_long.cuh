@@ -52,7 +52,7 @@ struct LongArgs {
     int stage;                // 0, 1, 2
     int s16;                  // stage 1 only: input block is short2
     long long k_abs;          // stage 1: absolute index of the block's first OUTPUT sample (63 kHz clock), for the NCO
-    const NcoParam* nco;      // stage 1: per-stream general NCO or null (reference table)
+    const NcoChan* nco;       // stage 1: [rows_in][2] per-stream general NCO or null (reference table)
     // "mix on load" (reference NCO table only): stage 1 leaves its output un-mixed, ONE 63 kHz row per stream (plain = 1), and the
     // tensor-core stage 2 applies the rotation of its row's channel while it converts the samples (mix_in = 1: the input has
     // rows_in / 2 rows, k_abs is the absolute index of the block's first INPUT sample) -- the same FP32 products in the same order
@@ -60,21 +60,7 @@ struct LongArgs {
     int plain, mix_in;
 };
 
-// taps of one stage regrouped per decimation phase + the reference NCO table: passed by value in the kernel parameter block
-constexpr int kLongTapSlots = 1152;             // D * J <= 1024 + D * kLongR
-struct LongStageTaps {
-    float h[kLongTapSlots];
-    float2 nco[kNcoPeriod];
-};
-
-LongStage long_stage(int D, int T);
-bool long_fill_taps(const LongStage& st, const double* h, LongStageTaps* out);
-cudaError_t long_launch(const LongArgs& a, const LongStage& st, const LongStageTaps& tp, long long in_pitch, cudaStream_t stream);
-// new_hist = last H samples of (old_hist ++ block[.][0..n)) per row; block rows are `pitch` samples apart, short2 if s16
-cudaError_t long_carry(const float2* old_hist, const void* block, long long pitch, float2* new_hist, int rows, int H, long long n,
-                       int s16, cudaStream_t stream);
-
-// ---- tensor-core variant of stages 1 and 2 (fir_long_tc.cu): tcgen05 3xTF32 Toeplitz GEMM, same contract as long_launch ----
+// ---- tensor-core variant of stages 1 and 2 (fir_long_tc.cu): tcgen05 3xTF32 Toeplitz GEMM, same contract as the CUDA-core stages ----
 struct LongTcStage;
 struct TcBand {
     int T, N, chunks, J, copies;      // padded taps, outputs per tile, K chunks per tile, band rows per copy, copies
@@ -87,5 +73,25 @@ LongTcStage* long_tc_prepare(int D, int T, const double* h, cudaStream_t stream)
 void long_tc_free(LongTcStage* s);
 bool long_tc_mixes_on_load(const LongTcStage* s);      // stage 2 served by the streaming kernel: LongArgs.mix_in is available
 cudaError_t long_tc_launch(const LongTcStage* s, const LongArgs& a, const LongStage& st, long long in_pitch, cudaStream_t stream);
+
+// ---- the long-tap path of one engine (S streams, two channels each) ----
+// It owns the stage taps, the per-stage histories, the y1 / y2 intermediates, the tensor-core stages and the choice of mix on
+// load.  The engine owns nvx_last_error() and nvx_stats: create and run report to it through a LongReport.
+struct LongPath;
+struct LongReport {
+    long long launches = 0;   // kernels launched (nvx_stats.aux_launches)
+    long long fallbacks = 0;  // stage launches meant for the tensor-core kernel that ran on the CUDA-core one (nvx_stats.long_tc_fallbacks)
+    char msg[256] = "";       // for nvx_last_error(): why the call failed, else a "note: ..." about a tensor-core fallback, else empty
+};
+// n[k] taps of stage k + 1, h[k] = null for the reference taps; nco = the engine's [S][2] per-stream offsets, or null for the
+// reference table.  Reads NVX_LONG_TC and NVX_LONG_MIX.  Returns 0 or an NVX_ERR_* code.
+int long_path_create(int S, long long max_block, const int n[3], const double* const h[3], const NcoChan* nco, cudaStream_t stream,
+                     LongPath** out, LongReport* rep);
+cudaError_t long_path_reset(LongPath* lp, cudaStream_t stream);     // zero histories: the next block starts after silence
+// one block x[S][n] in format fmt whose first 63 kHz output sits at tick; the 900 Hz output goes to y3[2 S][y3_pitch] from
+// y3_off on.  Returns 0 or an NVX_ERR_* code.
+int long_path_run(LongPath* lp, const void* x, long long n, SampleFmt fmt, long long tick, float2* y3, long long y3_pitch,
+                  long long y3_off, cudaStream_t stream, LongReport* rep);
+void long_path_free(LongPath* lp);
 
 }  // namespace nvx

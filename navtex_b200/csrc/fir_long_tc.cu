@@ -97,7 +97,7 @@ struct TcArgs {
     const float2* hist;
     float2* out;
     long long n_in, in_pitch, out_pitch, out_off, k_abs;
-    const NcoParam* nco;
+    const NcoChan* nco;
     int rows, s16, T, H, chunks, J, slots, box_rows, mix;
     int rows_src;                          // rows of the input: rows, or rows / 2 stream rows when the stage mixes on load
     int cpt, lead;                         // streaming kernel: chunks per tile advance (D N / chunk samples), chunks a window leads its tile by
@@ -511,11 +511,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) fir_tc_kernel(const __grid_cons
                     const long long kden = rden < 0 ? rden + kNcoDen : rden;
 #pragma unroll 2
                     for (int r = 0; r < r_max; ++r, dst += 2 * a.out_pitch) {
-                        const NcoParam np = a.nco[row0 + r];
+                        const int num[2] = {a.nco[2 * (row0 + r)].num, a.nco[2 * (row0 + r) + 1].num};
                         const float2 y = make_float2(rows0[r * kDumpPitch + m], rows0[r * kDumpPitch + NP + m]);
 #pragma unroll
                         for (int c = 0; c < 2; ++c) {
-                            const int phs = (int)((kden * np.num[c]) % kNcoDen);
+                            const int phs = (int)((kden * num[c]) % kNcoDen);
                             float tt = (float)phs * (2.0f / kNcoDen);
                             if (tt > 1.0f) tt -= 2.0f;
                             float sn, cs;
@@ -984,11 +984,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) fir_tcs_kernel(const __grid_con
                             const long long kden = rden < 0 ? rden + kNcoDen : rden;
 #pragma unroll 2
                             for (int rr = 0; rr < r_max; ++rr, dst += 2 * a.out_pitch) {
-                                const NcoParam np = a.nco[row0 + rr];
+                                const int num[2] = {a.nco[2 * (row0 + rr)].num, a.nco[2 * (row0 + rr) + 1].num};
                                 const float2 y = make_float2(rows0[rr * kDumpPitch + m], rows0[rr * kDumpPitch + NP + m]);
 #pragma unroll
                                 for (int c = 0; c < 2; ++c) {
-                                    const int phs = (int)((kden * np.num[c]) % kNcoDen);
+                                    const int phs = (int)((kden * num[c]) % kNcoDen);
                                     float tt = (float)phs * (2.0f / kNcoDen);
                                     if (tt > 1.0f) tt -= 2.0f;
                                     float sn, cs;
