@@ -101,6 +101,27 @@ void nvx_engine_destroy(nvx_engine *e);
 /* back to the state right after create (zero FIR history, decoder INIT, phasing search) */
 int nvx_engine_reset(nvx_engine *e);
 
+/* ---- per-stream lifecycle: one radio reconnects or is retuned while the others keep decoding ----------------------------
+ * streams[0..count): local indices 0..S-1 (duplicates are fine).  Each listed stream restarts as if the engine had just been
+ * created for it: zero FIR history, decoder INIT, phasing search, its partly received line and message dropped without being
+ * delivered (like nvx_engine_reset).  Takes effect at the start of the next push; every other stream is untouched.  Messages
+ * the stream completed in blocks pushed before still arrive.  Callable before the first push (harmless).
+ *
+ * The demod grids are absolute and shared by all channels (evaluation samples at 900 Hz index = 6 mod 9, the 567-sample
+ * correlation ring, the order of its FP64 sums), so a reset stream restarts on that grid: a reset that takes effect at input
+ * sample E (the total pushed per stream so far) restarts the stream at E0 = E - (E mod 158760), 158760 = 567 x 280.  From
+ * then on the stream is, bit for bit, what a freshly created engine produces when fed Z = E - E0 zero samples followed by the
+ * stream's input from E on: y3, bits, discriminator sums, events and messages (the Z < 158760 zeros make no decision: the
+ * ring is not full before 574 samples at 900 Hz).  On the long-tap path with its tensor-core stages "bit for bit" reads
+ * "to rounding", as for any change of blocking there (see n1 / n2 / n3).  The extra work -- one small kernel -- is only
+ * queued on pushes that carry a reset; it waits for the previous block's demod. */
+int nvx_engine_reset_streams(nvx_engine *e, const int *streams, int count);
+/* new channel offsets nco_hz[n_channels] (same rules as nvx_config.nco_hz) and optionally new tags freq_tag[n_channels]
+ * (NULL = keep the current ones) for one stream.  Implies nvx_engine_reset_streams for that stream, whose rule also places
+ * the new NCO's phase origin: phase 0 at E0.  Messages of blocks pushed before carry the old tags.  Returns NVX_ERR_ARG if
+ * the engine was created without nco_hz (reference-table engines cannot be retuned). */
+int nvx_engine_retune_stream(nvx_engine *e, int stream, const double *nco_hz, const int *freq_tag);
+
 /* ---- ingest: n samples for every stream.  Host variants copy H2D on a copy stream into one of two staging slots, so
  * the copy of block k+1 overlaps the kernels of block k.  A pageable buffer may be reused as soon as the call returns;
  * a pinned (cudaHostAlloc / cudaHostRegister) buffer is read asynchronously and must stay unchanged until
@@ -149,7 +170,8 @@ typedef struct {
     double demod_ms;            /* same for the demod/bit-sync/FSM kernel */
     long long cascade_launches;
     long long demod_launches;
-    long long aux_launches;     /* tail carry, second pass of five to eight channels, long-tap stages, 8-bit -> int16 widening (long-tap path) */
+    long long aux_launches;     /* tail carry, second pass of five to eight channels, long-tap stages, 8-bit -> int16 widening (long-tap path),
+                                 * per-stream resets */
     long long samples;          /* IQ samples (all streams) pushed */
     double demod_stage_ms[6];   /* split of demod_ms: angle/correlation, per-offset sums + arg max, history carry | symbol clock, bit decisions, SITOR-B state machine */
     long long long_tc_fallbacks;/* long-tap stage launches that were meant for the tensor-core kernel but ran on the CUDA-core one
@@ -199,13 +221,20 @@ int nvx_capture_write(nvx_capture *c, int stream, const short *xi, const short *
  * over (len = 2 num_samples).  Writing int16 to an 8-bit capture or 8-bit pairs to an int16 capture returns NVX_ERR_ARG;
  * overflow as for nvx_capture_write */
 int nvx_capture_write_u8(nvx_capture *c, int stream, const unsigned char *iq, unsigned num_samples);
-/* consumer: push what every stream has in common (multiple of 280, <= max_block) as one block in the capture's format.
+/* consumer: push what every attached stream has in common (multiple of 280, <= max_block) as one block in the capture's format.
  * Returns samples per stream pushed, 0 if there was less than 280, or a negative nvx_status */
 long long nvx_capture_pump(nvx_capture *c);
 /* or let a poller thread pump every poll_ms (<= 0: 50 ms, capt_sched.c:489); stop() drains what is left */
 int nvx_capture_start(nvx_capture *c, int poll_ms);
 int nvx_capture_stop(nvx_capture *c);
 long long nvx_capture_dropped(nvx_capture *c, int stream);
+/* a radio that stops delivering: a detached stream no longer holds the pump back.  Its rows of each pumped block are silence
+ * (0 for int16, 0x80 for 8-bit), and writes to it return NVX_ERR_ARG (nothing is counted as dropped).  attach flushes its ring
+ * and resets the stream in the engine (nvx_engine_reset_streams), ordered between two pumps: the radio's first samples after
+ * attach start a fresh decoder.  Detaching a detached or attaching an attached stream does nothing.  The pump returns 0
+ * while every stream is detached. */
+int nvx_capture_detach(nvx_capture *c, int stream);
+int nvx_capture_attach(nvx_capture *c, int stream);
 
 /* ---- in-memory message store behind add_message (message_store.c:59-97): newest message per (stream, B1B2B3B4) -------- */
 typedef struct nvx_store nvx_store;

@@ -5,8 +5,9 @@
 //   producer  StreamACallback  receiver/capt_sched.c:105-148  (xi[], xq[] int16 arrays, numSamples per callback,
 //                                                              interleaved into one ring of shorts under a mutex)
 //   consumer  main loop        receiver/capt_sched.c:484-528  (every 50 ms: drain the ring, sample_in_1 per I,Q pair)
-// Here every stream has its own ring of interleaved int16 I,Q; the consumer ("pump") takes what ALL streams have in
-// common, rounded down to a multiple of 280 samples, lays it out stream-major and pushes it as one int16 block.
+// Here every stream has its own ring of interleaved int16 I,Q; the consumer ("pump") takes what ALL attached streams have
+// in common, rounded down to a multiple of 280 samples, lays it out stream-major and pushes it as one int16 block (silence in
+// the rows of detached streams, so that one radio that stops delivering does not stall the others).
 // nvx_capture_create_u8 makes the same front end for RTL-SDR radios: rings of interleaved 8-bit I,Q bytes (the buffer
 // rtlsdr_read_async hands its callback), pumped with nvx_engine_push_host_u8.
 //
@@ -38,6 +39,7 @@ struct nvx_capture {
         long long head = 0, tail = 0;      // absolute sample counts written / consumed
         std::mutex mu;                     // in_mutex of capt_sched.c:109-112
         long long dropped = 0;
+        bool attached = true;              // changed under pump_mu and mu
     };
     std::vector<Ring> rings;
     // [S][n] staging, stream-major: two page-locked buffers (nvx_pinned_alloc), so that the engine's H2D copy of pump k is
@@ -54,11 +56,15 @@ struct nvx_capture {
 namespace {
 long long pump_locked(nvx_capture* c) {
     long long n = c->max_block;
+    bool any = false;
     for (auto& r : c->rings) {
         std::lock_guard<std::mutex> lk(r.mu);
+        if (!r.attached) continue;
+        any = true;
         const long long avail = r.head - r.tail;
         if (avail < n) n = avail;
     }
+    if (!any) return 0;
     n -= n % NVX_BLOCK_ALIGN;
     if (n <= 0) return 0;
     const unsigned which = c->pumps++ & 1;
@@ -70,6 +76,10 @@ long long pump_locked(nvx_capture* c) {
     for (int s = 0; s < c->S; ++s) {
         auto& r = c->rings[(size_t)s];
         uint8_t* dst = blk + (size_t)s * c->bps * (size_t)n;
+        if (!r.attached) {                 // the value 0: 0x80 in 8-bit offset binary
+            memset(dst, c->u8 ? 0x80 : 0, c->bps * (size_t)n);
+            continue;
+        }
         // the producer only ever writes beyond head, so [tail, tail + n) is stable without the lock
         long long at = r.tail % c->ring;
         long long first = n < c->ring - at ? n : c->ring - at;
@@ -116,6 +126,7 @@ int write_ring(nvx_capture* c, int stream, unsigned num_samples, Put put) {
     long long head, tail;
     {
         std::lock_guard<std::mutex> lk(r.mu);
+        if (!r.attached) return NVX_ERR_ARG;
         head = r.head;
         tail = r.tail;
     }
@@ -195,6 +206,27 @@ int nvx_capture_stop(nvx_capture* c) {
     const int rc = c->pump_rc ? c->pump_rc : (n < 0 ? (int)n : 0);
     c->pump_rc = 0;
     return rc;
+}
+
+int nvx_capture_detach(nvx_capture* c, int stream) {
+    if (!c || stream < 0 || stream >= c->S) return NVX_ERR_ARG;
+    std::lock_guard<std::mutex> lk(c->pump_mu);
+    std::lock_guard<std::mutex> lr(c->rings[(size_t)stream].mu);
+    c->rings[(size_t)stream].attached = false;
+    return 0;
+}
+
+int nvx_capture_attach(nvx_capture* c, int stream) {
+    if (!c || stream < 0 || stream >= c->S) return NVX_ERR_ARG;
+    std::lock_guard<std::mutex> lk(c->pump_mu);
+    auto& r = c->rings[(size_t)stream];
+    {
+        std::lock_guard<std::mutex> lr(r.mu);
+        if (r.attached) return 0;
+        r.tail = r.head;                   // whatever was left from before the detach is stale
+        r.attached = true;
+    }
+    return nvx_engine_reset_streams(c->eng, &stream, 1);
 }
 
 long long nvx_capture_dropped(nvx_capture* c, int stream) {

@@ -38,9 +38,6 @@ constexpr int kThreads = 128;           // feed-forward kernels: one warp per SM
 constexpr int kPer = 3;                 // samples per thread (independent dependency chains)
 constexpr int kTile = kThreads * kPer;  // samples per CTA
 
-enum { DS_INIT = 0, DS_WAIT = 1, DS_PENDING = 2 };   // decoder.h:16-19 (BIT_START / RECEIVING folded into PENDING)
-enum { BY_WAIT = 1, BY_GOT_DX = 2, BY_GOT_RX = 3 };                       // nav_b_sm.h:41-43
-
 __constant__ unsigned char c_ltrs[128];
 __constant__ unsigned char c_figs[128];
 __constant__ float c_tone_r[5];
@@ -258,6 +255,8 @@ __global__ void __launch_bounds__(kSumWarps * 32) offset_sum_kernel(const DemodA
     const bool mine = kk < 3 && unit < (long long)a.channels * n_rev;
     const int ch = mine ? (int)(unit / n_rev) : 0;
     const int K = k_lo + (mine ? (int)(unit % n_rev) : 0);
+    // first block-relative sample whose ring is full (decoder.C:181), counted from the channel's epoch (nvx_engine_reset_streams)
+    const int m_full = (int)max(kCorrLen + 7 - (a.seen - a.b.epoch[ch]), -(1ll << 30));
     // block-relative sample of the evaluation r = 0 of this thread; its class members sit 8 samples earlier
     const int m_first = (int)(16 + (long long)kCorrLen * K + j - a.seen);
     const double* cur = a.b.corr + (size_t)ch * pitch_c(a.b.p_max) + kHistC + (m_first - 8);
@@ -267,6 +266,7 @@ __global__ void __launch_bounds__(kSumWarps * 32) offset_sum_kernel(const DemodA
     const long long unit2 = ((long long)blockIdx.x * kSumWarps + warp) * 3 + kk2;
     const bool judge = kk2 < 3 && unit2 < (long long)a.channels * n_rev;
     const int ch2 = judge ? (int)(unit2 / n_rev) : 0;
+    const int w_full = (int)max(kCorrLen + 15 - (a.seen - a.b.epoch[ch2]), -(1ll << 30));     // first evaluation with a pick
     const int w_first = (int)(24 + (long long)kCorrLen * (k_lo + (judge ? (int)(unit2 % n_rev) : 0)) - a.seen);
     uint8_t* picks2 = a.b.picks + (size_t)ch2 * pitch_p(a.b.p_max);     // evaluation samples of a block: e0 + 9 q
 
@@ -315,14 +315,14 @@ __global__ void __launch_bounds__(kSumWarps * 32) offset_sum_kernel(const DemodA
 #pragma unroll
             for (int u = 0; u < kGroup; ++u) {
                 const int m = m0 + kSpb * u;
-                const bool ok = mine && m < a.n_new && a.seen + m >= kCorrLen + 7;     // ring full (decoder.C:181)
+                const bool ok = mine && m < a.n_new && m >= m_full;
                 s_os[warp][kk][u][j] = ok ? acc[u] : 0.0;
             }
         }
         __syncwarp();
         if (judge) {
             const int w = w_first + kSpb * (r0 + u2);
-            if (w >= 0 && w < a.n_new && a.seen + w >= kCorrLen + 15) {
+            if (w >= 0 && w < a.n_new && w >= w_full) {
                 double best = -1.0;
                 int pick = 0;
 #pragma unroll
@@ -381,13 +381,13 @@ __global__ void __launch_bounds__(kSeqWarps * 32) symbol_clock_kernel(const Demo
     const int seen9 = (int)(a.seen % kSpb);
     const int e0 = (6 - seen9 + kSpb) % kSpb;
     const int n_eval = e0 < a.n_new ? (a.n_new - 1 - e0) / kSpb + 1 : 0;
-    int q = 0;
-    {
-        const long long need = kCorrLen + 15 - a.seen - e0;
-        if (need > 0) q = (int)((need + kSpb - 1) / kSpb);
-        if (q > n_eval) q = n_eval;
+    int q = n_eval;
+    if (live) {     // the first evaluation after the channel's ring filled (its epoch: nvx_engine_reset_streams)
+        const long long need = kCorrLen + 15 - (a.seen - a.b.epoch[ch]) - e0;
+        q = need > 0 ? (int)min((need + kSpb - 1) / kSpb, (long long)n_eval) : 0;
     }
-    for (int c0 = (q / kSeqChunk) * kSeqChunk; c0 < n_eval || c0 == 0; c0 += kSeqChunk) {
+    const int q_warp = __reduce_min_sync(0xffffffffu, q);         // the chunks are staged by the whole warp
+    for (int c0 = (q_warp / kSeqChunk) * kSeqChunk; c0 < n_eval || c0 == 0; c0 += kSeqChunk) {
         const int c1 = min(n_eval, c0 + kSeqChunk);
         if (c1 > c0) stage_rows(rows, a.b.picks, pitch_p(a.b.p_max), ch0, a.channels, c0, c1 - c0, lane);
         const int lim = c1 == n_eval ? a.n_new : e0 + kSpb * c1;          // samples whose evaluations are staged
@@ -527,13 +527,8 @@ __global__ void init_state_kernel(ClockState* clock, FsmState* fsm, int channels
     const int ch = blockIdx.x * blockDim.x + threadIdx.x;
     if (ch >= channels) return;
     // decoder::decoder (decoder.C:6-39) and byte_state_machine::init (nav_b_sm.C:16-42)
-    ClockState c = {};
-    c.last_pick = -1;
-    c.dstate = DS_INIT;
-    clock[ch] = c;
-    FsmState s = {};
-    s.byte_state = BY_WAIT;
-    fsm[ch] = s;
+    clock[ch] = clock_state_init();
+    fsm[ch] = fsm_state_init();
 }
 
 }  // namespace
@@ -582,6 +577,7 @@ cudaError_t demod_init_state(const DemodBuffers& b, int channels, cudaStream_t s
     if ((e = cudaMemsetAsync(b.y3, 0, sizeof(float2) * (size_t)channels * (kHistY + b.p_max), stream)) != cudaSuccess) return e;
     if ((e = cudaMemsetAsync(b.corr, 0, sizeof(double) * (size_t)channels * (kHistC + b.p_max + kPadC), stream)) != cudaSuccess) return e;
     if ((e = cudaMemsetAsync(b.picks, 0, (size_t)channels * pitch_p(b.p_max), stream)) != cudaSuccess) return e;
+    if ((e = cudaMemsetAsync(b.epoch, 0, sizeof(long long) * (size_t)channels, stream)) != cudaSuccess) return e;
     init_state_kernel<<<(channels + 127) / 128, 128, 0, stream>>>(b.clock, b.fsm, channels);
     return cudaGetLastError();
 }
@@ -593,7 +589,10 @@ cudaError_t demod_launch(const DemodArgs& a, cudaStream_t s_ff, cudaStream_t s_s
     mark(0, s_ff);
     angle_corr_kernel<<<dim3((a.n_new + kTile - 1) / kTile, a.channels), kThreads, 0, s_ff>>>(a);
     mark(1, s_ff);
-    {   // ring revolutions with an evaluation sample in [-8, n_new): samples 16 + 567 K .. 582 + 567 K
+    // Ring revolutions with an evaluation sample in [-8, n_new): samples 16 + 567 K .. 582 + 567 K.  The revolutions are counted
+    // on the absolute grid, whatever the channels' epochs: epochs are multiples of 567, so a channel's revolutions are the ones a
+    // fresh engine would walk, and those before its ring filled produce sums and picks that its epoch-relative gates discard.
+    {
         const long long lo = a.seen - 8 - (kCorrLen + 15), hi = a.seen + a.n_new - 17;
         const int k_lo = lo <= 0 ? 0 : (int)((lo + kCorrLen - 1) / kCorrLen);
         if (hi >= 0 && (int)(hi / kCorrLen) >= k_lo) {

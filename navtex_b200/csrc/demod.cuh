@@ -16,6 +16,9 @@ constexpr int kHistY = 16;              // 900 Hz samples (angle needs 1, mask c
 constexpr int kHistC = 640;             // |mask correlation| values (the per-offset sum threads reach back up to 628)
 constexpr int kPadC = 64;               // readable slack behind the new samples (a thread's running prefix may run 46 past the block)
 
+enum { DS_INIT = 0, DS_WAIT = 1, DS_PENDING = 2 };   // decoder.h:16-19 (BIT_START / RECEIVING folded into PENDING)
+enum { BY_WAIT = 1, BY_GOT_DX = 2, BY_GOT_RX = 3 };  // nav_b_sm.h:41-43
+
 // What decoder.{h,C} keeps per channel and that is genuinely sequential: the slew-limited offset tracker and the
 // symbol clock of the mark/space discriminator (decoder.C:73-137, :217-249), in event form.
 struct ClockState {
@@ -36,6 +39,19 @@ struct FsmState {
     int eoe_count, prev_dx_alpha, holdoff, enabled;
 };
 
+// a channel's state at create: decoder::decoder (decoder.C:6-39) and byte_state_machine::init (nav_b_sm.C:16-42)
+__host__ __device__ inline ClockState clock_state_init() {
+    ClockState c = {};
+    c.last_pick = -1;
+    c.dstate = DS_INIT;
+    return c;
+}
+__host__ __device__ inline FsmState fsm_state_init() {
+    FsmState s = {};
+    s.byte_state = BY_WAIT;
+    return s;
+}
+
 struct DemodBuffers {
     float2* y3;               // [channels][kHistY + p_max]   (the cascade kernel writes at +kHistY); one per block in flight
     double* corr;             // [channels][kHistC + p_max + kPadC]   |mask correlation| per sample (two buffers, alternating per block)
@@ -45,6 +61,9 @@ struct DemodBuffers {
     int* nbits;               // [channels]              bits decided in the block
     ClockState* clock;        // [channels]
     FsmState* fsm;            // [channels]
+    // [channels] the channel's epoch: the 900 Hz sample its decoder (re)started at -- 0 from create and nvx_engine_reset, the
+    // E0 of nvx_engine_reset_streams after that.  Warm-up conditions count from it; the sample grids stay absolute.
+    long long* epoch;
     int p_max;
 };
 

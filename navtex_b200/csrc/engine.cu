@@ -12,7 +12,9 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <algorithm>
 #include <condition_variable>
+#include <deque>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -90,6 +92,70 @@ __global__ void tail_carry_kernel(const Sample* __restrict__ old_tail, const Sam
     *reinterpret_cast<int4*>(new_tail + (size_t)s * halo + k) = *src;
 }
 
+// nvx_config.nco_hz entry f -> its NCO row; false if f is off the 0.5 Hz grid or outside +-31.5 kHz
+bool nco_entry(double f, nvx::NcoChan* out) {
+    const double twice = 2.0 * f;
+    if (!(fabs(f) < 31500.0) || twice != nearbyint(twice)) return false;
+    long long num = (long long)twice % nvx::kNcoDen;
+    if (num < 0) num += nvx::kNcoDen;
+    out->num = (int)num;
+    out->phase0 = 0;
+    // same expression as fir2cpp.C:105-106 for table entry 1, rounded once to float
+    out->step = make_float2((float)cos((2 * M_PI * 1 * f) / 63000), (float)-sin((2 * M_PI * 1 * f) / 63000));
+    return true;
+}
+
+// Everything the next block would carry over from the past of the listed streams, cleared so that each restarts as an engine
+// created at its epoch e0 (nvx_engine_reset_streams).  Queued on the engine stream in push order, after the previous block's
+// sequential demod kernels (they still read its y3 buffer and the decoder state) and before this block's cascade.
+struct ResetArgs {
+    const int* streams;                 // [gridDim.x] local stream indices
+    int C;                              // channels per stream
+    long long e0;                       // the new epoch, 900 Hz samples (a multiple of 567)
+    uint32_t* tail;                     // fused path: the [S][tail_words] input tail the next block reads, else null
+    long long tail_words;
+    uint32_t tail_fill;                 // silence in the pushed format (0x80 bytes for 8-bit pairs)
+    nvx::LongHist lh;                   // long-tap path: the stage histories the next block reads (rows null without it)
+    float2* y3_prev;                    // the previous block's y3 / corr buffers, whose ends become this block's histories
+    long long y3_pitch;
+    double* corr_prev;
+    long long corr_pitch;
+    int n_prev;
+    nvx::ClockState* clock;
+    nvx::FsmState* fsm;
+    long long* epoch;
+    nvx::NcoChan* nco;                  // general-NCO rows (their phase origin moves to e0), or null: the reference table
+};
+
+// one CTA per listed stream
+__global__ void reset_streams_kernel(const ResetArgs a) {
+    const int s = a.streams[blockIdx.x];
+    const int t = threadIdx.x, nt = blockDim.x;
+    if (a.tail)
+        for (long long i = t; i < a.tail_words; i += nt) a.tail[(size_t)s * a.tail_words + i] = a.tail_fill;
+    for (int k = 0; k < 3; ++k)
+        if (a.lh.rows[k]) {
+            const long long len = (long long)a.lh.per_stream[k] * a.lh.H[k];
+            for (long long i = t; i < len; i += nt) a.lh.rows[k][(size_t)s * len + i] = make_float2(0.f, 0.f);
+        }
+    for (int c = 0; c < a.C; ++c) {
+        const size_t ch = (size_t)s * a.C + c;
+        for (int i = t; i < nvx::kHistY; i += nt) a.y3_prev[ch * a.y3_pitch + a.n_prev + i] = make_float2(0.f, 0.f);
+        for (int i = t; i < nvx::kHistC; i += nt) a.corr_prev[ch * a.corr_pitch + a.n_prev + i] = 0.0;
+    }
+    if (t < a.C) {
+        const size_t ch = (size_t)s * a.C + t;
+        a.clock[ch] = nvx::clock_state_init();
+        a.fsm[ch] = nvx::fsm_state_init();
+        a.epoch[ch] = a.e0;
+        if (a.nco) {     // the stage-1 output at e0 is number 70 e0; its phase becomes 0
+            const long long k0 = a.e0 * (nvx::kSuper / NVX_D1) % nvx::kNcoDen;
+            const int p = (int)(k0 * a.nco[ch].num % nvx::kNcoDen);
+            a.nco[ch].phase0 = p ? nvx::kNcoDen - p : 0;
+        }
+    }
+}
+
 }  // namespace
 
 constexpr int kBuf = 3;   // blocks in flight: cascade of block i+1/i+2 overlaps demod + event download of block i
@@ -130,8 +196,21 @@ struct nvx_engine {
     bool custom_taps = false;
     nvx::CascadeTaps taps;                // this engine's filter constants: passed in the parameter block of every cascade launch
     nvx::NcoChan* d_nco_ch = nullptr;     // [S][C] per-stream NCO parameters (nvx_config.nco_hz), else null: the reference table
+    std::vector<nvx::NcoChan> nco_host;   // the same rows with phase origin 0 (retunes edit them here first)
     nvx::LongPath* lp = nullptr;          // tap sets too long for the fused kernel: the three stage kernels (fir_long.cuh), else null
-    std::vector<int> stream_tag;          // optional [S][2] message tags
+    std::vector<int> stream_tag;          // optional [S][C] message tags (read by the worker; changed through markers)
+    // per-stream resets and retunes asked for since the last push; the next push applies them
+    struct TagChange { int stream; std::vector<int> tags; };
+    enum { kListed = 1, kNewNco = 2 };
+    std::vector<int> pend_streams;        // in call order, each once
+    std::vector<uint8_t> pend_flags;      // [S] kListed | kNewNco
+    std::vector<TagChange> pend_tags;
+    int* d_reset_list = nullptr;          // [S] the streams of one push's reset kernel
+    void* h_reset = nullptr;              // pinned: [S][C] NcoChan rows to upload, then [S] ints (the list)
+    cudaEvent_t reset_copied = nullptr;   // the copies out of h_reset are over
+    // what the worker does before it assembles block `block`: drop the reset streams' partial lines and messages, switch tags
+    struct Marker { long long block; std::vector<int> streams; std::vector<TagChange> tags; };
+    std::deque<Marker> markers;           // guarded by mu, in push order
     int target_warps[nvx::kSampleFmts] = {576, 576, 576};   // resident cascade warps per sample format
     nvx::MessageAssembler assembler;
     std::vector<nvx::AssembledMessage> ready, handed;
@@ -183,6 +262,8 @@ int free_engine(nvx_engine* e) {
     }
     if (e->stream_copy) cudaStreamDestroy(e->stream_copy);
     cudaFree(e->d_nco_ch);
+    cudaFree(e->db.epoch); cudaFree(e->d_reset_list); cudaFreeHost(e->h_reset);
+    if (e->reset_copied) cudaEventDestroy(e->reset_copied);
     nvx::long_path_free(e->lp);
     for (int k = 0; k < kBuf; ++k) {
         cudaFree(e->y3buf[k]); cudaFree(e->d_events[k]); cudaFree(e->d_ev_count[k]);
@@ -197,8 +278,21 @@ int free_engine(nvx_engine* e) {
     return 0;
 }
 
+void set_tags(nvx_engine* e, const nvx_engine::TagChange& t) {
+    if (e->stream_tag.empty())
+        for (int ch = 0; ch < e->channels; ++ch) e->stream_tag.push_back(e->cfg.freq_tag[(ch % e->C) & 1]);
+    std::copy(t.tags.begin(), t.tags.end(), e->stream_tag.begin() + (size_t)t.stream * e->C);
+}
+
 int reset_state(nvx_engine* e) {
     e->fmt = -1;                                    // the next push fixes the format and fills the fused path's tail
+    // per-stream resets still pending are part of this one; their new tags take effect now, their offsets are in nco_host
+    for (const auto& t : e->pend_tags) set_tags(e, t);
+    for (int s : e->pend_streams) e->pend_flags[(size_t)s] = 0;
+    e->pend_streams.clear();
+    e->pend_tags.clear();
+    if (e->d_nco_ch)   // every row's phase origin back to 0
+        CU_TRY(cudaMemcpyAsync(e->d_nco_ch, e->nco_host.data(), e->nco_host.size() * sizeof(nvx::NcoChan), cudaMemcpyHostToDevice, e->stream));
     if (e->lp) CU_TRY(nvx::long_path_reset(e->lp, e->stream));
     for (int k = 0; k < kBuf; ++k) {
         e->db.y3 = e->y3buf[k];
@@ -216,6 +310,7 @@ int reset_state(nvx_engine* e) {
         std::lock_guard<std::mutex> lk(e->mu);
         e->queued = e->drained = 0;
         e->worker_rc = 0;
+        e->markers.clear();
     }
     e->assembler.reset();
     e->ready.clear();
@@ -293,6 +388,19 @@ void worker_main(nvx_engine* e) {
             blk = e->drained;
         }
         const int b = (int)(blk % kBuf);
+        std::vector<nvx_engine::Marker> take;
+        {
+            std::lock_guard<std::mutex> lk(e->mu);
+            while (!e->markers.empty() && e->markers.front().block <= blk) {
+                take.push_back(std::move(e->markers.front()));
+                e->markers.pop_front();
+            }
+        }
+        for (const auto& m : take) {       // blocks before this one were assembled under the old state and tags
+            for (int s : m.streams)
+                for (int c = 0; c < e->C; ++c) e->assembler.reset_channel(s * e->C + c);
+            for (const auto& t : m.tags) set_tags(e, t);
+        }
         int rc = 0;
         if (cudaEventSynchronize(e->demod_done[b]) != cudaSuccess) rc = NVX_ERR_CUDA;
         else rc = drain_events(e, b);
@@ -355,6 +463,66 @@ int long_report(nvx_engine* e, int rc, const nvx::LongReport& rep) {
     return rc;
 }
 
+// the resets asked for since the last push, queued in front of this block (b = its buffer index): NCO rows of retuned streams,
+// the reset kernel, and the marker that tells the worker from which block on the streams' messages start over
+int apply_resets(nvx_engine* e, nvx::SampleFmt fmt, int b) {
+    using namespace nvx;
+    const int count = (int)e->pend_streams.size();
+    if (!count) return 0;
+    const size_t rows_bytes = (size_t)e->S * e->C * sizeof(NcoChan);
+    if (!e->d_reset_list) {
+        CU_TRY(cudaMalloc(&e->d_reset_list, (size_t)e->S * sizeof(int)));
+        CU_TRY(cudaHostAlloc(&e->h_reset, rows_bytes + (size_t)e->S * sizeof(int), cudaHostAllocDefault));
+        CU_TRY(cudaEventCreateWithFlags(&e->reset_copied, cudaEventDisableTiming));
+    } else {
+        CU_TRY(cudaEventSynchronize(e->reset_copied));      // the previous copies out of h_reset are over
+    }
+    NcoChan* h_rows = static_cast<NcoChan*>(e->h_reset);
+    int* h_list = reinterpret_cast<int*>(static_cast<char*>(e->h_reset) + rows_bytes);
+    int retuned = 0;
+    for (int i = 0; i < count; ++i) {
+        const int s = e->pend_streams[(size_t)i];
+        h_list[i] = s;
+        if (e->pend_flags[(size_t)s] & nvx_engine::kNewNco) {
+            NcoChan* src = h_rows + (size_t)retuned++ * e->C;
+            memcpy(src, &e->nco_host[(size_t)s * e->C], e->C * sizeof(NcoChan));
+            CU_TRY(cudaMemcpyAsync(e->d_nco_ch + (size_t)s * e->C, src, e->C * sizeof(NcoChan), cudaMemcpyHostToDevice, e->stream));
+        }
+        e->pend_flags[(size_t)s] = 0;
+    }
+    CU_TRY(cudaMemcpyAsync(e->d_reset_list, h_list, (size_t)count * sizeof(int), cudaMemcpyHostToDevice, e->stream));
+    CU_TRY(cudaEventRecord(e->reset_copied, e->stream));
+    if (e->blocks > 0) CU_TRY(cudaStreamWaitEvent(e->stream, e->demod_done[e->last_buf], 0));
+    ResetArgs ra = {};
+    ra.streams = e->d_reset_list;
+    ra.C = e->C;
+    ra.e0 = e->sb_abs - e->sb_abs % kCorrLen;
+    if (!e->lp) {
+        ra.tail = static_cast<uint32_t*>(e->tail[e->tail_cur]);
+        ra.tail_words = (long long)e->halo * sample_bytes(fmt) / 4;
+        ra.tail_fill = fmt == SampleFmt::U8 ? 0x80808080u : 0u;
+    } else {
+        ra.lh = long_path_hist(e->lp);
+    }
+    ra.y3_prev = e->y3buf[(b + kBuf - 1) % kBuf];
+    ra.y3_pitch = kHistY + e->P_max;
+    ra.corr_prev = e->corrbuf[(e->blocks & 1) ^ 1];
+    ra.corr_pitch = kHistC + e->P_max + kPadC;
+    ra.n_prev = e->last_P;
+    ra.clock = e->db.clock; ra.fsm = e->db.fsm; ra.epoch = e->db.epoch;
+    ra.nco = e->d_nco_ch;
+    reset_streams_kernel<<<(unsigned)count, 256, 0, e->stream>>>(ra);
+    CU_TRY(cudaGetLastError());
+    e->stats.aux_launches++;
+    {
+        std::lock_guard<std::mutex> lk(e->mu);
+        e->markers.push_back({e->blocks, std::move(e->pend_streams), std::move(e->pend_tags)});
+    }
+    e->pend_streams.clear();
+    e->pend_tags.clear();
+    return 0;
+}
+
 int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fmt) {
     using namespace nvx;
     if (e->fmt >= 0 && e->fmt != (int)fmt)
@@ -372,6 +540,7 @@ int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fm
     if (((uintptr_t)d_x & 15) != 0) return fail(NVX_ERR_ARG, "device block is not 16-byte aligned");
     const int b = (int)(e->blocks % kBuf);
     wait_drained(e, e->blocks - kBuf + 1);          // block (blocks - kBuf) used these buffers: long finished, normally
+    if (int rc = apply_resets(e, fmt, b)) return rc;
     if (e->timing && e->ev_used > 4000) {            // bound the event pool in long timed runs
         CU_TRY(cudaStreamSynchronize(e->stream));
         CU_TRY(cudaStreamSynchronize(e->stream_demod));
@@ -555,24 +724,17 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
     if ((long long)C * cfg->n_streams > 65535) { delete e; return fail(NVX_ERR_ARG, "n_streams x n_channels = %lld exceeds 65535 channel rows per engine", (long long)C * cfg->n_streams); }
     e->C = C;
     if (cfg->stream_freq_tag) e->stream_tag.assign(cfg->stream_freq_tag, cfg->stream_freq_tag + (size_t)C * (size_t)cfg->n_streams);
-    std::vector<nvx::NcoChan> nco;
     if (cfg->nco_hz) {
-        nco.resize((size_t)cfg->n_streams * C);
-        for (int k = 0; k < C * cfg->n_streams; ++k) {
-            const double f = cfg->nco_hz[k], twice = 2.0 * f;
-            if (!(fabs(f) < 31500.0) || twice != nearbyint(twice)) {
+        e->nco_host.resize((size_t)cfg->n_streams * C);
+        for (int k = 0; k < C * cfg->n_streams; ++k)
+            if (!nco_entry(cfg->nco_hz[k], &e->nco_host[(size_t)k])) {
                 delete e;
-                return fail(NVX_ERR_ARG, "nco_hz[%d] = %g is not a multiple of 0.5 Hz inside +-31.5 kHz", k, f);
+                return fail(NVX_ERR_ARG, "nco_hz[%d] = %g is not a multiple of 0.5 Hz inside +-31.5 kHz", k, cfg->nco_hz[k]);
             }
-            long long num = (long long)twice % nvx::kNcoDen;
-            if (num < 0) num += nvx::kNcoDen;
-            // same expression as fir2cpp.C:105-106 for table entry 1, rounded once to float
-            nco[(size_t)k].num = (int)num;
-            nco[(size_t)k].step = make_float2((float)cos((2 * M_PI * 1 * f) / 63000), (float)-sin((2 * M_PI * 1 * f) / 63000));
-        }
     }
     e->S = cfg->n_streams;
     e->channels = C * e->S;
+    e->pend_flags.assign((size_t)e->S, 0);
     e->P_max = (int)(cfg->max_block / nvx::kSuper);
     e->custom_taps = cfg->h1 || cfg->h2 || cfg->h3;
     // tap counts: reference lengths unless given; sets up to 37/47/71 and up to 61/75/111 run through the fused kernel
@@ -629,6 +791,7 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
     CREATE_TRY(cudaMemset(e->db.nbits, 0, (size_t)e->channels * sizeof(int)));
     CREATE_TRY(cudaMalloc(&e->db.clock, (size_t)e->channels * sizeof(nvx::ClockState)));
     CREATE_TRY(cudaMalloc(&e->db.fsm, (size_t)e->channels * sizeof(nvx::FsmState)));
+    CREATE_TRY(cudaMalloc(&e->db.epoch, (size_t)e->channels * sizeof(long long)));
     for (int k = 0; k < kBuf; ++k) {
         CREATE_TRY(cudaMalloc(&e->d_events[k], (size_t)e->channels * e->ev_cap));
         CREATE_TRY(cudaMalloc(&e->d_ev_count[k], sizeof(int) * e->channels));
@@ -643,10 +806,7 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
         CREATE_TRY(cudaMalloc(&e->d_bit_count, sizeof(int) * e->channels));
         CREATE_TRY(cudaMemset(e->d_bit_count, 0, sizeof(int) * e->channels));
     }
-    if (!nco.empty()) {
-        CREATE_TRY(cudaMalloc(&e->d_nco_ch, nco.size() * sizeof(nvx::NcoChan)));
-        CREATE_TRY(cudaMemcpy(e->d_nco_ch, nco.data(), nco.size() * sizeof(nvx::NcoChan), cudaMemcpyHostToDevice));
-    }
+    if (!e->nco_host.empty()) CREATE_TRY(cudaMalloc(&e->d_nco_ch, e->nco_host.size() * sizeof(nvx::NcoChan)));   // filled by reset_state
     if (e->tap_class < 0) {
         const double* const h[3] = {cfg->h1, cfg->h2, cfg->h3};
         nvx::LongReport rep;
@@ -677,6 +837,31 @@ int nvx_engine_reset(nvx_engine* e) {
         e->ready.clear();
     }
     return reset_state(e);
+}
+
+int nvx_engine_reset_streams(nvx_engine* e, const int* streams, int count) {
+    if (!e || count < 0 || (count && !streams)) return fail(NVX_ERR_ARG, "bad argument");
+    for (int i = 0; i < count; ++i)
+        if (streams[i] < 0 || streams[i] >= e->S) return fail(NVX_ERR_ARG, "stream %d outside 0..%d", streams[i], e->S - 1);
+    for (int i = 0; i < count; ++i) {
+        uint8_t& f = e->pend_flags[(size_t)streams[i]];
+        if (!(f & nvx_engine::kListed)) e->pend_streams.push_back(streams[i]);
+        f |= nvx_engine::kListed;
+    }
+    return 0;
+}
+
+int nvx_engine_retune_stream(nvx_engine* e, int stream, const double* nco_hz, const int* freq_tag) {
+    if (!e || !nco_hz || stream < 0 || stream >= e->S) return fail(NVX_ERR_ARG, "bad argument");
+    if (e->nco_host.empty()) return fail(NVX_ERR_ARG, "engine was created without nco_hz: its reference-table channels cannot be retuned");
+    std::vector<nvx::NcoChan> rows((size_t)e->C);
+    for (int c = 0; c < e->C; ++c)
+        if (!nco_entry(nco_hz[c], &rows[(size_t)c]))
+            return fail(NVX_ERR_ARG, "nco_hz[%d] = %g is not a multiple of 0.5 Hz inside +-31.5 kHz", c, nco_hz[c]);
+    std::copy(rows.begin(), rows.end(), e->nco_host.begin() + (size_t)stream * e->C);
+    if (freq_tag) e->pend_tags.push_back({stream, std::vector<int>(freq_tag, freq_tag + e->C)});
+    e->pend_flags[(size_t)stream] |= nvx_engine::kNewNco;
+    return nvx_engine_reset_streams(e, &stream, 1);
 }
 
 int nvx_engine_push_device_f32(nvx_engine* e, const void* d_iq, long long n) {

@@ -86,7 +86,7 @@ __global__ void __launch_bounds__(InFmt<kFmt, kClass, kCh>::kWarps * 32, kCtasPe
 #pragma unroll
         for (int c = 0; c < kCh; ++c) {
             const NcoChan pc = np[c];
-            nco_idx[c] = (int)((k0 * pc.num) % kNcoDen);
+            nco_idx[c] = (int)((k0 * pc.num + pc.phase0) % kNcoDen);
             nco_adv[c] = (int)(((long long)NVX_D2 * pc.num) % kNcoDen);
             nl.step[c] = pc.step;
         }

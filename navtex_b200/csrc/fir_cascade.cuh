@@ -172,6 +172,9 @@ constexpr int kNcoDen = 126000;
 // general-NCO variants and the long-tap path's stage 1 (two channels: entries 2 row + c) read the same array
 struct NcoChan {
     int num;           // (2 f) mod 126000
+    // (-(E0 / 4) num) mod 126000, added to every exact phase numerator: the row's phase is 0 at its epoch E0 (input samples;
+    // nvx_engine_reset_streams), as in an engine created there.  0 from create and nvx_engine_reset.
+    int phase0;
     float2 step;       // (cos, -sin)(2 pi f / 63000)
 };
 constexpr int kMaxFusedCh = 4;   // channels one pass of the fused kernel carries in registers (9 + 14 per channel complex partial sums)

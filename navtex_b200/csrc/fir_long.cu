@@ -146,8 +146,9 @@ __global__ void __launch_bounds__(long_threads(D)) fir_long_kernel(const LongArg
         // NCO mix: output k sits at 63 kHz clock tick k_abs + k; channel c gets y1 * (cos - j sin)(2 pi tick f_c / 63000)
         float2* out0 = a.out + (size_t)(2 * row_in) * a.out_pitch + a.out_off + k0 + (long long)kLongR * t;
         float2* out1 = out0 + a.out_pitch;
-        int num[2] = {0, 0};
-        if (a.nco) { num[0] = a.nco[2 * row_in].num; num[1] = a.nco[2 * row_in + 1].num; }
+        int num[2] = {0, 0}, phase0[2] = {0, 0};
+        if (a.nco)
+            for (int c = 0; c < 2; ++c) { num[c] = a.nco[2 * row_in + c].num; phase0[c] = a.nco[2 * row_in + c].phase0; }
         const long long tick0 = a.k_abs + k0 + (long long)kLongR * t;
         long long r9 = tick0 % kNcoPeriod, rden = tick0 % kNcoDen;
         int k9 = (int)(r9 < 0 ? r9 + kNcoPeriod : r9), kden = (int)(rden < 0 ? rden + kNcoDen : rden);
@@ -157,7 +158,7 @@ __global__ void __launch_bounds__(long_threads(D)) fir_long_kernel(const LongArg
             if (a.nco) {
 #pragma unroll
                 for (int c = 0; c < 2; ++c) {
-                    const int ph = (int)(((long long)kden * num[c]) % kNcoDen);
+                    const int ph = (int)(((long long)kden * num[c] + phase0[c]) % kNcoDen);
                     float tt = (float)ph * (2.0f / kNcoDen);
                     if (tt > 1.0f) tt -= 2.0f;
                     float sn, cs;
@@ -375,6 +376,16 @@ cudaError_t long_path_reset(LongPath* lp, cudaStream_t stream) {
     for (int k = 0; k < 3; ++k)
         for (int q = 0; q < 2 && e == cudaSuccess; ++q) e = cudaMemsetAsync(lp->hist[k][q], 0, hist_bytes(lp, k), stream);
     return e;
+}
+
+LongHist long_path_hist(const LongPath* lp) {
+    LongHist h;
+    for (int k = 0; k < 3; ++k) {
+        h.rows[k] = lp->hist[k][lp->cur];
+        h.H[k] = lp->st[k].H;
+        h.per_stream[k] = k == 0 || (k == 1 && lp->mix_on_load) ? 1 : 2;
+    }
+    return h;
 }
 
 // 3 stage launches and 3 history carries: 5 in nvx_stats.aux_launches, where the engine counts one per block for every path

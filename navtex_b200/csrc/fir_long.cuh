@@ -88,6 +88,13 @@ struct LongReport {
 int long_path_create(int S, long long max_block, const int n[3], const double* const h[3], const NcoChan* nco, cudaStream_t stream,
                      LongPath** out, LongReport* rep);
 cudaError_t long_path_reset(LongPath* lp, cudaStream_t stream);     // zero histories: the next block starts after silence
+// the histories the next block reads: stage k keeps per_stream[k] consecutive rows of H[k] float2 for each stream (1 for stage 1,
+// 2 for stages 2 and 3 -- one per channel -- or 1 for stage 2 when it mixes on load); zeroing a stream's rows restarts its filters
+struct LongHist {
+    float2* rows[3];
+    int H[3], per_stream[3];
+};
+LongHist long_path_hist(const LongPath* lp);
 // one block x[S][n] in format fmt whose first 63 kHz output sits at tick; the 900 Hz output goes to y3[2 S][y3_pitch] from
 // y3_off on.  Returns 0 or an NVX_ERR_* code.
 int long_path_run(LongPath* lp, const void* x, long long n, SampleFmt fmt, long long tick, float2* y3, long long y3_pitch,

@@ -511,11 +511,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) fir_tc_kernel(const __grid_cons
                     const long long kden = rden < 0 ? rden + kNcoDen : rden;
 #pragma unroll 2
                     for (int r = 0; r < r_max; ++r, dst += 2 * a.out_pitch) {
-                        const int num[2] = {a.nco[2 * (row0 + r)].num, a.nco[2 * (row0 + r) + 1].num};
+                        const NcoChan nc[2] = {a.nco[2 * (row0 + r)], a.nco[2 * (row0 + r) + 1]};
                         const float2 y = make_float2(rows0[r * kDumpPitch + m], rows0[r * kDumpPitch + NP + m]);
 #pragma unroll
                         for (int c = 0; c < 2; ++c) {
-                            const int phs = (int)((kden * num[c]) % kNcoDen);
+                            const int phs = (int)((kden * nc[c].num + nc[c].phase0) % kNcoDen);
                             float tt = (float)phs * (2.0f / kNcoDen);
                             if (tt > 1.0f) tt -= 2.0f;
                             float sn, cs;
@@ -984,11 +984,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) fir_tcs_kernel(const __grid_con
                             const long long kden = rden < 0 ? rden + kNcoDen : rden;
 #pragma unroll 2
                             for (int rr = 0; rr < r_max; ++rr, dst += 2 * a.out_pitch) {
-                                const int num[2] = {a.nco[2 * (row0 + rr)].num, a.nco[2 * (row0 + rr) + 1].num};
+                                const NcoChan nc[2] = {a.nco[2 * (row0 + rr)], a.nco[2 * (row0 + rr) + 1]};
                                 const float2 y = make_float2(rows0[rr * kDumpPitch + m], rows0[rr * kDumpPitch + NP + m]);
 #pragma unroll
                                 for (int c = 0; c < 2; ++c) {
-                                    const int phs = (int)((kden * num[c]) % kNcoDen);
+                                    const int phs = (int)((kden * nc[c].num + nc[c].phase0) % kNcoDen);
                                     float tt = (float)phs * (2.0f / kNcoDen);
                                     if (tt > 1.0f) tt -= 2.0f;
                                     float sn, cs;

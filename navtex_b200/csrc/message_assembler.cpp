@@ -24,6 +24,7 @@ MessageAssembler::~MessageAssembler() {
 
 void MessageAssembler::resize(int channels) { ch_.assign((size_t)channels, Channel()); }
 void MessageAssembler::reset() { ch_.assign(ch_.size(), Channel()); }
+void MessageAssembler::reset_channel(int ch) { ch_[(size_t)ch] = Channel(); }
 
 namespace {
 // Necessary conditions of the two patterns, checked before paying for regexec (most lines are plain text):

@@ -23,6 +23,8 @@ class MessageAssembler {
 
     void resize(int channels);
     void reset();
+    // drop channel ch's partial line and message without delivering them (nvx_engine_reset_streams)
+    void reset_channel(int ch);
     // feed `n` event bytes of channel `ch`; completed messages are appended to `out`
     void feed(int ch, int stream, int freq, const unsigned char* ev, size_t n, std::vector<AssembledMessage>* out);
 

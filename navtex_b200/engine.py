@@ -49,13 +49,14 @@ class SynthDesc(C.Structure):
 
 EXPORTS = (
     "nvx_default_config", "nvx_last_error", "nvx_engine_create", "nvx_engine_destroy", "nvx_engine_reset",
+    "nvx_engine_reset_streams", "nvx_engine_retune_stream",
     "nvx_engine_push_host_f32", "nvx_engine_push_host_s16", "nvx_engine_push_host_u8", "nvx_engine_push_device_f32",
     "nvx_engine_push_device_s16", "nvx_engine_push_device_u8",
     "nvx_engine_sync", "nvx_engine_wait_ingest", "nvx_engine_host_pushes", "nvx_engine_wait_ingest_of", "nvx_engine_poll_messages", "nvx_engine_try_poll_messages", "nvx_engine_set_message_callback", "nvx_engine_read_y3",
     "nvx_engine_read_bits", "nvx_engine_read_events", "nvx_engine_enable_timing", "nvx_engine_get_stats",
     "nvx_engine_stream", "nvx_engine_get_cascade_spans", "nvx_engine_fence", "nvx_pinned_alloc", "nvx_pinned_free", "nvx_synth_fill_device", "nvx_host_assemble", "nvx_debug_long_tc_band",
     "nvx_capture_create", "nvx_capture_create_u8", "nvx_capture_destroy", "nvx_capture_write", "nvx_capture_write_u8", "nvx_capture_pump",
-    "nvx_capture_start", "nvx_capture_stop",
+    "nvx_capture_start", "nvx_capture_stop", "nvx_capture_detach", "nvx_capture_attach",
     "nvx_capture_dropped", "nvx_store_create", "nvx_store_destroy", "nvx_store_add", "nvx_store_add_at", "nvx_store_sink",
     "nvx_store_count", "nvx_store_get", "nvx_store_purge", "nvx_store_dump_csv",
 )
@@ -79,6 +80,8 @@ def load_library():
     L.nvx_engine_destroy.argtypes = [C.c_void_p]
     L.nvx_engine_destroy.restype = None
     L.nvx_engine_reset.argtypes = [C.c_void_p]
+    L.nvx_engine_reset_streams.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.c_int]
+    L.nvx_engine_retune_stream.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_int)]
     for name in ("nvx_engine_push_host_f32", "nvx_engine_push_host_s16", "nvx_engine_push_host_u8", "nvx_engine_push_device_f32",
                  "nvx_engine_push_device_s16", "nvx_engine_push_device_u8"):
         getattr(L, name).argtypes = [C.c_void_p, C.c_void_p, C.c_longlong]
@@ -115,6 +118,8 @@ def load_library():
     L.nvx_capture_dropped.argtypes = [C.c_void_p, C.c_int]
     L.nvx_capture_start.argtypes = [C.c_void_p, C.c_int]
     L.nvx_capture_stop.argtypes = [C.c_void_p]
+    L.nvx_capture_detach.argtypes = [C.c_void_p, C.c_int]
+    L.nvx_capture_attach.argtypes = [C.c_void_p, C.c_int]
     L.nvx_store_create.restype = C.c_void_p
     L.nvx_store_destroy.argtypes = [C.c_void_p]
     L.nvx_store_destroy.restype = None
@@ -205,6 +210,26 @@ class Engine:
 
     def reset(self):
         _check(self.L.nvx_engine_reset(self._h))
+
+    def reset_streams(self, streams):
+        """Restart the listed streams (local indices) at the next push, as if the engine had just been created for them; the
+        other streams are untouched.  The restart sits on the shared 158 760-sample grid (nvx_engine_reset_streams)."""
+        s = np.ascontiguousarray(streams, dtype=np.int32).reshape(-1)
+        _check(self.L.nvx_engine_reset_streams(self._h, s.ctypes.data_as(C.POINTER(C.c_int)), s.size))
+
+    def retune_stream(self, stream: int, nco_hz, freq_tag=None):
+        """New channel offsets [n_channels] (Hz) and optionally tags for one stream of an engine created with nco_hz; implies
+        reset_streams([stream])."""
+        f = np.ascontiguousarray(nco_hz, dtype=np.float64).reshape(-1)
+        if f.size != self.C:
+            raise NvxError(f"retune_stream needs {self.C} offsets, got {f.size}")
+        tags = None
+        if freq_tag is not None:
+            t = np.ascontiguousarray(freq_tag, dtype=np.int32).reshape(-1)
+            if t.size != self.C:
+                raise NvxError(f"retune_stream needs {self.C} tags, got {t.size}")
+            tags = t.ctypes.data_as(C.POINTER(C.c_int))
+        _check(self.L.nvx_engine_retune_stream(self._h, stream, f.ctypes.data_as(C.POINTER(C.c_double)), tags))
 
     def push_host(self, iq: np.ndarray):
         """iq: [S, n, 2] (or [S, 2n]) float32, int16 or uint8 (8-bit offset binary, value u - 128), C-contiguous."""
@@ -393,6 +418,14 @@ class Capture:
 
     def dropped(self, stream: int) -> int:
         return int(self.L.nvx_capture_dropped(self._h, stream))
+
+    def detach(self, stream: int):
+        """The stream's radio stopped delivering: pump without it (its rows are silence) and refuse its writes."""
+        _check(self.L.nvx_capture_detach(self._h, stream))
+
+    def attach(self, stream: int):
+        """The radio is back: flush its ring and restart its decoder (Engine.reset_streams) before the next pump."""
+        _check(self.L.nvx_capture_attach(self._h, stream))
 
     def close(self):
         if self._h and self._h.value:
