@@ -1,11 +1,10 @@
 // engine.cu -- the C ABI of include/navtex_b200.h: per-GPU engine that owns the carried state of
-// S independent streams and queues, per pushed block, the fused FIR cascade (or the three long-tap
-// stage kernels), the tail carry, the demod / bit-sync / state-machine kernels and the event
+// S independent streams and queues, per pushed block, the FIR path (the fused cascade and its tail carry, or the
+// three long-tap stage kernels), the demod / bit-sync / state-machine kernels and the event
 // download; host side it runs the message assembler on a worker thread.
 //
 // Call contract it replaces: capt_sched.c:552-555 (init_dsp), :612 (init_fir2_wrapper) and the
 // consumer loop :484-528 that calls sample_in_1 once per IQ pair.
-#include <cuda.h>
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdarg.h>
@@ -43,55 +42,6 @@ int fail(int code, const char* fmt, ...) {
             return fail(NVX_ERR_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e__), __FILE__, __LINE__); \
     } while (0)
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn g_encode = nullptr;
-
-int load_encode() {
-    if (g_encode) return 0;
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres);
-    if (e != cudaSuccess || qres != cudaDriverEntryPointSuccess || !fn)
-        return fail(NVX_ERR_CUDA, "cuTensorMapEncodeTiled not available: %s", cudaGetErrorString(e));
-    g_encode = (EncodeTiledFn)fn;
-    return 0;
-}
-
-// 32-bit-element view of a stream-major sample array: [rows][2 * cols] floats for float2 samples, [rows][cols] words for
-// short2 samples (one word = one I,Q pair), [rows][cols / 2] words for 8-bit pairs (one word = two pairs; cols is a multiple
-// of 280); box = one ring stage x 32 rows
-int encode_rows(CUtensorMap* map, const void* base, long long cols, long long rows, nvx::SampleFmt f) {
-    if (int rc = load_encode()) return rc;
-    const long long row_bytes = cols * nvx::sample_bytes(f);
-    cuuint64_t dims[2] = {(cuuint64_t)(row_bytes / 4), (cuuint64_t)rows};
-    cuuint64_t strides[1] = {(cuuint64_t)row_bytes};
-    cuuint32_t box[2] = {(cuuint32_t)nvx::cascade_box_elems(f), 32};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = g_encode(map, f == nvx::SampleFmt::F32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_INT32, 2, const_cast<void*>(base), dims, strides, box, estr,
-                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(NVX_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) cols=%lld rows=%lld", (int)r, cols, rows);
-    return 0;
-}
-
-// new_tail[s] = last `halo` samples of (old_tail[s] ++ x[s][0..n)); kPer samples (16 bytes) per thread
-template <typename Sample>
-__global__ void tail_carry_kernel(const Sample* __restrict__ old_tail, const Sample* __restrict__ x, Sample* __restrict__ new_tail,
-                                  int streams, long long n, int halo) {
-    constexpr int kPer = 16 / (int)sizeof(Sample);
-    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const long long per = halo / kPer;
-    if (idx >= per * streams) return;
-    const int s = (int)(idx / per);
-    const long long k = (idx % per) * kPer;
-    const long long p = n - halo + k;                                            // n and halo are multiples of 280
-    const int4* src = p >= 0 ? reinterpret_cast<const int4*>(x + (size_t)s * n + p)
-                             : reinterpret_cast<const int4*>(old_tail + (size_t)s * halo + (halo + p));
-    *reinterpret_cast<int4*>(new_tail + (size_t)s * halo + k) = *src;
-}
-
 // nvx_config.nco_hz entry f -> its NCO row; false if f is off the 0.5 Hz grid or outside +-31.5 kHz
 bool nco_entry(double f, nvx::NcoChan* out) {
     const double twice = 2.0 * f;
@@ -112,10 +62,7 @@ struct ResetArgs {
     const int* streams;                 // [gridDim.x] local stream indices
     int C;                              // channels per stream
     long long e0;                       // the new epoch, 900 Hz samples (a multiple of 567)
-    uint32_t* tail;                     // fused path: the [S][tail_words] input tail the next block reads, else null
-    long long tail_words;
-    uint32_t tail_fill;                 // silence in the pushed format (0x80 bytes for 8-bit pairs)
-    nvx::LongHist lh;                   // long-tap path: the stage histories the next block reads (rows null without it)
+    nvx::CarriedRows rows;              // what the engine's FIR path carries into the next block
     float2* y3_prev;                    // the previous block's y3 / corr buffers, whose ends become this block's histories
     long long y3_pitch;
     double* corr_prev;
@@ -131,13 +78,8 @@ struct ResetArgs {
 __global__ void reset_streams_kernel(const ResetArgs a) {
     const int s = a.streams[blockIdx.x];
     const int t = threadIdx.x, nt = blockDim.x;
-    if (a.tail)
-        for (long long i = t; i < a.tail_words; i += nt) a.tail[(size_t)s * a.tail_words + i] = a.tail_fill;
     for (int k = 0; k < 3; ++k)
-        if (a.lh.rows[k]) {
-            const long long len = (long long)a.lh.per_stream[k] * a.lh.H[k];
-            for (long long i = t; i < len; i += nt) a.lh.rows[k][(size_t)s * len + i] = make_float2(0.f, 0.f);
-        }
+        for (long long i = t; i < a.rows.words[k]; i += nt) a.rows.base[k][(size_t)s * a.rows.words[k] + i] = a.rows.fill[k];
     for (int c = 0; c < a.C; ++c) {
         const size_t ch = (size_t)s * a.C + c;
         for (int i = t; i < nvx::kHistY; i += nt) a.y3_prev[ch * a.y3_pitch + a.n_prev + i] = make_float2(0.f, 0.f);
@@ -164,20 +106,13 @@ struct nvx_engine {
     nvx_config cfg;
     int S = 0, P_max = 0, channels = 0;
     int C = 2;                            // channels per stream (nvx_config.n_channels)
-    cudaStream_t stream = nullptr;        // cascade, tail carry, ingest copies / conversion
+    cudaStream_t stream = nullptr;        // FIR path, ingest copies / conversion
     cudaStream_t stream_demod = nullptr;  // demod kernels + event download, one block behind
     float2* y3buf[kBuf] = {};
     uint8_t* pickbuf[kBuf] = {};
     cudaEvent_t demod_done[kBuf] = {}, ff_done[kBuf] = {};
     long long blocks = 0;
     int last_buf = 0;
-    int tap_class = 0;                    // fused-kernel tap-length class (fir_cascade.cuh), -1 = long-tap path
-    int halo = 1960;                      // carried input samples per stream: 280 x the class's warm-up superblocks
-    // fused path: carried input tail, ping-pong, in the sample format being pushed: [S][halo] float2, short2 or 8-bit pairs
-    // (each buffer sized for float2); filled with silence and described to the TMA unit when the first push fixes the format
-    void* tail[2] = {};
-    CUtensorMap map_tail[2];
-    int tail_cur = 0;
     int fmt = -1;                         // -1 = nothing pushed since create/reset, else the nvx::SampleFmt of the pushes
     nvx::DemodBuffers db = {};
     double* corrbuf[2] = {nullptr, nullptr};   // |mask correlation| rows, alternating per block (each block reads its history from the other)
@@ -193,11 +128,12 @@ struct nvx_engine {
     long long host_pushes = 0;
     long long sb_abs = 0;
     int last_P = 0;
-    bool custom_taps = false;
-    nvx::CascadeTaps taps;                // this engine's filter constants: passed in the parameter block of every cascade launch
     nvx::NcoChan* d_nco_ch = nullptr;     // [S][C] per-stream NCO parameters (nvx_config.nco_hz), else null: the reference table
     std::vector<nvx::NcoChan> nco_host;   // the same rows with phase origin 0 (retunes edit them here first)
-    nvx::LongPath* lp = nullptr;          // tap sets too long for the fused kernel: the three stage kernels (fir_long.cuh), else null
+    // the FIR path, one of the two: the fused cascade (fir_cascade.cuh), or the three stage kernels of tap sets too long for it
+    // (fir_long.cuh)
+    nvx::CascadePath* cp = nullptr;
+    nvx::LongPath* lp = nullptr;
     std::vector<int> stream_tag;          // optional [S][C] message tags (read by the worker; changed through markers)
     // per-stream resets and retunes asked for since the last push; the next push applies them
     struct TagChange { int stream; std::vector<int> tags; };
@@ -211,7 +147,6 @@ struct nvx_engine {
     // what the worker does before it assembles block `block`: drop the reset streams' partial lines and messages, switch tags
     struct Marker { long long block; std::vector<int> streams; std::vector<TagChange> tags; };
     std::deque<Marker> markers;           // guarded by mu, in push order
-    int target_warps[nvx::kSampleFmts] = {576, 576, 576};   // resident cascade warps per sample format
     nvx::MessageAssembler assembler;
     std::vector<nvx::AssembledMessage> ready, handed;
     std::vector<nvx_message> view;
@@ -250,7 +185,6 @@ int free_engine(nvx_engine* e) {
         e->worker.join();
     }
     for (cudaEvent_t ev : e->ev_pool) cudaEventDestroy(ev);
-    cudaFree(e->tail[0]); cudaFree(e->tail[1]);
     cudaFree(e->corrbuf[0]); cudaFree(e->corrbuf[1]); cudaFree(e->db.clock); cudaFree(e->db.fsm);
     cudaFree(e->db.bitpos); cudaFree(e->db.bitval); cudaFree(e->db.nbits);
     cudaFree(e->d_bits); cudaFree(e->d_disc); cudaFree(e->d_bit_count);
@@ -264,6 +198,7 @@ int free_engine(nvx_engine* e) {
     cudaFree(e->d_nco_ch);
     cudaFree(e->db.epoch); cudaFree(e->d_reset_list); cudaFreeHost(e->h_reset);
     if (e->reset_copied) cudaEventDestroy(e->reset_copied);
+    nvx::cascade_path_free(e->cp);
     nvx::long_path_free(e->lp);
     for (int k = 0; k < kBuf; ++k) {
         cudaFree(e->y3buf[k]); cudaFree(e->d_events[k]); cudaFree(e->d_ev_count[k]);
@@ -285,7 +220,7 @@ void set_tags(nvx_engine* e, const nvx_engine::TagChange& t) {
 }
 
 int reset_state(nvx_engine* e) {
-    e->fmt = -1;                                    // the next push fixes the format and fills the fused path's tail
+    e->fmt = -1;                                    // the next push fixes the format
     // per-stream resets still pending are part of this one; their new tags take effect now, their offsets are in nco_host
     for (const auto& t : e->pend_tags) set_tags(e, t);
     for (int s : e->pend_streams) e->pend_flags[(size_t)s] = 0;
@@ -294,6 +229,7 @@ int reset_state(nvx_engine* e) {
     if (e->d_nco_ch)   // every row's phase origin back to 0
         CU_TRY(cudaMemcpyAsync(e->d_nco_ch, e->nco_host.data(), e->nco_host.size() * sizeof(nvx::NcoChan), cudaMemcpyHostToDevice, e->stream));
     if (e->lp) CU_TRY(nvx::long_path_reset(e->lp, e->stream));
+    else nvx::cascade_path_reset(e->cp);
     for (int k = 0; k < kBuf; ++k) {
         e->db.y3 = e->y3buf[k];
         e->db.picks = e->pickbuf[k];
@@ -301,7 +237,6 @@ int reset_state(nvx_engine* e) {
         CU_TRY(nvx::demod_init_state(e->db, e->channels, e->stream));
     }
     CU_TRY(cudaStreamSynchronize(e->stream));
-    e->tail_cur = 0;
     e->sb_abs = 0;
     e->last_P = 0;
     e->blocks = 0;
@@ -455,8 +390,8 @@ int sync_engine(nvx_engine* e) {
     return 0;
 }
 
-// what the long-tap path reports goes into this engine's nvx_stats and nvx_last_error()
-int long_report(nvx_engine* e, int rc, const nvx::LongReport& rep) {
+// what the FIR path reports goes into this engine's nvx_stats and nvx_last_error()
+int path_report(nvx_engine* e, int rc, const nvx::PathReport& rep) {
     e->stats.aux_launches += rep.launches;
     e->stats.long_tc_fallbacks += rep.fallbacks;
     if (rep.msg[0]) fail(rc, "%s", rep.msg);
@@ -465,7 +400,7 @@ int long_report(nvx_engine* e, int rc, const nvx::LongReport& rep) {
 
 // the resets asked for since the last push, queued in front of this block (b = its buffer index): NCO rows of retuned streams,
 // the reset kernel, and the marker that tells the worker from which block on the streams' messages start over
-int apply_resets(nvx_engine* e, nvx::SampleFmt fmt, int b) {
+int apply_resets(nvx_engine* e, int b) {
     using namespace nvx;
     const int count = (int)e->pend_streams.size();
     if (!count) return 0;
@@ -497,13 +432,7 @@ int apply_resets(nvx_engine* e, nvx::SampleFmt fmt, int b) {
     ra.streams = e->d_reset_list;
     ra.C = e->C;
     ra.e0 = e->sb_abs - e->sb_abs % kCorrLen;
-    if (!e->lp) {
-        ra.tail = static_cast<uint32_t*>(e->tail[e->tail_cur]);
-        ra.tail_words = (long long)e->halo * sample_bytes(fmt) / 4;
-        ra.tail_fill = fmt == SampleFmt::U8 ? 0x80808080u : 0u;
-    } else {
-        ra.lh = long_path_hist(e->lp);
-    }
+    ra.rows = e->lp ? long_path_carried(e->lp) : cascade_path_carried(e->cp);
     ra.y3_prev = e->y3buf[(b + kBuf - 1) % kBuf];
     ra.y3_pitch = kHistY + e->P_max;
     ra.corr_prev = e->corrbuf[(e->blocks & 1) ^ 1];
@@ -527,50 +456,19 @@ int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fm
     using namespace nvx;
     if (e->fmt >= 0 && e->fmt != (int)fmt)
         return fail(NVX_ERR_ARG, "sample format changed between pushes (float, int16 and 8-bit blocks cannot be mixed without a reset)");
-    if (e->fmt < 0 && !e->lp) {
-        // the warm-up before the first block sees silence: the value 0, which is the byte 128 in 8-bit offset binary
-        for (int k = 0; k < 2; ++k) {
-            CU_TRY(cudaMemsetAsync(e->tail[k], fmt == SampleFmt::U8 ? 128 : 0, (size_t)e->S * e->halo * sample_bytes(fmt), e->stream));
-            if (int rc = encode_rows(&e->map_tail[k], e->tail[k], e->halo, e->S, fmt)) return rc;
-        }
-    }
-    e->fmt = (int)fmt;
     if (n <= 0 || n % kSuper != 0) return fail(NVX_ERR_ARG, "block length %lld is not a positive multiple of %d", n, kSuper);
     if (n > e->cfg.max_block) return fail(NVX_ERR_ARG, "block length %lld exceeds max_block %lld", n, e->cfg.max_block);
     if (((uintptr_t)d_x & 15) != 0) return fail(NVX_ERR_ARG, "device block is not 16-byte aligned");
+    e->fmt = (int)fmt;                              // only a block that is accepted fixes the format
     const int b = (int)(e->blocks % kBuf);
     wait_drained(e, e->blocks - kBuf + 1);          // block (blocks - kBuf) used these buffers: long finished, normally
-    if (int rc = apply_resets(e, fmt, b)) return rc;
+    if (int rc = apply_resets(e, b)) return rc;
     if (e->timing && e->ev_used > 4000) {            // bound the event pool in long timed runs
         CU_TRY(cudaStreamSynchronize(e->stream));
         CU_TRY(cudaStreamSynchronize(e->stream_demod));
         collect_spans(e);
     }
-    CascadeArgs ca;
-    if (int rc = encode_rows(&ca.map_x, d_x, n, e->S, fmt)) return rc;
-    ca.map_tail = e->map_tail[e->tail_cur];
     const int n_super = (int)(n / kSuper);
-    const int groups = (e->S + 31) / 32;
-    // time segments: enough warps to fill the machine once, but keep the 7-superblock warm-up small
-    int segs = e->target_warps[(int)fmt] / groups;            // never more warps than are resident at once (no second wave)
-    const int min_seg = 63;
-    if (segs > n_super / min_seg) segs = n_super / min_seg;
-    if (segs < 1) segs = 1;
-    const int seg_super = (n_super + segs - 1) / segs;
-    segs = (n_super + seg_super - 1) / seg_super;
-    ca.y3 = e->y3buf[b];
-    ca.n = n;
-    ca.streams = e->S;
-    ca.segs = segs;
-    ca.seg_super = seg_super;
-    ca.n_super = n_super;
-    ca.sb_phase = (int)(e->sb_abs % kNcoPeriod);
-    ca.sb_abs = e->sb_abs;
-    ca.nco = e->d_nco_ch;
-    ca.y3_pitch = nvx::kHistY + e->P_max;
-    ca.y3_off = nvx::kHistY;
-    ca.ch_total = e->C;
-    ca.ch0 = 0;
 
     cudaEvent_t t0 = nullptr, t1 = nullptr, marks[8] = {};
     if (e->timing) {
@@ -585,41 +483,11 @@ int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fm
         }
         CU_TRY(cudaEventRecord(t0, e->stream));
     }
-    if (e->lp) {
-        LongReport rep;
-        const int rc = long_path_run(e->lp, d_x, n, fmt, e->sb_abs * (kSuper / NVX_D1), e->y3buf[b], ca.y3_pitch, ca.y3_off, e->stream, &rep);
-        if (long_report(e, rc, rep)) return rc;
-    } else {
-        // up to four channels share one pass over the input (stage 1 computed once for all of them); five to eight take two
-        for (int c0 = 0; c0 < e->C;) {
-            const int left = e->C - c0;
-            const int n_ch = left <= nvx::kMaxFusedCh ? left : (left + 1) / 2;      // 5 = 3 + 2, 6 = 3 + 3, 7 = 4 + 3, 8 = 4 + 4
-            ca.ch0 = c0;
-            CU_TRY(cascade_launch(ca, e->taps, e->tap_class, e->custom_taps, fmt, n_ch, e->stream));
-            if (c0) e->stats.aux_launches++;
-            c0 += n_ch;
-        }
-    }
-    if (e->timing) CU_TRY(cudaEventRecord(t1, e->stream));
-
-    if (!e->lp) {
-        const int nxt = e->tail_cur ^ 1;
-        const long long work = (long long)e->S * (e->halo / (16 / sample_bytes(fmt)));
-        const unsigned grid = (unsigned)((work + 255) / 256);
-        const void* old_tail = e->tail[e->tail_cur];
-        void* new_tail = e->tail[nxt];
-        if (fmt == SampleFmt::U8)
-            tail_carry_kernel<uchar2><<<grid, 256, 0, e->stream>>>(static_cast<const uchar2*>(old_tail), static_cast<const uchar2*>(d_x),
-                                                                   static_cast<uchar2*>(new_tail), e->S, n, e->halo);
-        else if (fmt == SampleFmt::S16)
-            tail_carry_kernel<short2><<<grid, 256, 0, e->stream>>>(static_cast<const short2*>(old_tail), static_cast<const short2*>(d_x),
-                                                                   static_cast<short2*>(new_tail), e->S, n, e->halo);
-        else
-            tail_carry_kernel<float2><<<grid, 256, 0, e->stream>>>(static_cast<const float2*>(old_tail), static_cast<const float2*>(d_x),
-                                                                   static_cast<float2*>(new_tail), e->S, n, e->halo);
-        CU_TRY(cudaGetLastError());
-        e->tail_cur = nxt;
-    }
+    PathReport rep;
+    const long long y3_pitch = kHistY + e->P_max;
+    const int rc = e->lp ? long_path_run(e->lp, d_x, n, fmt, e->sb_abs, e->y3buf[b], y3_pitch, kHistY, e->stream, t1, &rep)
+                         : cascade_path_run(e->cp, d_x, n, fmt, e->sb_abs, e->y3buf[b], y3_pitch, kHistY, e->stream, t1, &rep);
+    if (path_report(e, rc, rep)) return rc;
 
     // demod of this block runs on its own stream, overlapping the next block's cascade
     DemodArgs da;
@@ -657,7 +525,6 @@ int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fm
     e->last_P = n_super;
     e->stats.cascade_launches++;
     e->stats.demod_launches += nvx::demod_launches_per_block();
-    e->stats.aux_launches++;
     e->stats.samples += n * e->S;
     return 0;
 }
@@ -736,7 +603,6 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
     e->channels = C * e->S;
     e->pend_flags.assign((size_t)e->S, 0);
     e->P_max = (int)(cfg->max_block / nvx::kSuper);
-    e->custom_taps = cfg->h1 || cfg->h2 || cfg->h3;
     // tap counts: reference lengths unless given; sets up to 37/47/71 and up to 61/75/111 run through the fused kernel
     // (zero-padded to the class), longer ones through the long-tap path
     const int n[3] = {cfg->n1 ? cfg->n1 : NVX_T1, cfg->n2 ? cfg->n2 : NVX_T2, cfg->n3 ? cfg->n3 : NVX_T3};
@@ -746,12 +612,13 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
     }
     for (int k = 0; k < 3; ++k)
         if (n[k] < 1 || n[k] > nvx::kLongMaxTaps) { delete e; return fail(NVX_ERR_ARG, "tap count %d outside 1..%d", n[k], nvx::kLongMaxTaps); }
-    e->tap_class = nvx::cascade_tap_class(n[0], n[1], n[2]);
-    if (C != 2 && e->tap_class != 0) {
+    // the FIR path: the fused cascade for sets it takes, else the long-tap path; only the fused reference class serves other than
+    // the reference's two channels
+    const int tap_class = nvx::cascade_tap_class(n[0], n[1], n[2]);
+    if (C != 2 && tap_class != 0) {
         delete e;
         return fail(NVX_ERR_ARG, "n_channels = %d is served by the fused kernel's reference tap class only (up to %d / %d / %d taps)", C, NVX_T1, NVX_T2, NVX_T3);
     }
-    e->halo = nvx::kSuper * nvx::cascade_warm_super(e->tap_class);
     // per block and channel: at most one character plus one abort per 14 bits ... generous bound
     e->ev_cap = 2 * (e->P_max / 63 + 2) + 8;
     e->bit_cap = cfg->keep_bits ? e->P_max / 8 + 2 : 0;      // the symbol clock may run one sample per bit fast while it slews
@@ -779,8 +646,6 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
         CREATE_TRY(cudaEventCreateWithFlags(&e->demod_done[k], cudaEventDisableTiming));
         CREATE_TRY(cudaEventCreateWithFlags(&e->ff_done[k], cudaEventDisableTiming));
     }
-    if (e->tap_class >= 0)
-        for (int k = 0; k < 2; ++k) CREATE_TRY(cudaMalloc(&e->tail[k], (size_t)e->S * e->halo * nvx::sample_bytes(nvx::SampleFmt::F32)));
     e->db.p_max = e->P_max;
     for (int k = 0; k < kBuf; ++k) CREATE_TRY(cudaMalloc(&e->y3buf[k], (size_t)e->channels * (nvx::kHistY + e->P_max) * sizeof(float2)));
     for (int k = 0; k < 2; ++k) CREATE_TRY(cudaMalloc(&e->corrbuf[k], (size_t)e->channels * (nvx::kHistC + e->P_max + nvx::kPadC) * sizeof(double)));
@@ -807,17 +672,15 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
         CREATE_TRY(cudaMemset(e->d_bit_count, 0, sizeof(int) * e->channels));
     }
     if (!e->nco_host.empty()) CREATE_TRY(cudaMalloc(&e->d_nco_ch, e->nco_host.size() * sizeof(nvx::NcoChan)));   // filled by reset_state
-    if (e->tap_class < 0) {
-        const double* const h[3] = {cfg->h1, cfg->h2, cfg->h3};
-        nvx::LongReport rep;
-        const int rc = nvx::long_path_create(e->S, cfg->max_block, n, h, e->d_nco_ch, e->stream, &e->lp, &rep);
-        if (long_report(e, rc, rep)) { free_engine(e); return rc; }
-    } else {
-        nvx::cascade_fill_taps(e->tap_class, cfg->h1, n[0], cfg->h2, n[1], cfg->h3, n[2], &e->taps);
-    }
 #undef CREATE_TRY
-    for (int f = 0; f < nvx::kSampleFmts; ++f)
-        e->target_warps[f] = nvx::cascade_target_warps(cfg->device, nvx::demod_reserved_sms(e->channels), (nvx::SampleFmt)f, e->tap_class, C > 2);
+    {
+        const double* const h[3] = {cfg->h1, cfg->h2, cfg->h3};
+        nvx::PathReport rep;
+        const int rc = tap_class >= 0
+                           ? nvx::cascade_path_create(e->S, C, n, h, e->d_nco_ch, cfg->device, nvx::demod_reserved_sms(e->channels), &e->cp, &rep)
+                           : nvx::long_path_create(e->S, cfg->max_block, n, h, e->d_nco_ch, e->stream, &e->lp, &rep);
+        if (path_report(e, rc, rep)) { free_engine(e); return rc; }
+    }
     e->assembler.resize(e->channels);
     if (int rc = reset_state(e)) { free_engine(e); return rc; }
     e->worker = std::thread(worker_main, e);
@@ -872,14 +735,12 @@ int nvx_engine_push_device_f32(nvx_engine* e, const void* d_iq, long long n) {
 
 int nvx_engine_push_device_s16(nvx_engine* e, const void* d_iq, long long n) {
     if (!e || !d_iq) return fail(NVX_ERR_ARG, "null argument");
-    if (((uintptr_t)d_iq & 15) != 0) return fail(NVX_ERR_ARG, "device block is not 16-byte aligned");
     CU_TRY(cudaSetDevice(e->cfg.device));
     return process_block(e, d_iq, n, nvx::SampleFmt::S16);
 }
 
 int nvx_engine_push_device_u8(nvx_engine* e, const void* d_iq, long long n) {
     if (!e || !d_iq) return fail(NVX_ERR_ARG, "null argument");
-    if (((uintptr_t)d_iq & 15) != 0) return fail(NVX_ERR_ARG, "device block is not 16-byte aligned");
     CU_TRY(cudaSetDevice(e->cfg.device));
     return process_block(e, d_iq, n, nvx::SampleFmt::U8);
 }

@@ -208,20 +208,45 @@ struct CascadeParams {
     NcoTable nco;
 };
 static_assert(sizeof(CascadeParams<kTapClasses - 1>) <= 4096, "kernel parameter block");
-// host-side copy of an engine's filter constants (both classes' layouts; only the engine's own class is filled)
-struct CascadeTaps {
-    TapSet<0> t0;
-    TapSet<1> t1;
-    NcoTable nco;
-};
 
-// host side (fir_cascade.cu)
-int cascade_box_elems(SampleFmt f);
-int cascade_tap_class(int n1, int n2, int n3);
-int cascade_warm_super(int tap_class);
-void cascade_fill_taps(int tap_class, const double* h1, int n1, const double* h2, int n2, const double* h3, int n3, CascadeTaps* out);
-cudaError_t cascade_launch(const CascadeArgs& a, const CascadeTaps& taps, int tap_class, bool custom_taps, SampleFmt f, int n_ch, cudaStream_t stream);
-int cascade_target_warps(int device, int reserved_sms, SampleFmt f, int tap_class, bool heavy);
+// ---- host side (fir_cascade.cu) ----
+// what a call of either FIR path (the fused one below, the long-tap one of fir_long.cuh) reports to the engine
+struct PathReport {
+    long long launches = 0;   // nvx_stats.aux_launches: every launch of the call but the fused path's first channel pass
+    long long fallbacks = 0;  // stage launches meant for the tensor-core kernel that ran on the CUDA-core one (nvx_stats.long_tc_fallbacks)
+    char msg[256] = "";       // for nvx_last_error(): why the call failed, else a "note: ..." about a tensor-core fallback, else empty
+};
+int say(PathReport* rep, int code, const char* fmt, ...);     // rep->msg = the formatted message; returns code
+// what a path carries into the next block: region k of stream s is base[k][s words[k] .. + words[k]); setting a stream's regions
+// to fill[k] restarts its filters after silence (nvx_engine_reset_streams)
+struct CarriedRows { uint32_t* base[3]; long long words[3]; uint32_t fill[3]; };
+
+// the driver's tiled tensor-map encoder (looked up once), or null when the driver has none
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+EncodeTiledFn tensor_map_encoder();
+// entry k of the reference's NCO table: (cos, -sin)(2 pi k 14000 / 63000), fir2cpp.C:105-106, rounded once to float
+float2 reference_nco(int k);
+extern const double* const kRefTaps[3];      // the reference tap sets of stages 1, 2 and 3 (NVX_H*_VALUES)
+
+int cascade_tap_class(int n1, int n2, int n3);   // tap class a set of lengths needs, or -1 if it takes the long-tap path
+
+// ---- the fused path of one engine (S streams, C channels each): it owns the tap set, the carried input tail with its tensor
+// maps, and the launch policy (time segments, channel passes) ----
+struct CascadePath;
+// n[k] taps of stage k + 1, h[k] = null for the reference taps; nco = the engine's [S][C] per-stream offsets, or null for the
+// reference table (not owned: retunes and resets write it); reserved_sms SMs are left to the sequential demod kernels.  Returns 0
+// or an NVX_ERR_* code.
+int cascade_path_create(int S, int C, const int n[3], const double* const h[3], const NcoChan* nco, int device, int reserved_sms,
+                        CascadePath** out, PathReport* rep);
+void cascade_path_reset(CascadePath* cp);        // the next block starts after silence, in whatever format it comes
+CarriedRows cascade_path_carried(const CascadePath* cp);
+// one block x[S][n] in format fmt that starts at 900 Hz sample sb_abs; the 900 Hz output goes to y3[C S][y3_pitch] from y3_off
+// on.  after_fir (if not null) is recorded once the FIR work is queued, before the tail carry.  Returns 0 or an NVX_ERR_* code.
+int cascade_path_run(CascadePath* cp, const void* x, long long n, SampleFmt fmt, long long sb_abs, float2* y3, long long y3_pitch,
+                     long long y3_off, cudaStream_t stream, cudaEvent_t after_fir, PathReport* rep);
+void cascade_path_free(CascadePath* cp);
 
 #ifdef NVX_CASCADE_DEVICE_CODE
 

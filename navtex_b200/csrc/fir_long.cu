@@ -2,9 +2,6 @@
 // runs them (see fir_long.cuh).
 #include "fir_long.cuh"
 
-#include <math.h>
-#include <stdarg.h>
-#include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
 
@@ -234,14 +231,6 @@ __global__ void widen_u8_kernel(const uchar2* __restrict__ in, short2* __restric
     dst[1] = make_int4(o[4], o[5], o[6], o[7]);
 }
 
-int say(LongReport* rep, int code, const char* fmt, ...) {
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(rep->msg, sizeof rep->msg, fmt, ap);
-    va_end(ap);
-    return code;
-}
-
 LongStage long_stage(int D, int T) {
     LongStage s;
     s.D = D;
@@ -261,8 +250,7 @@ bool long_fill_taps(const LongStage& st, const double* h, LongStageTaps* out) {
             const int i = st.D * j + st.D - 1 - p;
             out->h[p * st.J + j] = i < st.T ? (float)h[i] : 0.f;
         }
-    for (int k = 0; k < kNcoPeriod; ++k)       // same expression as fir2cpp.C:105-106, rounded once to float
-        out->nco[k] = make_float2((float)cos((2 * M_PI * k * 14000) / 63000), (float)-sin((2 * M_PI * k * 14000) / 63000));
+    for (int k = 0; k < kNcoPeriod; ++k) out->nco[k] = reference_nco(k);
     return true;
 }
 
@@ -311,7 +299,7 @@ size_t hist_bytes(const LongPath* lp, int k) { return (size_t)(k == 0 ? lp->S : 
 
 // stage k + 1: on the tensor cores where they serve it, else on the CUDA-core kernel (counted and explained when the tensor cores
 // were asked for); then its history carry, the last H inputs of each of `rows` rows (S stream rows of y1 when stage 2 mixes on load)
-int run_stage(LongPath* lp, int k, const LongArgs& a, long long in_pitch, int rows, cudaStream_t stream, LongReport* rep) {
+int run_stage(LongPath* lp, int k, const LongArgs& a, long long in_pitch, int rows, cudaStream_t stream, PathReport* rep) {
     cudaError_t e = lp->tc[k] ? long_tc_launch(lp->tc[k], a, lp->st[k], in_pitch, stream) : cudaErrorNotSupported;
     if (e == cudaErrorNotSupported && a.mix_in)      // (cannot happen: y1 and its pitch are 16-byte aligned)
         return say(rep, NVX_ERR_CUDA, "long-tap stage 2: the tensor-core kernel refused the block and the stage-1 output is un-mixed");
@@ -330,9 +318,8 @@ int run_stage(LongPath* lp, int k, const LongArgs& a, long long in_pitch, int ro
 }  // namespace
 
 int long_path_create(int S, long long max_block, const int n[3], const double* const h[3], const NcoChan* nco, cudaStream_t stream,
-                     LongPath** out, LongReport* rep) {
-    static const double ref1[NVX_T1] = {NVX_H1_VALUES}, ref2[NVX_T2] = {NVX_H2_VALUES}, ref3[NVX_T3] = {NVX_H3_VALUES};
-    const double* hh[3] = {h[0] ? h[0] : ref1, h[1] ? h[1] : ref2, h[2] ? h[2] : ref3};
+                     LongPath** out, PathReport* rep) {
+    const double* hh[3] = {h[0] ? h[0] : kRefTaps[0], h[1] ? h[1] : kRefTaps[1], h[2] ? h[2] : kRefTaps[2]};
     const int D[3] = {NVX_D1, NVX_D2, NVX_D3};
     LongPath* lp = new LongPath();
     lp->S = S; lp->max_block = max_block; lp->nco = nco;
@@ -378,19 +365,18 @@ cudaError_t long_path_reset(LongPath* lp, cudaStream_t stream) {
     return e;
 }
 
-LongHist long_path_hist(const LongPath* lp) {
-    LongHist h;
-    for (int k = 0; k < 3; ++k) {
-        h.rows[k] = lp->hist[k][lp->cur];
-        h.H[k] = lp->st[k].H;
-        h.per_stream[k] = k == 0 || (k == 1 && lp->mix_on_load) ? 1 : 2;
+CarriedRows long_path_carried(const LongPath* lp) {
+    CarriedRows r = {};
+    for (int k = 0; k < 3; ++k) {      // per stream: 1 or 2 rows of H float2 (two words each), zeroed
+        r.base[k] = reinterpret_cast<uint32_t*>(lp->hist[k][lp->cur]);
+        r.words[k] = 2LL * (k == 0 || (k == 1 && lp->mix_on_load) ? 1 : 2) * lp->st[k].H;
     }
-    return h;
+    return r;
 }
 
-// 3 stage launches and 3 history carries: 5 in nvx_stats.aux_launches, where the engine counts one per block for every path
-int long_path_run(LongPath* lp, const void* x, long long n, SampleFmt fmt, long long tick, float2* y3, long long y3_pitch,
-                  long long y3_off, cudaStream_t stream, LongReport* rep) {
+// 3 stage launches, 3 history carries and, for 8-bit input, the widening kernel: all in rep->launches
+int long_path_run(LongPath* lp, const void* x, long long n, SampleFmt fmt, long long sb_abs, float2* y3, long long y3_pitch,
+                  long long y3_off, cudaStream_t stream, cudaEvent_t after_fir, PathReport* rep) {
     const int S = lp->S;
     // 8-bit input: widened to the int16 values u - 128 in front of the unchanged int16 path (same results bit for bit)
     if (fmt == SampleFmt::U8) {
@@ -402,6 +388,7 @@ int long_path_run(LongPath* lp, const void* x, long long n, SampleFmt fmt, long 
         rep->launches++;
         x = lp->u8_wide;
     }
+    const long long tick = sb_abs * (kSuper / NVX_D1);                                       // the block's first 63 kHz output
     const long long p1 = lp->max_block / NVX_D1, p2 = lp->max_block / (NVX_D1 * NVX_D2);     // row pitches of y1 and y2
     LongArgs a1 = {};         // 252 k -> 63 k: mixed, one row per channel, or un-mixed, one row per stream (mix on load)
     a1.in = x; a1.hist = lp->hist[0][lp->cur]; a1.out = lp->y1; a1.n_in = n; a1.out_pitch = p1;
@@ -416,8 +403,9 @@ int long_path_run(LongPath* lp, const void* x, long long n, SampleFmt fmt, long 
     a3.rows_in = 2 * S; a3.stage = 2;
     if (int rc = run_stage(lp, 2, a3, p2, 2 * S, stream, rep)) return rc;
     lp->cur ^= 1;
-    rep->launches += 5;
-    return 0;
+    rep->launches += 6;
+    const cudaError_t e = after_fir ? cudaEventRecord(after_fir, stream) : cudaSuccess;
+    return e == cudaSuccess ? 0 : say(rep, NVX_ERR_CUDA, "cudaEventRecord failed: %s", cudaGetErrorString(e));
 }
 
 void long_path_free(LongPath* lp) {

@@ -76,29 +76,20 @@ cudaError_t long_tc_launch(const LongTcStage* s, const LongArgs& a, const LongSt
 
 // ---- the long-tap path of one engine (S streams, two channels each) ----
 // It owns the stage taps, the per-stage histories, the y1 / y2 intermediates, the tensor-core stages and the choice of mix on
-// load.  The engine owns nvx_last_error() and nvx_stats: create and run report to it through a LongReport.
+// load.  Same calls as the fused path (fir_cascade.cuh); create and run report to the engine through a PathReport.
 struct LongPath;
-struct LongReport {
-    long long launches = 0;   // kernels launched (nvx_stats.aux_launches)
-    long long fallbacks = 0;  // stage launches meant for the tensor-core kernel that ran on the CUDA-core one (nvx_stats.long_tc_fallbacks)
-    char msg[256] = "";       // for nvx_last_error(): why the call failed, else a "note: ..." about a tensor-core fallback, else empty
-};
 // n[k] taps of stage k + 1, h[k] = null for the reference taps; nco = the engine's [S][2] per-stream offsets, or null for the
 // reference table.  Reads NVX_LONG_TC and NVX_LONG_MIX.  Returns 0 or an NVX_ERR_* code.
 int long_path_create(int S, long long max_block, const int n[3], const double* const h[3], const NcoChan* nco, cudaStream_t stream,
-                     LongPath** out, LongReport* rep);
+                     LongPath** out, PathReport* rep);
 cudaError_t long_path_reset(LongPath* lp, cudaStream_t stream);     // zero histories: the next block starts after silence
 // the histories the next block reads: stage k keeps per_stream[k] consecutive rows of H[k] float2 for each stream (1 for stage 1,
 // 2 for stages 2 and 3 -- one per channel -- or 1 for stage 2 when it mixes on load); zeroing a stream's rows restarts its filters
-struct LongHist {
-    float2* rows[3];
-    int H[3], per_stream[3];
-};
-LongHist long_path_hist(const LongPath* lp);
-// one block x[S][n] in format fmt whose first 63 kHz output sits at tick; the 900 Hz output goes to y3[2 S][y3_pitch] from
-// y3_off on.  Returns 0 or an NVX_ERR_* code.
-int long_path_run(LongPath* lp, const void* x, long long n, SampleFmt fmt, long long tick, float2* y3, long long y3_pitch,
-                  long long y3_off, cudaStream_t stream, LongReport* rep);
+CarriedRows long_path_carried(const LongPath* lp);
+// one block x[S][n] in format fmt that starts at 900 Hz sample sb_abs; the 900 Hz output goes to y3[2 S][y3_pitch] from y3_off on.
+// after_fir (if not null) is recorded after the last launch.  Returns 0 or an NVX_ERR_* code.
+int long_path_run(LongPath* lp, const void* x, long long n, SampleFmt fmt, long long sb_abs, float2* y3, long long y3_pitch,
+                  long long y3_off, cudaStream_t stream, cudaEvent_t after_fir, PathReport* rep);
 void long_path_free(LongPath* lp);
 
 }  // namespace nvx

@@ -1018,10 +1018,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) fir_tcs_kernel(const __grid_con
     if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem));
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
 float tf32_rna(float x) {                  // round to nearest, ties away, 10-bit mantissa (cvt.rna.tf32.f32)
     uint32_t u;
     memcpy(&u, &x, 4);
@@ -1101,7 +1097,6 @@ struct LongTcStage {
     bool streaming = false;
     float *d_gh = nullptr, *d_gl = nullptr;
     CUtensorMap map_gh, map_gl;
-    EncodeTiledFn enc = nullptr;
 };
 
 // host side of the band matrix (no GPU needed; also behind nvx_debug_long_tc_band for the CPU tests): padded tap count, tile
@@ -1147,9 +1142,8 @@ bool long_tc_band(int D, int T_taps, const double* h, TcBand* b) {
 LongTcStage* long_tc_prepare(int D, int T_taps, const double* h, cudaStream_t stream) {
     TcBand band;
     if (!long_tc_band(D, T_taps, h, &band)) return nullptr;
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) != cudaSuccess || !fn) return nullptr;
+    const EncodeTiledFn enc = tensor_map_encoder();
+    if (!enc) return nullptr;
     LongTcStage* s = new LongTcStage();
     s->D = D; s->T = band.T; s->N = band.N;
     s->streaming = band.streaming;
@@ -1163,7 +1157,6 @@ LongTcStage* long_tc_prepare(int D, int T_taps, const double* h, cudaStream_t st
     ok = ok && cudaMemcpyAsync(s->d_gl, gl.data(), gl.size() * 4, cudaMemcpyHostToDevice, stream) == cudaSuccess;
     ok = ok && cudaStreamSynchronize(stream) == cudaSuccess;
     if (ok) {
-        EncodeTiledFn enc = s->enc = (EncodeTiledFn)fn;
         cuuint64_t dims[2] = {(cuuint64_t)kKB, (cuuint64_t)P * s->J};
         cuuint64_t strides[1] = {(cuuint64_t)kKB * 4};
         cuuint32_t box[2] = {kKB, (cuuint32_t)s->box_rows};
@@ -1200,10 +1193,7 @@ cudaError_t long_tc_launch(const LongTcStage* s, const LongArgs& la, const LongS
     a.nco = la.nco; a.rows = la.rows_in; a.s16 = la.s16; a.T = s->T; a.H = st.H; a.chunks = s->chunks; a.J = s->J; a.slots = 4; a.box_rows = s->box_rows;
     a.mix = la.stage == 0 && !la.plain;
     a.rows_src = la.mix_in ? la.rows_in / 2 : la.rows_in;
-    for (int k = 0; k < kNcoPeriod + 16; ++k) {      // same expression as fir2cpp.C:105-106, rounded once to float
-        const int k9 = k % kNcoPeriod;
-        a.nco_tab[k] = make_float2((float)cos((2 * M_PI * k9 * 14000) / 63000), (float)-sin((2 * M_PI * k9 * 14000) / 63000));
-    }
+    for (int k = 0; k < kNcoPeriod + 16; ++k) a.nco_tab[k] = reference_nco(k % kNcoPeriod);
     // TMA boxes and 16-byte cp.async pieces: the block and its rows must start on 16-byte boundaries (tile windows do by
     // construction).  The block as a 2-D tensor of 32-bit (float2 input) or 16-bit (short2 input) elements, two per sample:
     if (((uintptr_t)la.in & 15) || ((in_pitch * (la.s16 ? 4 : 8)) & 15)) return cudaErrorNotSupported;
@@ -1215,7 +1205,7 @@ cudaError_t long_tc_launch(const LongTcStage* s, const LongArgs& la, const LongS
         cuuint64_t strides[1] = {(cuuint64_t)in_pitch * 2 * esz};
         cuuint32_t box[2] = {(cuuint32_t)(128 / esz), (cuuint32_t)(la.mix_in ? kRows / 2 : kRows)};
         cuuint32_t es[2] = {1, 1};
-        if (s->enc(&a.map_x, la.s16 ? CU_TENSOR_MAP_DATA_TYPE_UINT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(la.in), dims, strides,
+        if (tensor_map_encoder()(&a.map_x, la.s16 ? CU_TENSOR_MAP_DATA_TYPE_UINT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(la.in), dims, strides,
                    box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
             return cudaErrorNotSupported;

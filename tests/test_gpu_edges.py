@@ -105,11 +105,20 @@ def test_reset_reproduces_and_formats_do_not_mix():
 
 
 def test_argument_errors():
+    import torch
+
     eng = engine.Engine(2, 2800)
     with pytest.raises(engine.NvxError):
         eng.push_host(np.zeros((2, 281, 2), dtype=np.float32))       # not a multiple of 280
     with pytest.raises(engine.NvxError):
         eng.push_host(np.zeros((2, 5600, 2), dtype=np.float32))      # longer than max_block
+    # a rejected device push does not fix the sample format: the next valid push may come in another one
+    xf = torch.zeros((2, 2800, 2), dtype=torch.float32, device="cuda")
+    xs = torch.zeros((2, 2800, 2), dtype=torch.int16, device="cuda")
+    with pytest.raises(engine.NvxError):
+        eng.push_device(xf.data_ptr(), 2790)
+    eng.push_device(xs.data_ptr(), 2800, s16=True)
+    eng.sync()
     eng.close()
     with pytest.raises(engine.NvxError):
         engine.Engine(0, 2800)
