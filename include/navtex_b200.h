@@ -122,6 +122,41 @@ int nvx_engine_reset_streams(nvx_engine *e, const int *streams, int count);
  * the engine was created without nco_hz (reference-table engines cannot be retuned). */
 int nvx_engine_retune_stream(nvx_engine *e, int stream, const double *nco_hz, const int *freq_tag);
 
+/* ---- saved stream state: a stream survives an engine restart or moves to another engine ---------------------------------
+ * A stream saved after input sample E (the total pushed per stream) and loaded into an engine created with the same
+ * configuration continues bit for bit as the uninterrupted stream would: y3, bits, discriminator sums, events and messages.  A
+ * bulletin in flight at the save completes on the destination, its full text delivered once, labelled with the destination's
+ * stream id and the tags the state carries.  This holds on both FIR paths, the long-tap tensor-core stages included, as long as
+ * the blocks pushed after the load are those the source would have pushed.
+ *
+ * Position rule: the demod grids and the reference NCO table are absolute, so a load is accepted only where the destination's
+ * pushed total E' satisfies E' = E (mod 158760), 158760 = 567 x 280 as in nvx_engine_reset_streams.  An engine that has pushed
+ * nothing since create or reset adopts E instead (this is what a restart uses): its streams that are not loaded start as
+ * streams reset at E, and a second load before its first push must agree with the first modulo 158760.  Epochs move by E' - E
+ * and general-NCO rows keep their phase.
+ * Compatibility: the state records the FIR path (fused reference or medium tap class, or long-tap path), the tap values as
+ * the kernels read them, what the path carries per stream, n_channels, reference table or per-stream NCO offsets, and the sample
+ * format.  A load into an engine that differs in any of these, or whose pushes already fixed another sample format, returns
+ * NVX_ERR_ARG and changes nothing; so does a state whose magic number, version or checksum is wrong (a truncated or altered
+ * state is never half-applied).  The bytes are in the host's byte order.
+ *
+ * Loading a stream into one engine while another engine still runs it delivers its bulletins twice: reset or detach the source.
+ * Like every call, a load belongs to the engine's one caller thread; a capture poller (nvx_capture_start) pushing on another
+ * thread meanwhile is outside that contract: stop it first. */
+/* State of streams[0..count) (each listed once) after the last pushed block (implies nvx_engine_sync), as one self-contained
+ * byte string.  out = NULL or cap too small: *size receives the bytes needed, NVX_ERR_OVERFLOW if out was given.  Read-only:
+ * the engine and the listed streams carry on untouched.  NVX_ERR_ARG if nothing was pushed since create or reset, or if a listed
+ * stream has a reset, retune or load pending. */
+int nvx_engine_save_streams(nvx_engine *e, const int *streams, int count, void *out, size_t cap, size_t *size);
+/* Record k of the state goes to local stream streams[k] (count = the number of records in it; each stream listed once).  Takes
+ * effect at the start of the next push, like nvx_engine_reset_streams; per stream, the last reset / retune / load called before
+ * a push wins.  A load also gives the stream the saved channel offsets and tags, which a later reset or retune keeps unless it
+ * replaces them.  Messages the stream completed in blocks pushed before the load still arrive under the old state. */
+int nvx_engine_load_streams(nvx_engine *e, const int *streams, int count, const void *state, size_t size);
+/* host-only (no GPU): validate a saved state and report its record count, input position E (samples per stream), channels per
+ * stream and sample format (0 = float, 1 = int16, 2 = 8-bit); any output may be NULL */
+int nvx_stream_state_info(const void *state, size_t size, int *count, long long *position, int *n_channels, int *sample_format);
+
 /* ---- ingest: n samples for every stream.  Host variants copy H2D on a copy stream into one of two staging slots, so
  * the copy of block k+1 overlaps the kernels of block k.  A pageable buffer may be reused as soon as the call returns;
  * a pinned (cudaHostAlloc / cudaHostRegister) buffer is read asynchronously and must stay unchanged until

@@ -8,6 +8,7 @@
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdarg.h>
+#include <stddef.h>
 #include <stdio.h>
 #include <string.h>
 
@@ -55,11 +56,38 @@ bool nco_entry(double f, nvx::NcoChan* out) {
     return true;
 }
 
-// Everything the next block would carry over from the past of the listed streams, cleared so that each restarts as an engine
-// created at its epoch e0 (nvx_engine_reset_streams).  Queued on the engine stream in push order, after the previous block's
-// sequential demod kernels (they still read its y3 buffer and the decoder state) and before this block's cascade.
+// One stream's record of saved state (nvx_engine_save_streams), in 32-bit words: the FIR path's carried rows, then per channel
+// the y3 and correlation histories, ClockState, FsmState, epoch and, for general-NCO engines, the NcoChan row.  The offsets
+// inside a channel's part are fixed; the rest follows from the path's CarriedRows, the channel count and the NCO kind.
+constexpr int kRecY3 = 0, kRecCorr = kRecY3 + 2 * nvx::kHistY, kRecClock = kRecCorr + 2 * nvx::kHistC;
+constexpr int kRecFsm = kRecClock + (int)sizeof(nvx::ClockState) / 4, kRecEpoch = kRecFsm + (int)sizeof(nvx::FsmState) / 4;
+constexpr int kRecNco = kRecEpoch + 2, kRecNcoWords = (int)sizeof(nvx::NcoChan) / 4;
+static_assert(sizeof(nvx::ClockState) % 4 == 0 && sizeof(nvx::FsmState) % 4 == 0 && sizeof(nvx::NcoChan) % 4 == 0, "word records");
+struct StateLayout {
+    long long rows[3];                  // offset of each carried region
+    long long chan;                     // offset of channel 0's part
+    long long ch_words;                 // words per channel
+    long long words;                    // the whole record
+};
+StateLayout state_layout(const long long words[3], int C, bool gen_nco) {
+    StateLayout l;
+    long long at = 0;
+    for (int k = 0; k < 3; ++k) { l.rows[k] = at; at += words[k]; }
+    l.chan = (at + 1) & ~1LL;
+    l.ch_words = kRecNco + (gen_nco ? kRecNcoWords : 0);
+    l.words = l.chan + C * l.ch_words;
+    return l;
+}
+
+// Everything the next block would carry over from the past of the listed streams.  A reset clears it so that each stream restarts
+// as an engine created at its epoch e0 (nvx_engine_reset_streams); a load writes a saved record over it (nvx_engine_load_streams);
+// a save copies it out (nvx_engine_save_streams).  Resets and loads are queued on the engine stream in push order, after the
+// previous block's sequential demod kernels (they still read its y3 buffer and the decoder state) and before this block's cascade.
 struct ResetArgs {
     const int* streams;                 // [gridDim.x] local stream indices
+    const int* recs;                    // [gridDim.x] record each stream loads, -1 = reset (null when saving)
+    uint32_t* rec;                      // records [][lay.words]: a load's input, a save's output (record k = streams[k])
+    StateLayout lay;
     int C;                              // channels per stream
     long long e0;                       // the new epoch, 900 Hz samples (a multiple of 567)
     nvx::CarriedRows rows;              // what the engine's FIR path carries into the next block
@@ -74,9 +102,40 @@ struct ResetArgs {
     nvx::NcoChan* nco;                  // general-NCO rows (their phase origin moves to e0), or null: the reference table
 };
 
-// one CTA per listed stream
+template <bool kSave>
+__device__ void move_words(uint32_t* state, uint32_t* rec, long long n) {
+    for (long long i = threadIdx.x; i < n; i += blockDim.x) {
+        if (kSave) rec[i] = state[i];
+        else state[i] = rec[i];
+    }
+}
+
+// stream s's carried state -> rec (kSave) or back; the addresses are those reset_streams_kernel clears
+template <bool kSave>
+__device__ void move_stream(const ResetArgs& a, int s, uint32_t* rec) {
+    for (int k = 0; k < 3; ++k) move_words<kSave>(a.rows.base[k] + (size_t)s * a.rows.words[k], rec + a.lay.rows[k], a.rows.words[k]);
+    for (int c = 0; c < a.C; ++c) {
+        const size_t ch = (size_t)s * a.C + c;
+        uint32_t* r = rec + a.lay.chan + c * a.lay.ch_words;
+        move_words<kSave>(reinterpret_cast<uint32_t*>(a.y3_prev + ch * a.y3_pitch + a.n_prev), r + kRecY3, 2 * nvx::kHistY);
+        move_words<kSave>(reinterpret_cast<uint32_t*>(a.corr_prev + ch * a.corr_pitch + a.n_prev), r + kRecCorr, 2 * nvx::kHistC);
+        move_words<kSave>(reinterpret_cast<uint32_t*>(a.clock + ch), r + kRecClock, kRecFsm - kRecClock);
+        move_words<kSave>(reinterpret_cast<uint32_t*>(a.fsm + ch), r + kRecFsm, kRecEpoch - kRecFsm);
+        move_words<kSave>(reinterpret_cast<uint32_t*>(a.epoch + ch), r + kRecEpoch, 2);
+        if (a.nco) move_words<kSave>(reinterpret_cast<uint32_t*>(a.nco + ch), r + kRecNco, kRecNcoWords);
+    }
+}
+
+// one CTA per listed stream: record k <- stream streams[k]
+__global__ void save_streams_kernel(const ResetArgs a) { move_stream<true>(a, a.streams[blockIdx.x], a.rec + (size_t)blockIdx.x * a.lay.words); }
+
+// one CTA per listed stream: its record, or the state of an engine created at e0
 __global__ void reset_streams_kernel(const ResetArgs a) {
     const int s = a.streams[blockIdx.x];
+    if (a.recs[blockIdx.x] >= 0) {
+        move_stream<false>(a, s, a.rec + (size_t)a.recs[blockIdx.x] * a.lay.words);
+        return;
+    }
     const int t = threadIdx.x, nt = blockDim.x;
     for (int k = 0; k < 3; ++k)
         for (long long i = t; i < a.rows.words[k]; i += nt) a.rows.base[k][(size_t)s * a.rows.words[k] + i] = a.rows.fill[k];
@@ -134,18 +193,27 @@ struct nvx_engine {
     // (fir_long.cuh)
     nvx::CascadePath* cp = nullptr;
     nvx::LongPath* lp = nullptr;
+    int path = 0;                         // what saved state records: 0 / 1 = the fused path's tap class, 2 = the long-tap path
     std::vector<int> stream_tag;          // optional [S][C] message tags (read by the worker; changed through markers)
-    // per-stream resets and retunes asked for since the last push; the next push applies them
+    // per-stream resets, retunes and loads asked for since the last push; the next push applies them
     struct TagChange { int stream; std::vector<int> tags; };
-    enum { kListed = 1, kNewNco = 2 };
+    enum { kListed = 1, kNewNco = 2, kLoad = 4 };
     std::vector<int> pend_streams;        // in call order, each once
-    std::vector<uint8_t> pend_flags;      // [S] kListed | kNewNco
+    std::vector<uint8_t> pend_flags;      // [S] kListed | kNewNco | kLoad
     std::vector<TagChange> pend_tags;
-    int* d_reset_list = nullptr;          // [S] the streams of one push's reset kernel
-    void* h_reset = nullptr;              // pinned: [S][C] NcoChan rows to upload, then [S] ints (the list)
+    std::vector<int> pend_rec;            // [S] with kLoad: the stream's record in pend_records / pend_text
+    std::vector<uint32_t> pend_records;   // loaded records [][layout words], epochs and NCO phases already moved to this engine
+    std::vector<std::vector<nvx::MessageAssembler::Channel>> pend_text;   // [record][C] the loaded partial lines and messages
+    bool adopted = false;                 // a load placed this engine, which had pushed nothing, at the saved position
+    int* d_reset_list = nullptr;          // [2 S] the streams of one push's reset kernel, then the record each loads (-1: none)
+    void* h_reset = nullptr;              // pinned: [S][C] NcoChan rows to upload, then [2 S] ints (the list)
     cudaEvent_t reset_copied = nullptr;   // the copies out of h_reset are over
-    // what the worker does before it assembles block `block`: drop the reset streams' partial lines and messages, switch tags
-    struct Marker { long long block; std::vector<int> streams; std::vector<TagChange> tags; };
+    uint32_t* d_records = nullptr;        // records of one save (gather output) or of one push's loads; grown on demand
+    size_t records_cap = 0;               // bytes
+    // what the worker does before it assembles block `block`: drop the reset streams' partial lines and messages, put in the
+    // loaded streams' ones, switch tags
+    struct Loaded { int stream; std::vector<nvx::MessageAssembler::Channel> text; };
+    struct Marker { long long block; std::vector<int> streams; std::vector<TagChange> tags; std::vector<Loaded> loads; };
     std::deque<Marker> markers;           // guarded by mu, in push order
     nvx::MessageAssembler assembler;
     std::vector<nvx::AssembledMessage> ready, handed;
@@ -196,7 +264,7 @@ int free_engine(nvx_engine* e) {
     }
     if (e->stream_copy) cudaStreamDestroy(e->stream_copy);
     cudaFree(e->d_nco_ch);
-    cudaFree(e->db.epoch); cudaFree(e->d_reset_list); cudaFreeHost(e->h_reset);
+    cudaFree(e->db.epoch); cudaFree(e->d_reset_list); cudaFreeHost(e->h_reset); cudaFree(e->d_records);
     if (e->reset_copied) cudaEventDestroy(e->reset_copied);
     nvx::cascade_path_free(e->cp);
     nvx::long_path_free(e->lp);
@@ -226,6 +294,9 @@ int reset_state(nvx_engine* e) {
     for (int s : e->pend_streams) e->pend_flags[(size_t)s] = 0;
     e->pend_streams.clear();
     e->pend_tags.clear();
+    e->pend_records.clear();
+    e->pend_text.clear();
+    e->adopted = false;
     if (e->d_nco_ch)   // every row's phase origin back to 0
         CU_TRY(cudaMemcpyAsync(e->d_nco_ch, e->nco_host.data(), e->nco_host.size() * sizeof(nvx::NcoChan), cudaMemcpyHostToDevice, e->stream));
     if (e->lp) CU_TRY(nvx::long_path_reset(e->lp, e->stream));
@@ -334,6 +405,8 @@ void worker_main(nvx_engine* e) {
         for (const auto& m : take) {       // blocks before this one were assembled under the old state and tags
             for (int s : m.streams)
                 for (int c = 0; c < e->C; ++c) e->assembler.reset_channel(s * e->C + c);
+            for (const auto& l : m.loads)
+                for (int c = 0; c < e->C; ++c) e->assembler.set_channel(l.stream * e->C + c, l.text[(size_t)c]);
             for (const auto& t : m.tags) set_tags(e, t);
         }
         int rc = 0;
@@ -398,57 +471,98 @@ int path_report(nvx_engine* e, int rc, const nvx::PathReport& rep) {
     return rc;
 }
 
-// the resets asked for since the last push, queued in front of this block (b = its buffer index): NCO rows of retuned streams,
-// the reset kernel, and the marker that tells the worker from which block on the streams' messages start over
-int apply_resets(nvx_engine* e, int b) {
+// the addresses of every stream's carried state as the next block reads it (list, records and e0 are the caller's)
+ResetArgs state_args(nvx_engine* e) {
+    using namespace nvx;
+    ResetArgs a = {};
+    a.C = e->C;
+    a.rows = e->lp ? long_path_carried(e->lp) : cascade_path_carried(e->cp);
+    a.lay = state_layout(a.rows.words, e->C, e->d_nco_ch != nullptr);
+    a.y3_prev = e->y3buf[(e->blocks + kBuf - 1) % kBuf];
+    a.y3_pitch = kHistY + e->P_max;
+    a.corr_prev = e->corrbuf[(e->blocks & 1) ^ 1];
+    a.corr_pitch = kHistC + e->P_max + kPadC;
+    a.n_prev = e->last_P;
+    a.clock = e->db.clock; a.fsm = e->db.fsm; a.epoch = e->db.epoch;
+    a.nco = e->d_nco_ch;
+    return a;
+}
+
+int reset_buffers(nvx_engine* e) {
+    if (e->d_reset_list) return 0;
+    CU_TRY(cudaMalloc(&e->d_reset_list, 2 * (size_t)e->S * sizeof(int)));
+    CU_TRY(cudaHostAlloc(&e->h_reset, (size_t)e->S * e->C * sizeof(nvx::NcoChan) + 2 * (size_t)e->S * sizeof(int), cudaHostAllocDefault));
+    CU_TRY(cudaEventCreateWithFlags(&e->reset_copied, cudaEventDisableTiming));
+    CU_TRY(cudaEventRecord(e->reset_copied, e->stream));
+    return 0;
+}
+
+// d_records holds at least `bytes` (the engine stream's earlier work on it is over before it is replaced)
+int records_buffer(nvx_engine* e, size_t bytes) {
+    if (e->records_cap >= bytes) return 0;
+    CU_TRY(cudaStreamSynchronize(e->stream));
+    cudaFree(e->d_records);
+    e->d_records = nullptr;
+    e->records_cap = 0;
+    CU_TRY(cudaMalloc(&e->d_records, bytes));
+    e->records_cap = bytes;
+    return 0;
+}
+
+// the resets and loads asked for since the last push, queued in front of this block: NCO rows of retuned and loaded streams, the
+// loaded records, the reset kernel, and the marker that tells the worker from which block on the streams' messages start over
+// (or go on from the loaded partial lines and messages)
+int apply_resets(nvx_engine* e) {
     using namespace nvx;
     const int count = (int)e->pend_streams.size();
     if (!count) return 0;
     const size_t rows_bytes = (size_t)e->S * e->C * sizeof(NcoChan);
-    if (!e->d_reset_list) {
-        CU_TRY(cudaMalloc(&e->d_reset_list, (size_t)e->S * sizeof(int)));
-        CU_TRY(cudaHostAlloc(&e->h_reset, rows_bytes + (size_t)e->S * sizeof(int), cudaHostAllocDefault));
-        CU_TRY(cudaEventCreateWithFlags(&e->reset_copied, cudaEventDisableTiming));
-    } else {
-        CU_TRY(cudaEventSynchronize(e->reset_copied));      // the previous copies out of h_reset are over
-    }
+    if (int rc = reset_buffers(e)) return rc;
+    CU_TRY(cudaEventSynchronize(e->reset_copied));      // the previous copies out of h_reset are over
     NcoChan* h_rows = static_cast<NcoChan*>(e->h_reset);
     int* h_list = reinterpret_cast<int*>(static_cast<char*>(e->h_reset) + rows_bytes);
     int retuned = 0;
+    nvx_engine::Marker mk;
     for (int i = 0; i < count; ++i) {
         const int s = e->pend_streams[(size_t)i];
+        const uint8_t f = e->pend_flags[(size_t)s];
         h_list[i] = s;
-        if (e->pend_flags[(size_t)s] & nvx_engine::kNewNco) {
+        h_list[count + i] = f & nvx_engine::kLoad ? e->pend_rec[(size_t)s] : -1;
+        if (f & nvx_engine::kNewNco) {
             NcoChan* src = h_rows + (size_t)retuned++ * e->C;
             memcpy(src, &e->nco_host[(size_t)s * e->C], e->C * sizeof(NcoChan));
             CU_TRY(cudaMemcpyAsync(e->d_nco_ch + (size_t)s * e->C, src, e->C * sizeof(NcoChan), cudaMemcpyHostToDevice, e->stream));
         }
+        if (f & nvx_engine::kLoad) mk.loads.push_back({s, std::move(e->pend_text[(size_t)e->pend_rec[(size_t)s]])});
+        else mk.streams.push_back(s);
         e->pend_flags[(size_t)s] = 0;
     }
-    CU_TRY(cudaMemcpyAsync(e->d_reset_list, h_list, (size_t)count * sizeof(int), cudaMemcpyHostToDevice, e->stream));
+    CU_TRY(cudaMemcpyAsync(e->d_reset_list, h_list, 2 * (size_t)count * sizeof(int), cudaMemcpyHostToDevice, e->stream));
     CU_TRY(cudaEventRecord(e->reset_copied, e->stream));
+    ResetArgs ra = state_args(e);
+    if (!e->pend_records.empty()) {
+        const size_t bytes = e->pend_records.size() * sizeof(uint32_t);
+        if (int rc = records_buffer(e, bytes)) return rc;
+        CU_TRY(cudaMemcpyAsync(e->d_records, e->pend_records.data(), bytes, cudaMemcpyHostToDevice, e->stream));
+        ra.rec = e->d_records;
+    }
     if (e->blocks > 0) CU_TRY(cudaStreamWaitEvent(e->stream, e->demod_done[e->last_buf], 0));
-    ResetArgs ra = {};
     ra.streams = e->d_reset_list;
-    ra.C = e->C;
+    ra.recs = e->d_reset_list + count;
     ra.e0 = e->sb_abs - e->sb_abs % kCorrLen;
-    ra.rows = e->lp ? long_path_carried(e->lp) : cascade_path_carried(e->cp);
-    ra.y3_prev = e->y3buf[(b + kBuf - 1) % kBuf];
-    ra.y3_pitch = kHistY + e->P_max;
-    ra.corr_prev = e->corrbuf[(e->blocks & 1) ^ 1];
-    ra.corr_pitch = kHistC + e->P_max + kPadC;
-    ra.n_prev = e->last_P;
-    ra.clock = e->db.clock; ra.fsm = e->db.fsm; ra.epoch = e->db.epoch;
-    ra.nco = e->d_nco_ch;
     reset_streams_kernel<<<(unsigned)count, 256, 0, e->stream>>>(ra);
     CU_TRY(cudaGetLastError());
     e->stats.aux_launches++;
+    mk.block = e->blocks;
+    mk.tags = std::move(e->pend_tags);
     {
         std::lock_guard<std::mutex> lk(e->mu);
-        e->markers.push_back({e->blocks, std::move(e->pend_streams), std::move(e->pend_tags)});
+        e->markers.push_back(std::move(mk));
     }
     e->pend_streams.clear();
     e->pend_tags.clear();
+    e->pend_records.clear();
+    e->pend_text.clear();
     return 0;
 }
 
@@ -462,7 +576,7 @@ int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fm
     e->fmt = (int)fmt;                              // only a block that is accepted fixes the format
     const int b = (int)(e->blocks % kBuf);
     wait_drained(e, e->blocks - kBuf + 1);          // block (blocks - kBuf) used these buffers: long finished, normally
-    if (int rc = apply_resets(e, b)) return rc;
+    if (int rc = apply_resets(e)) return rc;
     if (e->timing && e->ev_used > 4000) {            // bound the event pool in long timed runs
         CU_TRY(cudaStreamSynchronize(e->stream));
         CU_TRY(cudaStreamSynchronize(e->stream_demod));
@@ -553,6 +667,80 @@ int push_host(nvx_engine* e, const void* iq, long long n, nvx::SampleFmt fmt) {
     return 0;
 }
 
+// ---- saved stream state (nvx_engine_save_streams): header | count device records of rec_words words | per record and channel:
+// tag, in_message, the lengths of line / text / bbbb, then their bytes.  Native byte order.
+constexpr uint32_t kStateMagic = 0x5358564eu;      // "NVXS"
+constexpr uint32_t kStateVersion = 1;
+constexpr long long kStateGrid = (long long)nvx::kCorrLen * nvx::kSuper;     // 158760: positions must agree modulo this
+struct StateHeader {
+    uint32_t magic, version;
+    uint64_t bytes;                     // the whole state
+    uint64_t checksum;                  // hash_bytes of every byte but these eight
+    long long position;                 // E: input samples per stream pushed before the save
+    long long words[3];                 // the FIR path's CarriedRows words
+    uint64_t taps;                      // the path's tap hash
+    long long rec_words;                // words per device record
+    int32_t count, n_channels, fmt, path, gen_nco, reserved;
+};
+static_assert(sizeof(StateHeader) == 96, "state header layout");
+constexpr size_t kChecksumAt = offsetof(StateHeader, checksum);
+using ChannelText = nvx::MessageAssembler::Channel;
+
+uint64_t state_checksum(const uint8_t* p, size_t n) {
+    return nvx::hash_bytes(p + kChecksumAt + 8, n - kChecksumAt - 8, nvx::hash_bytes(p, kChecksumAt));
+}
+
+const char* path_name(int path) { return path == 0 ? "fused path (reference tap class)" : path == 1 ? "fused path (medium tap class)" : "long-tap path"; }
+
+// validates a saved state completely (nothing is half-applied) and returns its header and [record][channel] texts and tags
+int parse_state(const void* state, size_t size, StateHeader* h, std::vector<std::vector<ChannelText>>* text, std::vector<std::vector<int>>* tags) {
+    if (!state || size < sizeof(StateHeader)) return fail(NVX_ERR_ARG, "saved stream state: %zu bytes, shorter than its %zu-byte header", state ? size : 0, sizeof(StateHeader));
+    const uint8_t* p = static_cast<const uint8_t*>(state);
+    memcpy(h, p, sizeof *h);
+    if (h->magic != kStateMagic) return fail(NVX_ERR_ARG, "saved stream state: bad magic number 0x%08x", h->magic);
+    if (h->version != kStateVersion) return fail(NVX_ERR_ARG, "saved stream state: version %u, this library reads version %u", h->version, kStateVersion);
+    if (h->bytes != size) return fail(NVX_ERR_ARG, "saved stream state: %zu bytes given, the state has %llu (truncated?)", size, (unsigned long long)h->bytes);
+    if (state_checksum(p, size) != h->checksum) return fail(NVX_ERR_ARG, "saved stream state: checksum mismatch (the bytes were altered)");
+    const long long rec_words = state_layout(h->words, h->n_channels, h->gen_nco != 0).words;
+    if (h->count < 0 || h->n_channels < 1 || h->n_channels > nvx::kMaxChannels || h->fmt < 0 || h->fmt >= nvx::kSampleFmts || h->path < 0 ||
+        h->path > 2 || (h->gen_nco != 0 && h->gen_nco != 1) || h->position < 0 || h->position % nvx::kSuper || h->words[0] < 0 ||
+        h->words[1] < 0 || h->words[2] < 0 || h->rec_words != rec_words)
+        return fail(NVX_ERR_ARG, "saved stream state: inconsistent header");
+    size_t at = sizeof(StateHeader);
+    if ((size - at) / sizeof(uint32_t) / (size_t)rec_words < (size_t)h->count) return fail(NVX_ERR_ARG, "saved stream state: records cut short");
+    at += (size_t)h->count * rec_words * sizeof(uint32_t);
+    text->assign((size_t)h->count, std::vector<ChannelText>((size_t)h->n_channels));
+    tags->assign((size_t)h->count, std::vector<int>((size_t)h->n_channels));
+    for (int k = 0; k < h->count; ++k)
+        for (int c = 0; c < h->n_channels; ++c) {
+            int32_t v[5];
+            if (size - at < sizeof v) return fail(NVX_ERR_ARG, "saved stream state: message part cut short");
+            memcpy(v, p + at, sizeof v);
+            at += sizeof v;
+            ChannelText& t = (*text)[(size_t)k][(size_t)c];
+            (*tags)[(size_t)k][(size_t)c] = v[0];
+            t.in_message = v[1] != 0;
+            std::string* str[3] = {&t.line, &t.text, &t.bbbb};
+            for (int i = 0; i < 3; ++i) {
+                if (v[2 + i] < 0 || (size_t)v[2 + i] > size - at) return fail(NVX_ERR_ARG, "saved stream state: message part cut short");
+                str[i]->assign(reinterpret_cast<const char*>(p + at), (size_t)v[2 + i]);
+                at += (size_t)v[2 + i];
+            }
+        }
+    if (at != size) return fail(NVX_ERR_ARG, "saved stream state: %zu bytes after the last record", size - at);
+    return 0;
+}
+
+// streams[0..count) are local streams, each listed once
+int check_stream_list(const nvx_engine* e, const int* streams, int count) {
+    std::vector<char> seen((size_t)e->S, 0);
+    for (int i = 0; i < count; ++i) {
+        if (streams[i] < 0 || streams[i] >= e->S) return fail(NVX_ERR_ARG, "stream %d outside 0..%d", streams[i], e->S - 1);
+        if (seen[(size_t)streams[i]]++) return fail(NVX_ERR_ARG, "stream %d is listed twice", streams[i]);
+    }
+    return 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -602,6 +790,7 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
     e->S = cfg->n_streams;
     e->channels = C * e->S;
     e->pend_flags.assign((size_t)e->S, 0);
+    e->pend_rec.assign((size_t)e->S, -1);
     e->P_max = (int)(cfg->max_block / nvx::kSuper);
     // tap counts: reference lengths unless given; sets up to 37/47/71 and up to 61/75/111 run through the fused kernel
     // (zero-padded to the class), longer ones through the long-tap path
@@ -615,6 +804,7 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
     // the FIR path: the fused cascade for sets it takes, else the long-tap path; only the fused reference class serves other than
     // the reference's two channels
     const int tap_class = nvx::cascade_tap_class(n[0], n[1], n[2]);
+    e->path = tap_class >= 0 ? tap_class : 2;
     if (C != 2 && tap_class != 0) {
         delete e;
         return fail(NVX_ERR_ARG, "n_channels = %d is served by the fused kernel's reference tap class only (up to %d / %d / %d taps)", C, NVX_T1, NVX_T2, NVX_T3);
@@ -709,7 +899,7 @@ int nvx_engine_reset_streams(nvx_engine* e, const int* streams, int count) {
     for (int i = 0; i < count; ++i) {
         uint8_t& f = e->pend_flags[(size_t)streams[i]];
         if (!(f & nvx_engine::kListed)) e->pend_streams.push_back(streams[i]);
-        f |= nvx_engine::kListed;
+        f = (uint8_t)((f | nvx_engine::kListed) & ~nvx_engine::kLoad);     // a reset after a load wins
     }
     return 0;
 }
@@ -725,6 +915,148 @@ int nvx_engine_retune_stream(nvx_engine* e, int stream, const double* nco_hz, co
     if (freq_tag) e->pend_tags.push_back({stream, std::vector<int>(freq_tag, freq_tag + e->C)});
     e->pend_flags[(size_t)stream] |= nvx_engine::kNewNco;
     return nvx_engine_reset_streams(e, &stream, 1);
+}
+
+int nvx_engine_save_streams(nvx_engine* e, const int* streams, int count, void* out, size_t cap, size_t* size) {
+    if (!e || !size || count < 0 || (count && !streams)) return fail(NVX_ERR_ARG, "bad argument");
+    if (int rc = check_stream_list(e, streams, count)) return rc;
+    if (int rc = sync_engine(e)) return rc;
+    if (e->blocks == 0) return fail(NVX_ERR_ARG, "nothing has been pushed since create or reset: there is no stream state to save");
+    for (int i = 0; i < count; ++i)
+        if (e->pend_flags[(size_t)streams[i]])
+            return fail(NVX_ERR_ARG, "stream %d has a reset, retune or load pending: push a block before saving it", streams[i]);
+    ResetArgs a = state_args(e);
+    std::vector<uint8_t> msg;           // the message part: tags and the assembler's partial lines and messages
+    for (int i = 0; i < count; ++i)
+        for (int c = 0; c < e->C; ++c) {
+            const size_t ch = (size_t)streams[i] * e->C + c;
+            const ChannelText& t = e->assembler.channel((int)ch);
+            const int32_t v[5] = {e->stream_tag.empty() ? e->cfg.freq_tag[c & 1] : e->stream_tag[ch], t.in_message ? 1 : 0,
+                                  (int32_t)t.line.size(), (int32_t)t.text.size(), (int32_t)t.bbbb.size()};
+            const uint8_t* pv = reinterpret_cast<const uint8_t*>(v);
+            msg.insert(msg.end(), pv, pv + sizeof v);
+            for (const std::string* str : {&t.line, &t.text, &t.bbbb}) msg.insert(msg.end(), str->begin(), str->end());
+        }
+    const size_t rec_bytes = (size_t)count * a.lay.words * sizeof(uint32_t);
+    *size = sizeof(StateHeader) + rec_bytes + msg.size();
+    if (!out) return 0;
+    if (cap < *size) return fail(NVX_ERR_OVERFLOW, "the saved state needs %zu bytes, the buffer holds %zu", *size, cap);
+    uint8_t* o = static_cast<uint8_t*>(out);
+    if (count) {
+        if (int rc = reset_buffers(e)) return rc;
+        if (int rc = records_buffer(e, rec_bytes)) return rc;
+        CU_TRY(cudaMemcpyAsync(e->d_reset_list, streams, (size_t)count * sizeof(int), cudaMemcpyHostToDevice, e->stream));
+        a.streams = e->d_reset_list;
+        a.rec = e->d_records;
+        save_streams_kernel<<<(unsigned)count, 256, 0, e->stream>>>(a);
+        CU_TRY(cudaGetLastError());
+        CU_TRY(cudaMemcpyAsync(o + sizeof(StateHeader), e->d_records, rec_bytes, cudaMemcpyDeviceToHost, e->stream));
+        CU_TRY(cudaStreamSynchronize(e->stream));
+    }
+    StateHeader h = {};
+    h.magic = kStateMagic;
+    h.version = kStateVersion;
+    h.bytes = *size;
+    h.position = e->sb_abs * nvx::kSuper;
+    for (int k = 0; k < 3; ++k) h.words[k] = a.rows.words[k];
+    h.taps = e->lp ? nvx::long_path_taps_hash(e->lp) : nvx::cascade_path_taps_hash(e->cp);
+    h.rec_words = a.lay.words;
+    h.count = count;
+    h.n_channels = e->C;
+    h.fmt = e->fmt;
+    h.path = e->path;
+    h.gen_nco = e->d_nco_ch != nullptr;
+    memcpy(o, &h, sizeof h);
+    if (!msg.empty()) memcpy(o + sizeof h + rec_bytes, msg.data(), msg.size());
+    h.checksum = state_checksum(o, *size);
+    memcpy(o + kChecksumAt, &h.checksum, sizeof h.checksum);
+    return 0;
+}
+
+int nvx_engine_load_streams(nvx_engine* e, const int* streams, int count, const void* state, size_t size) {
+    using namespace nvx;
+    if (!e || count < 0 || (count && !streams)) return fail(NVX_ERR_ARG, "bad argument");
+    StateHeader h;
+    std::vector<std::vector<ChannelText>> text;
+    std::vector<std::vector<int>> tags;
+    if (int rc = parse_state(state, size, &h, &text, &tags)) return rc;
+    if (h.count != count) return fail(NVX_ERR_ARG, "the saved state holds %d streams, %d were listed", h.count, count);
+    if (int rc = check_stream_list(e, streams, count)) return rc;
+    const bool gen = e->d_nco_ch != nullptr;
+    if (h.path != e->path) return fail(NVX_ERR_ARG, "the state was saved on the %s, this engine runs the %s", path_name(h.path), path_name(e->path));
+    if (h.taps != (e->lp ? long_path_taps_hash(e->lp) : cascade_path_taps_hash(e->cp))) return fail(NVX_ERR_ARG, "the state was saved with another tap set");
+    if (h.n_channels != e->C) return fail(NVX_ERR_ARG, "the state has %d channels per stream, this engine %d", h.n_channels, e->C);
+    if ((h.gen_nco != 0) != gen)
+        return fail(NVX_ERR_ARG, "the state was saved %s, this engine runs %s", h.gen_nco ? "with per-stream NCO offsets" : "on the reference NCO table",
+                    gen ? "per-stream NCO offsets" : "the reference NCO table");
+    if (e->fmt >= 0 && e->fmt != h.fmt) return fail(NVX_ERR_ARG, "the state holds sample format %d, this engine takes format %d", h.fmt, e->fmt);
+    // an engine that has pushed nothing since create or reset adopts the saved position; any other must be on the same grid
+    const bool adopt = e->blocks == 0 && !e->adopted;
+    const long long here = adopt ? h.position : e->sb_abs * kSuper;
+    if ((here - h.position) % kStateGrid)
+        return fail(NVX_ERR_ARG, "the state was saved after input sample %lld, this engine is at %lld: the two must agree modulo %lld (567 x 280)",
+                    (long long)h.position, here, kStateGrid);
+    CU_TRY(cudaSetDevice(e->cfg.device));
+    if (e->cp) {      // a fresh engine's tails take the saved format now (it would fill them with its silence at the first push)
+        PathReport rep;
+        const int rc = cascade_path_prepare(e->cp, (SampleFmt)h.fmt, e->stream, &rep);
+        if (path_report(e, rc, rep)) return rc;
+    }
+    const CarriedRows rows = e->lp ? long_path_carried(e->lp) : cascade_path_carried(e->cp);
+    for (int k = 0; k < 3; ++k)
+        if (rows.words[k] != h.words[k])
+            return fail(NVX_ERR_ARG, "the state carries %lld words of FIR stage %d per stream, this engine %lld", (long long)h.words[k], k + 1, rows.words[k]);
+
+    // accepted: nothing below fails
+    if (adopt) {      // its other streams start as streams reset at the saved position
+        e->sb_abs = h.position / kSuper;
+        e->adopted = true;
+        for (int s = 0; s < e->S; ++s) nvx_engine_reset_streams(e, &s, 1);
+    }
+    e->fmt = h.fmt;
+    const StateLayout lay = state_layout(h.words, e->C, gen);
+    const long long d_sb = (here - h.position) / kSuper;                        // epochs: 900 Hz samples
+    const long long d_tick = ((here - h.position) / NVX_D1) % kNcoDen;         // NCO phases: 63 kHz ticks
+    const uint32_t* recs = reinterpret_cast<const uint32_t*>(static_cast<const uint8_t*>(state) + sizeof(StateHeader));
+    for (int k = 0; k < count; ++k) {
+        const int s = streams[k];
+        const size_t r0 = e->pend_records.size();
+        e->pend_records.resize(r0 + (size_t)lay.words);
+        memcpy(&e->pend_records[r0], recs + (size_t)k * lay.words, (size_t)lay.words * sizeof(uint32_t));
+        for (int c = 0; c < e->C; ++c) {
+            uint32_t* r = &e->pend_records[r0 + (size_t)(lay.chan + c * lay.ch_words)];
+            long long epoch;
+            memcpy(&epoch, r + kRecEpoch, sizeof epoch);
+            epoch += d_sb;
+            memcpy(r + kRecEpoch, &epoch, sizeof epoch);
+            if (gen) {     // the row keeps its phase: (tick + d_tick) num + phase0' = tick num + phase0
+                NcoChan n;
+                memcpy(&n, r + kRecNco, sizeof n);
+                n.phase0 = (int)(((n.phase0 - (d_tick + kNcoDen) % kNcoDen * n.num) % kNcoDen + kNcoDen) % kNcoDen);
+                memcpy(r + kRecNco, &n, sizeof n);
+                e->nco_host[(size_t)s * e->C + c] = {n.num, 0, n.step};     // a later reset or nvx_engine_reset keeps the offsets
+            }
+        }
+        uint8_t& f = e->pend_flags[(size_t)s];
+        if (!(f & nvx_engine::kListed)) e->pend_streams.push_back(s);
+        f |= nvx_engine::kListed | nvx_engine::kLoad | (gen ? nvx_engine::kNewNco : 0);
+        e->pend_rec[(size_t)s] = (int)e->pend_text.size();
+        e->pend_text.push_back(std::move(text[(size_t)k]));
+        e->pend_tags.push_back({s, std::move(tags[(size_t)k])});
+    }
+    return 0;
+}
+
+int nvx_stream_state_info(const void* state, size_t size, int* count, long long* position, int* n_channels, int* sample_format) {
+    StateHeader h;
+    std::vector<std::vector<ChannelText>> text;
+    std::vector<std::vector<int>> tags;
+    if (int rc = parse_state(state, size, &h, &text, &tags)) return rc;
+    if (count) *count = h.count;
+    if (position) *position = h.position;
+    if (n_channels) *n_channels = h.n_channels;
+    if (sample_format) *sample_format = h.fmt;
+    return 0;
 }
 
 int nvx_engine_push_device_f32(nvx_engine* e, const void* d_iq, long long n) {

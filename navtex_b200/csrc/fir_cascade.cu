@@ -5,6 +5,7 @@
 #include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
+#include <string.h>
 
 #include "../../include/navtex_b200.h"
 
@@ -187,6 +188,21 @@ float2 reference_nco(int k) { return make_float2((float)cos((2 * M_PI * k * 1400
 static const double kRef1[NVX_T1] = {NVX_H1_VALUES}, kRef2[NVX_T2] = {NVX_H2_VALUES}, kRef3[NVX_T3] = {NVX_H3_VALUES};
 const double* const kRefTaps[3] = {kRef1, kRef2, kRef3};
 
+uint64_t hash_bytes(const void* p, size_t n, uint64_t h) {
+    const uint8_t* b = static_cast<const uint8_t*>(p);
+    for (; n >= 8; n -= 8, b += 8) {
+        uint64_t w;
+        memcpy(&w, b, 8);
+        h = (h ^ w) * 0x100000001b3ULL;
+        h ^= h >> 29;
+    }
+    for (; n; --n, ++b) {
+        h = (h ^ *b) * 0x100000001b3ULL;
+        h ^= h >> 29;
+    }
+    return h;
+}
+
 // 32-bit-element view of a stream-major sample array: [rows][2 * cols] floats for float2 samples, [rows][cols] words for
 // short2 samples (one word = one I,Q pair), [rows][cols / 2] words for 8-bit pairs (one word = two pairs; cols is a multiple
 // of 280); box = one ring stage x 32 rows
@@ -366,18 +382,26 @@ CarriedRows cascade_path_carried(const CascadePath* cp) {
 }
 
 // the first launch is nvx_stats.cascade_launches; the second channel pass and the tail carry count in rep->launches
+int cascade_path_prepare(CascadePath* cp, SampleFmt fmt, cudaStream_t stream, PathReport* rep) {
+    if (cp->fmt == (int)fmt) return 0;
+    // the warm-up before the first block sees silence: the value 0, which is the byte 128 in 8-bit offset binary
+    for (int k = 0; k < 2; ++k) {
+        if (int rc = check(rep, cudaMemsetAsync(cp->tail[k], fmt == SampleFmt::U8 ? 128 : 0, (size_t)cp->S * cp->halo * sample_bytes(fmt), stream),
+                           "fused path: filling the input tail"))
+            return rc;
+        if (int rc = encode_rows(&cp->map_tail[k], cp->tail[k], cp->halo, cp->S, fmt, rep)) return rc;
+    }
+    cp->fmt = (int)fmt;
+    return 0;
+}
+
+uint64_t cascade_path_taps_hash(const CascadePath* cp) {
+    return cp->tap_class == 1 ? hash_bytes(&cp->taps.t1, sizeof cp->taps.t1) : hash_bytes(&cp->taps.t0, sizeof cp->taps.t0);
+}
+
 int cascade_path_run(CascadePath* cp, const void* x, long long n, SampleFmt fmt, long long sb_abs, float2* y3, long long y3_pitch,
                      long long y3_off, cudaStream_t stream, cudaEvent_t after_fir, PathReport* rep) {
-    if (cp->fmt != (int)fmt) {
-        // the warm-up before the first block sees silence: the value 0, which is the byte 128 in 8-bit offset binary
-        for (int k = 0; k < 2; ++k) {
-            if (int rc = check(rep, cudaMemsetAsync(cp->tail[k], fmt == SampleFmt::U8 ? 128 : 0, (size_t)cp->S * cp->halo * sample_bytes(fmt), stream),
-                               "fused path: filling the input tail"))
-                return rc;
-            if (int rc = encode_rows(&cp->map_tail[k], cp->tail[k], cp->halo, cp->S, fmt, rep)) return rc;
-        }
-        cp->fmt = (int)fmt;
-    }
+    if (int rc = cascade_path_prepare(cp, fmt, stream, rep)) return rc;
     CascadeArgs ca;
     if (int rc = encode_rows(&ca.map_x, x, n, cp->S, fmt, rep)) return rc;
     ca.map_tail = cp->map_tail[cp->cur];

@@ -229,6 +229,10 @@ EncodeTiledFn tensor_map_encoder();
 // entry k of the reference's NCO table: (cos, -sin)(2 pi k 14000 / 63000), fir2cpp.C:105-106, rounded once to float
 float2 reference_nco(int k);
 extern const double* const kRefTaps[3];      // the reference tap sets of stages 1, 2 and 3 (NVX_H*_VALUES)
+// 64-bit hash of n bytes, continuing from h: every step is a bijection of the running value, so changing any one 8-byte word
+// (or tail byte) changes the result (saved stream state: checksum and tap fingerprint)
+constexpr uint64_t kHashSeed = 1469598103934665603ULL;
+uint64_t hash_bytes(const void* p, size_t n, uint64_t h = kHashSeed);
 
 int cascade_tap_class(int n1, int n2, int n3);   // tap class a set of lengths needs, or -1 if it takes the long-tap path
 
@@ -241,7 +245,12 @@ struct CascadePath;
 int cascade_path_create(int S, int C, const int n[3], const double* const h[3], const NcoChan* nco, int device, int reserved_sms,
                         CascadePath** out, PathReport* rep);
 void cascade_path_reset(CascadePath* cp);        // the next block starts after silence, in whatever format it comes
+// the carried tails hold format fmt: if they hold another (or none), both are filled with its silence and described to the TMA
+// unit again, queued on `stream`.  Every run does this first; a load of saved state into a fresh engine does it before the
+// state's tails are written.  Returns 0 or an NVX_ERR_* code.
+int cascade_path_prepare(CascadePath* cp, SampleFmt fmt, cudaStream_t stream, PathReport* rep);
 CarriedRows cascade_path_carried(const CascadePath* cp);
+uint64_t cascade_path_taps_hash(const CascadePath* cp);   // of the tap set as the kernels read it (class, zero padding included)
 // one block x[S][n] in format fmt that starts at 900 Hz sample sb_abs; the 900 Hz output goes to y3[C S][y3_pitch] from y3_off
 // on.  after_fir (if not null) is recorded once the FIR work is queued, before the tail carry.  Returns 0 or an NVX_ERR_* code.
 int cascade_path_run(CascadePath* cp, const void* x, long long n, SampleFmt fmt, long long sb_abs, float2* y3, long long y3_pitch,

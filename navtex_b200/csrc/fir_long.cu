@@ -374,6 +374,15 @@ CarriedRows long_path_carried(const LongPath* lp) {
     return r;
 }
 
+uint64_t long_path_taps_hash(const LongPath* lp) {
+    uint64_t h = kHashSeed;
+    for (int k = 0; k < 3; ++k) {
+        h = hash_bytes(&lp->st[k], sizeof lp->st[k], h);
+        h = hash_bytes(lp->taps[k].h, sizeof lp->taps[k].h, h);
+    }
+    return h;
+}
+
 // 3 stage launches, 3 history carries and, for 8-bit input, the widening kernel: all in rep->launches
 int long_path_run(LongPath* lp, const void* x, long long n, SampleFmt fmt, long long sb_abs, float2* y3, long long y3_pitch,
                   long long y3_off, cudaStream_t stream, cudaEvent_t after_fir, PathReport* rep) {

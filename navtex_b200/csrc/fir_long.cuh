@@ -86,6 +86,7 @@ cudaError_t long_path_reset(LongPath* lp, cudaStream_t stream);     // zero hist
 // the histories the next block reads: stage k keeps per_stream[k] consecutive rows of H[k] float2 for each stream (1 for stage 1,
 // 2 for stages 2 and 3 -- one per channel -- or 1 for stage 2 when it mixes on load); zeroing a stream's rows restarts its filters
 CarriedRows long_path_carried(const LongPath* lp);
+uint64_t long_path_taps_hash(const LongPath* lp);     // of the stage geometries and the tap blocks the kernels read
 // one block x[S][n] in format fmt that starts at 900 Hz sample sb_abs; the 900 Hz output goes to y3[2 S][y3_pitch] from y3_off on.
 // after_fir (if not null) is recorded after the last launch.  Returns 0 or an NVX_ERR_* code.
 int long_path_run(LongPath* lp, const void* x, long long n, SampleFmt fmt, long long sb_abs, float2* y3, long long y3_pitch,

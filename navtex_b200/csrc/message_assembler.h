@@ -28,11 +28,15 @@ class MessageAssembler {
     // feed `n` event bytes of channel `ch`; completed messages are appended to `out`
     void feed(int ch, int stream, int freq, const unsigned char* ev, size_t n, std::vector<AssembledMessage>* out);
 
-  private:
+    // a channel's partial line and message (nvx_engine_save_streams / nvx_engine_load_streams)
     struct Channel {
         std::string line, text, bbbb;
         bool in_message = false;
     };
+    const Channel& channel(int ch) const { return ch_[(size_t)ch]; }
+    void set_channel(int ch, const Channel& c) { ch_[(size_t)ch] = c; }
+
+  private:
     void line_done(Channel& c, int stream, int freq, std::vector<AssembledMessage>* out);
     std::vector<Channel> ch_;
     regex_t som_, eom_;

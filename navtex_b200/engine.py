@@ -49,7 +49,8 @@ class SynthDesc(C.Structure):
 
 EXPORTS = (
     "nvx_default_config", "nvx_last_error", "nvx_engine_create", "nvx_engine_destroy", "nvx_engine_reset",
-    "nvx_engine_reset_streams", "nvx_engine_retune_stream",
+    "nvx_engine_reset_streams", "nvx_engine_retune_stream", "nvx_engine_save_streams", "nvx_engine_load_streams",
+    "nvx_stream_state_info",
     "nvx_engine_push_host_f32", "nvx_engine_push_host_s16", "nvx_engine_push_host_u8", "nvx_engine_push_device_f32",
     "nvx_engine_push_device_s16", "nvx_engine_push_device_u8",
     "nvx_engine_sync", "nvx_engine_wait_ingest", "nvx_engine_host_pushes", "nvx_engine_wait_ingest_of", "nvx_engine_poll_messages", "nvx_engine_try_poll_messages", "nvx_engine_set_message_callback", "nvx_engine_read_y3",
@@ -82,6 +83,10 @@ def load_library():
     L.nvx_engine_reset.argtypes = [C.c_void_p]
     L.nvx_engine_reset_streams.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.c_int]
     L.nvx_engine_retune_stream.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_int)]
+    L.nvx_engine_save_streams.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.c_int, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
+    L.nvx_engine_load_streams.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.c_int, C.c_void_p, C.c_size_t]
+    L.nvx_stream_state_info.argtypes = [C.c_void_p, C.c_size_t, C.POINTER(C.c_int), C.POINTER(C.c_longlong), C.POINTER(C.c_int),
+                                        C.POINTER(C.c_int)]
     for name in ("nvx_engine_push_host_f32", "nvx_engine_push_host_s16", "nvx_engine_push_host_u8", "nvx_engine_push_device_f32",
                  "nvx_engine_push_device_s16", "nvx_engine_push_device_u8"):
         getattr(L, name).argtypes = [C.c_void_p, C.c_void_p, C.c_longlong]
@@ -165,6 +170,15 @@ def long_tc_band(decimation: int, h):
     return g, hi.reshape(shape), lo.reshape(shape)
 
 
+def stream_state_info(state: bytes) -> dict:
+    """Validate a saved stream state (host only, no GPU) and return its record count, input position (samples per stream),
+    channels per stream and sample format ("f32", "s16" or "u8"); raises NvxError on a corrupt or truncated state."""
+    L = load_library()
+    count, n_ch, fmt, pos = C.c_int(), C.c_int(), C.c_int(), C.c_longlong()
+    _check(L.nvx_stream_state_info(state, len(state), C.byref(count), C.byref(pos), C.byref(n_ch), C.byref(fmt)))
+    return {"count": count.value, "position": pos.value, "n_channels": n_ch.value, "sample_format": ("f32", "s16", "u8")[fmt.value]}
+
+
 def _check(rc, allow_overflow=False):
     if rc == 0 or (allow_overflow and rc == -4):
         return rc
@@ -230,6 +244,23 @@ class Engine:
                 raise NvxError(f"retune_stream needs {self.C} tags, got {t.size}")
             tags = t.ctypes.data_as(C.POINTER(C.c_int))
         _check(self.L.nvx_engine_retune_stream(self._h, stream, f.ctypes.data_as(C.POINTER(C.c_double)), tags))
+
+    def save_streams(self, streams) -> bytes:
+        """The receive state of the listed streams (local indices) after the last pushed block, as one byte string (implies
+        sync; read-only).  Load it into an engine created with the same configuration to continue the streams bit for bit."""
+        s = np.ascontiguousarray(streams, dtype=np.int32).reshape(-1)
+        sp = s.ctypes.data_as(C.POINTER(C.c_int))
+        size = C.c_size_t()
+        _check(self.L.nvx_engine_save_streams(self._h, sp, s.size, None, 0, C.byref(size)))
+        out = C.create_string_buffer(size.value)
+        _check(self.L.nvx_engine_save_streams(self._h, sp, s.size, out, size.value, C.byref(size)))
+        return out.raw[: size.value]
+
+    def load_streams(self, streams, state: bytes):
+        """Record k of a saved state goes to local stream streams[k] at the next push (nvx_engine_load_streams: the position rule
+        and compatibility checks are there)."""
+        s = np.ascontiguousarray(streams, dtype=np.int32).reshape(-1)
+        _check(self.L.nvx_engine_load_streams(self._h, s.ctypes.data_as(C.POINTER(C.c_int)), s.size, state, len(state)))
 
     def push_host(self, iq: np.ndarray):
         """iq: [S, n, 2] (or [S, 2n]) float32, int16 or uint8 (8-bit offset binary, value u - 128), C-contiguous."""
