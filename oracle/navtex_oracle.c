@@ -533,6 +533,25 @@ void nvo_free(nvo_chain *c) {
     free(c);
 }
 
+/* the per-channel tail of the chain: one 900 Hz sample into channel ch's decoder and state machine, with its taps recorded */
+static void chain_900(nvo_chain *c, int ch, double ci, double cq) {
+    if (c->prm.record_taps) bytes_add_2d(&c->y3[ch], ci, cq);
+    c->n3[ch]++;
+    float sums[4];
+    char bit = nvo_decoder_sample(&c->dec[ch], ci, cq, sums);
+    if (c->dec[ch].pick_fresh) {
+        c->dec[ch].pick_fresh = 0;
+        if (c->prm.record_taps) { double rec[2] = {(double)c->n3[ch], c->dec[ch].pick_margin}; bytes_add(&c->pickm[ch], rec, sizeof rec); }
+    }
+    if (bit) {
+        int32_t pos = (int32_t)c->n3[ch];
+        bytes_add_c(&c->bits[ch], bit);
+        bytes_add(&c->bitpos[ch], &pos, sizeof pos);
+        bytes_add(&c->disc[ch], sums, sizeof sums);
+        bsm_bit(&c->bsm[ch], bit);
+    }
+}
+
 static void chain_sample(nvo_chain *c, double xi, double xq) {
     double ai, aq;
     if (!fir_push(&c->f1, xi, xq, &ai, &aq)) return;
@@ -548,21 +567,7 @@ static void chain_sample(nvo_chain *c, double xi, double xq) {
         if (!fir_push(&c->f2[ch], mi, mq, &bi, &bq)) continue;
         if (c->prm.record_taps) bytes_add_2d(&c->y2[ch], bi, bq);
         if (!fir_push(&c->f3[ch], bi, bq, &ci, &cq)) continue;
-        if (c->prm.record_taps) bytes_add_2d(&c->y3[ch], ci, cq);
-        c->n3[ch]++;
-        float sums[4];
-        char bit = nvo_decoder_sample(&c->dec[ch], ci, cq, sums);
-        if (c->dec[ch].pick_fresh) {
-            c->dec[ch].pick_fresh = 0;
-            if (c->prm.record_taps) { double rec[2] = {(double)c->n3[ch], c->dec[ch].pick_margin}; bytes_add(&c->pickm[ch], rec, sizeof rec); }
-        }
-        if (bit) {
-            int32_t pos = (int32_t)c->n3[ch];
-            bytes_add_c(&c->bits[ch], bit);
-            bytes_add(&c->bitpos[ch], &pos, sizeof pos);
-            bytes_add(&c->disc[ch], sums, sizeof sums);
-            bsm_bit(&c->bsm[ch], bit);
-        }
+        chain_900(c, ch, ci, cq);
     }
 }
 
@@ -574,6 +579,10 @@ void nvo_push_f32(nvo_chain *c, const float *iq, size_t n) {
 }
 void nvo_push_s16(nvo_chain *c, const int16_t *iq, size_t n) {
     for (size_t k = 0; k < n; ++k) chain_sample(c, (double)iq[2 * k], (double)iq[2 * k + 1]);   /* capt_sched.c:511 */
+}
+void nvo_push_900(nvo_chain *c, int ch, const double *iq, size_t n) {
+    if (ch < 0 || ch >= c->nch) return;
+    for (size_t k = 0; k < n; ++k) chain_900(c, ch, iq[2 * k], iq[2 * k + 1]);
 }
 
 size_t nvo_y1(const nvo_chain *c, const double **iq) { *iq = (const double *)c->y1.p; return c->y1.n / 16; }

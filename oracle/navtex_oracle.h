@@ -53,6 +53,10 @@ void nvo_free(nvo_chain *c);
 void nvo_push(nvo_chain *c, const double *iq, size_t n);
 void nvo_push_f32(nvo_chain *c, const float *iq, size_t n);
 void nvo_push_s16(nvo_chain *c, const int16_t *iq, size_t n);
+/* feed n 900 Hz samples (interleaved I,Q doubles) straight to channel ch's decoder and state machine, as if they had come out of
+ * its third filter stage; y3 records them.  For tests of the demodulator alone.  A chain is fed through nvo_push* or through
+ * nvo_push_900, never both: the 900 Hz sample counts (bitpos, pick margins) would no longer match either input */
+void nvo_push_900(nvo_chain *c, int ch, const double *iq, size_t n);
 
 /* recorded taps; pointers stay valid until the next push.  counts are complex samples */
 size_t nvo_y1(const nvo_chain *c, const double **iq);

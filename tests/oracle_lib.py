@@ -41,8 +41,7 @@ _lib = None
 def lib():
     global _lib
     if _lib is None:
-        if not os.path.exists(ORACLE_SO):
-            build_oracle()
+        build_oracle()          # every time: make rebuilds a library older than its sources, and leaves a current one alone
         L = C.CDLL(ORACLE_SO)
         L.nvo_new.restype = C.c_void_p
         L.nvo_new.argtypes = [C.POINTER(Params)]
@@ -50,6 +49,7 @@ def lib():
         L.nvo_default_params.argtypes = [C.POINTER(Params)]
         for name, t in (("nvo_push", C.c_double), ("nvo_push_f32", C.c_float), ("nvo_push_s16", C.c_int16)):
             getattr(L, name).argtypes = [C.c_void_p, C.POINTER(t), C.c_size_t]
+        L.nvo_push_900.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_double), C.c_size_t]
         L.nvo_y1.restype = C.c_size_t
         L.nvo_y1.argtypes = [C.c_void_p, C.POINTER(C.POINTER(C.c_double))]
         for name, t in (("nvo_y2", C.c_double), ("nvo_y3", C.c_double), ("nvo_bits", C.c_char),
@@ -118,6 +118,26 @@ def run_oracle(iq, h1=None, h2=None, h3=None, nco_hz=(14000.0, -14000.0), nco_pe
     else:
         iq = iq.astype(np.float64)
         L.nvo_push(ch, iq.ctypes.data_as(C.POINTER(C.c_double)), n)
+    return _collect(L, ch, n_ch)
+
+
+def run_oracle_900(y3_row, freq_tag=518) -> Result:
+    """One channel fed straight at 900 Hz (nvo_push_900): y3_row is a complex 1-D array, taken as FP64.  The Result holds that
+    channel under key "518" (y3 = the input), its decisions, pick margins, events and messages."""
+    L = lib()
+    p = Params()
+    L.nvo_default_params(C.byref(p))
+    p.n_channels = 1
+    p.freq_tag[0] = freq_tag
+    p.record_taps = 1
+    ch = L.nvo_new(C.byref(p))
+    iq = np.ascontiguousarray(np.asarray(y3_row, dtype=np.complex128)).view(np.float64)
+    L.nvo_push_900(ch, 0, iq.ctypes.data_as(C.POINTER(C.c_double)), iq.size // 2)
+    return _collect(L, ch, 1)
+
+
+def _collect(L, ch, n_ch) -> Result:
+    """the taps, events and messages of chain `ch`, which is freed"""
     r = Result()
     pd = C.POINTER(C.c_double)()
     r.y1 = _cplx(pd, L.nvo_y1(ch, C.byref(pd)))
