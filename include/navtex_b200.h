@@ -23,7 +23,8 @@
  * owns all device state; one caller thread per engine; return 0 on success, negative nvx_status
  * otherwise (nvx_last_error() gives a message).  Sample blocks are stream-major:
  * element (s, k) of a block of n samples per stream is at base[(s * n + k) * 2 + {0 = I, 1 = Q}].
- * n must be a multiple of NVX_BLOCK_ALIGN (280 = 4*7*10, one 900 Hz output).
+ * n must be a multiple of NVX_BLOCK_ALIGN (280 = 4*7*10, one 900 Hz output); on an engine fed at another rate
+ * (nvx_config.input_rate_hz) n counts input samples and must be a multiple of that rate's alignment.
  */
 #ifndef NAVTEX_B200_H
 #define NAVTEX_B200_H
@@ -80,6 +81,14 @@ typedef struct {
      * in registers -- five to eight in two passes.  Reference tap class only (up to 37 / 47 / 71 taps).  Results are laid out
      * [stream][channel] everywhere (y3, bits, events, messages). */
     int n_channels;
+    /* the radio's sample rate in S/s: 0 or NVX_FS_HZ (252000) = the engine's own rate, pushed as it is (no extra launch, no
+     * extra allocation).  Any other multiple of 100 in [96000, 3200000] is resampled on the device to 252 kS/s in front of
+     * the FIR path (nvx_resampler_info gives the filter); other rates return NVX_ERR_ARG.  On such an engine every count of
+     * samples is in input samples at this rate: max_block, the n of every push, nvx_stats.samples and every stream position
+     * (E in nvx_engine_reset_streams, the saved states' positions).  n and max_block must be multiples of the rate's
+     * alignment r / gcd(r, 900), the smallest input count that makes a whole number of 280-sample blocks at 252 kS/s, and
+     * the 158760-sample restart grid of nvx_engine_reset_streams is 0.63 r input samples. */
+    int input_rate_hz;
 } nvx_config;
 
 typedef struct {
@@ -94,6 +103,16 @@ typedef struct {
 typedef int (*nvx_message_cb)(void *user, int stream, char *bbbb, char *message, int freq);
 
 void nvx_default_config(nvx_config *cfg);
+
+/* host-only (no GPU): the rational resampler an engine with nvx_config.input_rate_hz = input_rate_hz runs.  252000 / r = up /
+ * down in lowest terms; output k at 252 kS/s (absolute, since create) is y[k] = sum_j h[p + j up] x[t - j], t = floor(k down /
+ * up), p = k down - t up, input samples before the first being 0 -- scipy.signal.upfirdn(h, x, up, down)[k].  h: a
+ * Kaiser-windowed sinc at up x r, pass band +-31.5 kHz (ripple <= 0.01 dB), stop band from min(r, 252000) - 31.5 kHz at
+ * least 80 dB down, each of its up polyphase branches summing to 1 within 1e-3; the kernel uses the float rounding of these
+ * FP64 taps and accumulates in FP32.  *block_align = r / gcd(r, 900), the multiple every push length and max_block must be.
+ * h may be NULL (or cap too small: NVX_ERR_OVERFLOW) to query *n_taps; any other output may be NULL.  252000 gives 1 / 1 / 280
+ * and one unit tap; an unsupported rate returns NVX_ERR_ARG. */
+int nvx_resampler_info(int input_rate_hz, int *up, int *down, long long *block_align, double *h, size_t cap, size_t *n_taps);
 const char *nvx_last_error(void);
 
 int nvx_engine_create(const nvx_config *cfg, nvx_engine **out);
@@ -206,15 +225,19 @@ typedef struct {
     long long cascade_launches;
     long long demod_launches;
     long long aux_launches;     /* tail carry, second pass of five to eight channels, long-tap stages, 8-bit -> int16 widening (long-tap path),
-                                 * per-stream resets */
-    long long samples;          /* IQ samples (all streams) pushed */
+                                 * per-stream resets, the resampler (engines with an input_rate_hz other than 252000; one launch per
+                                 * block, outside the cascade_ms spans) */
+    long long samples;          /* IQ samples (all streams) pushed, at the input rate */
     double demod_stage_ms[6];   /* split of demod_ms: angle/correlation, per-offset sums + arg max, history carry | symbol clock, bit decisions, SITOR-B state machine */
     long long long_tc_fallbacks;/* long-tap stage launches that were meant for the tensor-core kernel but ran on the CUDA-core one
                                  * (tap set outside its tile geometry, or a block the TMA unit cannot address); nvx_last_error() says why */
     long long messages;         /* messages completed (delivered to the callback or queued for poll) */
     double cascade_ms_min, cascade_ms_max;   /* fastest / slowest single launch of the fused-FIR kernel (or the long-path stage trio) */
+    double resample_ms;         /* sum of the resampler kernel's time (engines with an input_rate_hz other than 252000), CUDA events
+                                 * around its launch on the engine stream while timing is on; not part of cascade_ms */
 } nvx_stats;
-/* on: 0 = off, 1 = time the fused-FIR kernel only (two event records per block), 2 = also every demod stage */
+/* on: 0 = off, 1 = time the fused-FIR kernel (two event records per block) and the resampler (two more, where there is one),
+ * 2 = also every demod stage */
 int nvx_engine_enable_timing(nvx_engine *e, int on);
 int nvx_engine_get_stats(nvx_engine *e, nvx_stats *out, int reset);
 /* the per-launch times behind cascade_ms (milliseconds, in launch order, since the last get_stats(reset)); *count = how many
@@ -256,8 +279,10 @@ int nvx_capture_write(nvx_capture *c, int stream, const short *xi, const short *
  * over (len = 2 num_samples).  Writing int16 to an 8-bit capture or 8-bit pairs to an int16 capture returns NVX_ERR_ARG;
  * overflow as for nvx_capture_write */
 int nvx_capture_write_u8(nvx_capture *c, int stream, const unsigned char *iq, unsigned num_samples);
-/* consumer: push what every attached stream has in common (multiple of 280, <= max_block) as one block in the capture's format.
- * Returns samples per stream pushed, 0 if there was less than 280, or a negative nvx_status */
+/* consumer: push what every attached stream has in common (a multiple of the engine's alignment -- 280, or the input rate's,
+ * see nvx_resampler_info -- <= max_block) as one block in the capture's format.  Rings and max_block count input samples; create
+ * returns NVX_ERR_ARG unless max_block is a multiple of that alignment.
+ * Returns samples per stream pushed, 0 if there was less than one aligned block, or a negative nvx_status */
 long long nvx_capture_pump(nvx_capture *c);
 /* or let a poller thread pump every poll_ms (<= 0: 50 ms, capt_sched.c:489); stop() drains what is left */
 int nvx_capture_start(nvx_capture *c, int poll_ms);

@@ -6,7 +6,8 @@
 //                                                              interleaved into one ring of shorts under a mutex)
 //   consumer  main loop        receiver/capt_sched.c:484-528  (every 50 ms: drain the ring, sample_in_1 per I,Q pair)
 // Here every stream has its own ring of interleaved int16 I,Q; the consumer ("pump") takes what ALL attached streams have
-// in common, rounded down to a multiple of 280 samples, lays it out stream-major and pushes it as one int16 block (silence in
+// in common, rounded down to a multiple of the engine's alignment (280 samples, or the input rate's on an engine that
+// resamples: rings and blocks count input samples), lays it out stream-major and pushes it as one int16 block (silence in
 // the rows of detached streams, so that one radio that stops delivering does not stall the others).
 // nvx_capture_create_u8 makes the same front end for RTL-SDR radios: rings of interleaved 8-bit I,Q bytes (the buffer
 // rtlsdr_read_async hands its callback), pumped with nvx_engine_push_host_u8.
@@ -27,11 +28,16 @@
 
 #include "../../include/navtex_b200.h"
 
+namespace nvx {
+long long engine_block_align(const nvx_engine* e);      // engine.cu: push lengths are multiples of this
+}
+
 struct nvx_capture {
     nvx_engine* eng = nullptr;
     int S = 0;
     long long ring = 0;                    // samples per stream
     long long max_block = 0;
+    long long align = NVX_BLOCK_ALIGN;     // the engine's
     bool u8 = false;                       // 8-bit I,Q pairs (nvx_capture_create_u8), else int16
     size_t bps = 4;                        // bytes per I,Q pair in the rings and the staging buffers
     struct Ring {
@@ -65,7 +71,7 @@ long long pump_locked(nvx_capture* c) {
         if (avail < n) n = avail;
     }
     if (!any) return 0;
-    n -= n % NVX_BLOCK_ALIGN;
+    n -= n % c->align;
     if (n <= 0) return 0;
     const unsigned which = c->pumps++ & 1;
     uint8_t* const blk = c->block[which];
@@ -94,8 +100,10 @@ long long pump_locked(nvx_capture* c) {
     return n;
 }
 int create(nvx_engine* e, int n_streams, long long max_block, long long ring_samples, bool u8, nvx_capture** out) {
-    if (!e || !out || n_streams <= 0 || max_block <= 0 || max_block % NVX_BLOCK_ALIGN != 0 || ring_samples < 2 * max_block) return NVX_ERR_ARG;
+    if (!e || !out || n_streams <= 0 || max_block <= 0 || max_block % nvx::engine_block_align(e) != 0 || ring_samples < 2 * max_block)
+        return NVX_ERR_ARG;
     nvx_capture* c = new nvx_capture();
+    c->align = nvx::engine_block_align(e);
     c->eng = e;
     c->S = n_streams;
     c->ring = ring_samples;

@@ -25,6 +25,7 @@
 #include "fir_cascade.cuh"
 #include "fir_long.cuh"
 #include "message_assembler.h"
+#include "resample.cuh"
 
 namespace {
 
@@ -57,8 +58,9 @@ bool nco_entry(double f, nvx::NcoChan* out) {
 }
 
 // One stream's record of saved state (nvx_engine_save_streams), in 32-bit words: the FIR path's carried rows, then per channel
-// the y3 and correlation histories, ClockState, FsmState, epoch and, for general-NCO engines, the NcoChan row.  The offsets
-// inside a channel's part are fixed; the rest follows from the path's CarriedRows, the channel count and the NCO kind.
+// the y3 and correlation histories, ClockState, FsmState, epoch and, for general-NCO engines, the NcoChan row, then, on engines
+// fed at another input rate, the resampler's history.  The offsets inside a channel's part are fixed; the rest follows from the
+// path's CarriedRows, the channel count, the NCO kind and the resampler's history words (0 on engines fed at 252 kS/s).
 constexpr int kRecY3 = 0, kRecCorr = kRecY3 + 2 * nvx::kHistY, kRecClock = kRecCorr + 2 * nvx::kHistC;
 constexpr int kRecFsm = kRecClock + (int)sizeof(nvx::ClockState) / 4, kRecEpoch = kRecFsm + (int)sizeof(nvx::FsmState) / 4;
 constexpr int kRecNco = kRecEpoch + 2, kRecNcoWords = (int)sizeof(nvx::NcoChan) / 4;
@@ -67,15 +69,17 @@ struct StateLayout {
     long long rows[3];                  // offset of each carried region
     long long chan;                     // offset of channel 0's part
     long long ch_words;                 // words per channel
+    long long pre;                      // offset of the resampler's history
     long long words;                    // the whole record
 };
-StateLayout state_layout(const long long words[3], int C, bool gen_nco) {
+StateLayout state_layout(const long long words[3], int C, bool gen_nco, long long pre_words) {
     StateLayout l;
     long long at = 0;
     for (int k = 0; k < 3; ++k) { l.rows[k] = at; at += words[k]; }
     l.chan = (at + 1) & ~1LL;
     l.ch_words = kRecNco + (gen_nco ? kRecNcoWords : 0);
-    l.words = l.chan + C * l.ch_words;
+    l.pre = l.chan + C * l.ch_words;
+    l.words = l.pre + pre_words;
     return l;
 }
 
@@ -91,6 +95,7 @@ struct ResetArgs {
     int C;                              // channels per stream
     long long e0;                       // the new epoch, 900 Hz samples (a multiple of 567)
     nvx::CarriedRows rows;              // what the engine's FIR path carries into the next block
+    nvx::CarriedRows pre;               // what the resampler carries (region 0; nothing on engines fed at 252 kS/s)
     float2* y3_prev;                    // the previous block's y3 / corr buffers, whose ends become this block's histories
     long long y3_pitch;
     double* corr_prev;
@@ -114,6 +119,7 @@ __device__ void move_words(uint32_t* state, uint32_t* rec, long long n) {
 template <bool kSave>
 __device__ void move_stream(const ResetArgs& a, int s, uint32_t* rec) {
     for (int k = 0; k < 3; ++k) move_words<kSave>(a.rows.base[k] + (size_t)s * a.rows.words[k], rec + a.lay.rows[k], a.rows.words[k]);
+    move_words<kSave>(a.pre.base[0] + (size_t)s * a.pre.words[0], rec + a.lay.pre, a.pre.words[0]);
     for (int c = 0; c < a.C; ++c) {
         const size_t ch = (size_t)s * a.C + c;
         uint32_t* r = rec + a.lay.chan + c * a.lay.ch_words;
@@ -139,6 +145,7 @@ __global__ void reset_streams_kernel(const ResetArgs a) {
     const int t = threadIdx.x, nt = blockDim.x;
     for (int k = 0; k < 3; ++k)
         for (long long i = t; i < a.rows.words[k]; i += nt) a.rows.base[k][(size_t)s * a.rows.words[k] + i] = a.rows.fill[k];
+    for (long long i = t; i < a.pre.words[0]; i += nt) a.pre.base[0][(size_t)s * a.pre.words[0] + i] = a.pre.fill[0];
     for (int c = 0; c < a.C; ++c) {
         const size_t ch = (size_t)s * a.C + c;
         for (int i = t; i < nvx::kHistY; i += nt) a.y3_prev[ch * a.y3_pitch + a.n_prev + i] = make_float2(0.f, 0.f);
@@ -193,6 +200,11 @@ struct nvx_engine {
     // (fir_long.cuh)
     nvx::CascadePath* cp = nullptr;
     nvx::LongPath* lp = nullptr;
+    // in front of it, on engines fed at another rate than 252 kS/s (nvx_config.input_rate_hz), the resampler; null otherwise
+    nvx::ResamplePath* rp = nullptr;
+    int rate = 0;                         // that input rate, 0 = 252 kS/s
+    int up = 1, down = 1;                 // 252000 / rate = up / down
+    long long align = nvx::kSuper;        // push lengths and max_block are multiples of this many input samples
     int path = 0;                         // what saved state records: 0 / 1 = the fused path's tap class, 2 = the long-tap path
     std::vector<int> stream_tag;          // optional [S][C] message tags (read by the worker; changed through markers)
     // per-stream resets, retunes and loads asked for since the last push; the next push applies them
@@ -268,6 +280,7 @@ int free_engine(nvx_engine* e) {
     if (e->reset_copied) cudaEventDestroy(e->reset_copied);
     nvx::cascade_path_free(e->cp);
     nvx::long_path_free(e->lp);
+    nvx::resample_path_free(e->rp);
     for (int k = 0; k < kBuf; ++k) {
         cudaFree(e->y3buf[k]); cudaFree(e->d_events[k]); cudaFree(e->d_ev_count[k]);
         cudaFreeHost(e->h_events[k]); cudaFreeHost(e->h_ev_count[k]);
@@ -301,6 +314,7 @@ int reset_state(nvx_engine* e) {
         CU_TRY(cudaMemcpyAsync(e->d_nco_ch, e->nco_host.data(), e->nco_host.size() * sizeof(nvx::NcoChan), cudaMemcpyHostToDevice, e->stream));
     if (e->lp) CU_TRY(nvx::long_path_reset(e->lp, e->stream));
     else nvx::cascade_path_reset(e->cp);
+    if (e->rp) CU_TRY(nvx::resample_path_reset(e->rp, e->stream));
     for (int k = 0; k < kBuf; ++k) {
         e->db.y3 = e->y3buf[k];
         e->db.picks = e->pickbuf[k];
@@ -323,6 +337,8 @@ int reset_state(nvx_engine* e) {
     return 0;
 }
 
+constexpr int kSpanResample = 8;          // span kinds: 0 cascade, 1 demod chain, 2 .. 7 demod stages, 8 resampler
+
 cudaEvent_t next_event(nvx_engine* e) {
     if (e->ev_used == e->ev_pool.size()) {
         cudaEvent_t ev;
@@ -344,6 +360,7 @@ void collect_spans(nvx_engine* e) {
             if (ms > e->stats.cascade_ms_max) e->stats.cascade_ms_max = ms;
         }
         else if (sp.kind == 1) e->stats.demod_ms += ms;
+        else if (sp.kind == kSpanResample) e->stats.resample_ms += ms;
         else e->stats.demod_stage_ms[sp.kind - 2] += ms;
     }
     e->spans.clear();
@@ -477,7 +494,8 @@ ResetArgs state_args(nvx_engine* e) {
     ResetArgs a = {};
     a.C = e->C;
     a.rows = e->lp ? long_path_carried(e->lp) : cascade_path_carried(e->cp);
-    a.lay = state_layout(a.rows.words, e->C, e->d_nco_ch != nullptr);
+    if (e->rp) a.pre = resample_path_carried(e->rp);
+    a.lay = state_layout(a.rows.words, e->C, e->d_nco_ch != nullptr, a.pre.words[0]);
     a.y3_prev = e->y3buf[(e->blocks + kBuf - 1) % kBuf];
     a.y3_pitch = kHistY + e->P_max;
     a.corr_prev = e->corrbuf[(e->blocks & 1) ^ 1];
@@ -570,7 +588,7 @@ int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fm
     using namespace nvx;
     if (e->fmt >= 0 && e->fmt != (int)fmt)
         return fail(NVX_ERR_ARG, "sample format changed between pushes (float, int16 and 8-bit blocks cannot be mixed without a reset)");
-    if (n <= 0 || n % kSuper != 0) return fail(NVX_ERR_ARG, "block length %lld is not a positive multiple of %d", n, kSuper);
+    if (n <= 0 || n % e->align != 0) return fail(NVX_ERR_ARG, "block length %lld is not a positive multiple of %lld", n, e->align);
     if (n > e->cfg.max_block) return fail(NVX_ERR_ARG, "block length %lld exceeds max_block %lld", n, e->cfg.max_block);
     if (((uintptr_t)d_x & 15) != 0) return fail(NVX_ERR_ARG, "device block is not 16-byte aligned");
     e->fmt = (int)fmt;                              // only a block that is accepted fixes the format
@@ -582,7 +600,24 @@ int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fm
         CU_TRY(cudaStreamSynchronize(e->stream_demod));
         collect_spans(e);
     }
-    const int n_super = (int)(n / kSuper);
+    // the FIR path runs at 252 kS/s: on the resampler's float output when the engine is fed at another rate
+    const void* x = d_x;
+    long long n_fir = n;
+    SampleFmt fir_fmt = fmt;
+    if (e->rp) {
+        PathReport rrep;
+        const float2* y = nullptr;
+        if (e->timing) {
+            e->spans.push_back({(int)e->ev_used, (int)e->ev_used + 1, kSpanResample});
+            CU_TRY(cudaEventRecord(next_event(e), e->stream));
+        }
+        const int rc = resample_path_run(e->rp, d_x, n, fmt, e->stream, &y, &n_fir, &rrep);
+        if (path_report(e, rc, rrep)) return rc;
+        if (e->timing) CU_TRY(cudaEventRecord(next_event(e), e->stream));
+        x = y;
+        fir_fmt = SampleFmt::F32;
+    }
+    const int n_super = (int)(n_fir / kSuper);
 
     cudaEvent_t t0 = nullptr, t1 = nullptr, marks[8] = {};
     if (e->timing) {
@@ -599,8 +634,8 @@ int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fm
     }
     PathReport rep;
     const long long y3_pitch = kHistY + e->P_max;
-    const int rc = e->lp ? long_path_run(e->lp, d_x, n, fmt, e->sb_abs, e->y3buf[b], y3_pitch, kHistY, e->stream, t1, &rep)
-                         : cascade_path_run(e->cp, d_x, n, fmt, e->sb_abs, e->y3buf[b], y3_pitch, kHistY, e->stream, t1, &rep);
+    const int rc = e->lp ? long_path_run(e->lp, x, n_fir, fir_fmt, e->sb_abs, e->y3buf[b], y3_pitch, kHistY, e->stream, t1, &rep)
+                         : cascade_path_run(e->cp, x, n_fir, fir_fmt, e->sb_abs, e->y3buf[b], y3_pitch, kHistY, e->stream, t1, &rep);
     if (path_report(e, rc, rep)) return rc;
 
     // demod of this block runs on its own stream, overlapping the next block's cascade
@@ -645,7 +680,7 @@ int process_block(nvx_engine* e, const void* d_x, long long n, nvx::SampleFmt fm
 
 // H2D on the copy stream into staging slot k % 2, then the block's kernels on the main stream
 int push_host(nvx_engine* e, const void* iq, long long n, nvx::SampleFmt fmt) {
-    if (n <= 0 || n % nvx::kSuper != 0 || n > e->cfg.max_block) return fail(NVX_ERR_ARG, "bad block length %lld", n);
+    if (n <= 0 || n % e->align != 0 || n > e->cfg.max_block) return fail(NVX_ERR_ARG, "bad block length %lld (a positive multiple of %lld up to max_block)", n, e->align);
     CU_TRY(cudaSetDevice(e->cfg.device));
     const size_t bytes = (size_t)e->S * (size_t)n * nvx::sample_bytes(fmt);
     const int slot = (int)(e->host_pushes % 2);
@@ -680,7 +715,8 @@ struct StateHeader {
     long long words[3];                 // the FIR path's CarriedRows words
     uint64_t taps;                      // the path's tap hash
     long long rec_words;                // words per device record
-    int32_t count, n_channels, fmt, path, gen_nco, reserved;
+    int32_t count, n_channels, fmt, path, gen_nco;
+    int32_t rate;                       // input rate of an engine that resamples (nvx_config.input_rate_hz), 0 = 252 kS/s
 };
 static_assert(sizeof(StateHeader) == 96, "state header layout");
 constexpr size_t kChecksumAt = offsetof(StateHeader, checksum);
@@ -688,6 +724,19 @@ using ChannelText = nvx::MessageAssembler::Channel;
 
 uint64_t state_checksum(const uint8_t* p, size_t n) {
     return nvx::hash_bytes(p + kChecksumAt + 8, n - kChecksumAt - 8, nvx::hash_bytes(p, kChecksumAt));
+}
+
+// input samples per stream pushed so far, and the restart grid, in input samples (158760 x down / up)
+long long in_position(const nvx_engine* e) { return e->sb_abs * nvx::kSuper / e->up * e->down; }
+long long in_grid(const nvx_engine* e) { return kStateGrid / e->up * e->down; }
+
+// words of the resampler's history per stream at that input rate (0 = 252 kS/s); -1 for a rate no engine takes
+long long resampler_words(int rate) {
+    if (rate == 0) return 0;
+    nvx::ResampleDesign d;
+    const char* why = "";
+    if (rate == NVX_FS_HZ || !nvx::resample_geometry(rate, &d, &why)) return -1;
+    return 2LL * (d.J - 1);
 }
 
 const char* path_name(int path) { return path == 0 ? "fused path (reference tap class)" : path == 1 ? "fused path (medium tap class)" : "long-tap path"; }
@@ -701,9 +750,14 @@ int parse_state(const void* state, size_t size, StateHeader* h, std::vector<std:
     if (h->version != kStateVersion) return fail(NVX_ERR_ARG, "saved stream state: version %u, this library reads version %u", h->version, kStateVersion);
     if (h->bytes != size) return fail(NVX_ERR_ARG, "saved stream state: %zu bytes given, the state has %llu (truncated?)", size, (unsigned long long)h->bytes);
     if (state_checksum(p, size) != h->checksum) return fail(NVX_ERR_ARG, "saved stream state: checksum mismatch (the bytes were altered)");
-    const long long rec_words = state_layout(h->words, h->n_channels, h->gen_nco != 0).words;
+    const long long pre_words = resampler_words(h->rate);
+    if (pre_words < 0) return fail(NVX_ERR_ARG, "saved stream state: inconsistent header");
+    nvx::ResampleDesign rd;
+    const char* why = "";
+    nvx::resample_geometry(h->rate ? h->rate : NVX_FS_HZ, &rd, &why);
+    const long long rec_words = state_layout(h->words, h->n_channels, h->gen_nco != 0, pre_words).words;
     if (h->count < 0 || h->n_channels < 1 || h->n_channels > nvx::kMaxChannels || h->fmt < 0 || h->fmt >= nvx::kSampleFmts || h->path < 0 ||
-        h->path > 2 || (h->gen_nco != 0 && h->gen_nco != 1) || h->position < 0 || h->position % nvx::kSuper || h->words[0] < 0 ||
+        h->path > 2 || (h->gen_nco != 0 && h->gen_nco != 1) || h->position < 0 || h->position % rd.align || h->words[0] < 0 ||
         h->words[1] < 0 || h->words[2] < 0 || h->rec_words != rec_words)
         return fail(NVX_ERR_ARG, "saved stream state: inconsistent header");
     size_t at = sizeof(StateHeader);
@@ -743,6 +797,10 @@ int check_stream_list(const nvx_engine* e, const int* streams, int count) {
 
 }  // namespace
 
+namespace nvx {
+long long engine_block_align(const nvx_engine* e) { return e->align; }
+}  // namespace nvx
+
 extern "C" {
 
 const char* nvx_last_error(void) { return g_err; }
@@ -755,14 +813,35 @@ void nvx_default_config(nvx_config* cfg) {
     cfg->freq_tag[1] = 490;
 }
 
+int nvx_resampler_info(int input_rate_hz, int* up, int* down, long long* block_align, double* h, size_t cap, size_t* n_taps) {
+    nvx::ResampleDesign d;
+    const char* why = "";
+    if (!(h ? nvx::resample_design(input_rate_hz, &d, &why) : nvx::resample_geometry(input_rate_hz, &d, &why)))
+        return fail(NVX_ERR_ARG, "input rate %d: %s", input_rate_hz, why);
+    if (up) *up = d.L;
+    if (down) *down = d.M;
+    if (block_align) *block_align = d.align;
+    if (n_taps) *n_taps = (size_t)d.L * d.J;
+    if (!h) return 0;
+    if (cap < d.h.size()) return fail(NVX_ERR_OVERFLOW, "the resampler has %zu taps, the buffer holds %zu", d.h.size(), cap);
+    memcpy(h, d.h.data(), d.h.size() * sizeof(double));
+    return 0;
+}
+
 int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
     if (!cfg || !out) return fail(NVX_ERR_ARG, "null argument");
-    if (cfg->n_streams <= 0 || cfg->max_block <= 0 || cfg->max_block % nvx::kSuper != 0)
-        return fail(NVX_ERR_ARG, "n_streams must be > 0 and max_block a positive multiple of %d", nvx::kSuper);
+    // input rate: 252 kS/s as it is, or resampled on the device; every count of samples below is in input samples
+    nvx::ResampleDesign rd;
+    const char* why = "";
+    if (cfg->input_rate_hz != 0 && !nvx::resample_geometry(cfg->input_rate_hz, &rd, &why))
+        return fail(NVX_ERR_ARG, "input_rate_hz %d: %s", cfg->input_rate_hz, why);
+    if (cfg->n_streams <= 0 || cfg->max_block <= 0 || cfg->max_block % rd.align != 0)
+        return fail(NVX_ERR_ARG, "n_streams must be > 0 and max_block a positive multiple of %lld", rd.align);
+    const long long max_fir = cfg->max_block / rd.M * rd.L;       // the largest block at 252 kS/s
     if (cfg->n_streams > 32767)       // channel rows index the y dimension of the demod grids (65535 max)
         return fail(NVX_ERR_ARG, "n_streams %d exceeds 32767 per engine: shard the streams over more engines", cfg->n_streams);
-    if (cfg->max_block / nvx::kSuper > (1 << 24))
-        return fail(NVX_ERR_ARG, "max_block %lld is too long (at most %d samples per push)", cfg->max_block, nvx::kSuper << 24);
+    if (max_fir / nvx::kSuper > (1 << 24))
+        return fail(NVX_ERR_ARG, "max_block %lld is too long (at most %d samples per push at 252 kS/s)", cfg->max_block, nvx::kSuper << 24);
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || cfg->device < 0 || cfg->device >= ndev)
         return fail(NVX_ERR_CUDA, "no usable CUDA device %d (%d visible): this library has no CPU path", cfg->device, ndev);
@@ -778,6 +857,8 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
     if (C != 2 && !cfg->nco_hz) { delete e; return fail(NVX_ERR_ARG, "n_channels = %d needs nco_hz (only the reference's two channels have default offsets)", C); }
     if ((long long)C * cfg->n_streams > 65535) { delete e; return fail(NVX_ERR_ARG, "n_streams x n_channels = %lld exceeds 65535 channel rows per engine", (long long)C * cfg->n_streams); }
     e->C = C;
+    e->rate = rd.L != rd.M ? cfg->input_rate_hz : 0;
+    e->up = rd.L; e->down = rd.M; e->align = rd.align;
     if (cfg->stream_freq_tag) e->stream_tag.assign(cfg->stream_freq_tag, cfg->stream_freq_tag + (size_t)C * (size_t)cfg->n_streams);
     if (cfg->nco_hz) {
         e->nco_host.resize((size_t)cfg->n_streams * C);
@@ -791,7 +872,7 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
     e->channels = C * e->S;
     e->pend_flags.assign((size_t)e->S, 0);
     e->pend_rec.assign((size_t)e->S, -1);
-    e->P_max = (int)(cfg->max_block / nvx::kSuper);
+    e->P_max = (int)(max_fir / nvx::kSuper);
     // tap counts: reference lengths unless given; sets up to 37/47/71 and up to 61/75/111 run through the fused kernel
     // (zero-padded to the class), longer ones through the long-tap path
     const int n[3] = {cfg->n1 ? cfg->n1 : NVX_T1, cfg->n2 ? cfg->n2 : NVX_T2, cfg->n3 ? cfg->n3 : NVX_T3};
@@ -868,7 +949,12 @@ int nvx_engine_create(const nvx_config* cfg, nvx_engine** out) {
         nvx::PathReport rep;
         const int rc = tap_class >= 0
                            ? nvx::cascade_path_create(e->S, C, n, h, e->d_nco_ch, cfg->device, nvx::demod_reserved_sms(e->channels), &e->cp, &rep)
-                           : nvx::long_path_create(e->S, cfg->max_block, n, h, e->d_nco_ch, e->stream, &e->lp, &rep);
+                           : nvx::long_path_create(e->S, max_fir, n, h, e->d_nco_ch, e->stream, &e->lp, &rep);
+        if (path_report(e, rc, rep)) { free_engine(e); return rc; }
+    }
+    if (e->rate) {
+        nvx::PathReport rep;
+        const int rc = nvx::resample_path_create(e->rate, e->S, cfg->max_block, &e->rp, &rep);
         if (path_report(e, rc, rep)) { free_engine(e); return rc; }
     }
     e->assembler.resize(e->channels);
@@ -957,9 +1043,11 @@ int nvx_engine_save_streams(nvx_engine* e, const int* streams, int count, void* 
     h.magic = kStateMagic;
     h.version = kStateVersion;
     h.bytes = *size;
-    h.position = e->sb_abs * nvx::kSuper;
+    h.position = in_position(e);
     for (int k = 0; k < 3; ++k) h.words[k] = a.rows.words[k];
     h.taps = e->lp ? nvx::long_path_taps_hash(e->lp) : nvx::cascade_path_taps_hash(e->cp);
+    if (e->rp) h.taps = nvx::hash_bytes(&h.taps, sizeof h.taps, nvx::resample_path_taps_hash(e->rp));
+    h.rate = e->rate;
     h.rec_words = a.lay.words;
     h.count = count;
     h.n_channels = e->C;
@@ -983,8 +1071,13 @@ int nvx_engine_load_streams(nvx_engine* e, const int* streams, int count, const 
     if (h.count != count) return fail(NVX_ERR_ARG, "the saved state holds %d streams, %d were listed", h.count, count);
     if (int rc = check_stream_list(e, streams, count)) return rc;
     const bool gen = e->d_nco_ch != nullptr;
+    if (h.rate != e->rate)
+        return fail(NVX_ERR_ARG, "the state was saved on an engine fed at %d S/s, this engine is fed at %d S/s", h.rate ? h.rate : NVX_FS_HZ,
+                    e->rate ? e->rate : NVX_FS_HZ);
     if (h.path != e->path) return fail(NVX_ERR_ARG, "the state was saved on the %s, this engine runs the %s", path_name(h.path), path_name(e->path));
-    if (h.taps != (e->lp ? long_path_taps_hash(e->lp) : cascade_path_taps_hash(e->cp))) return fail(NVX_ERR_ARG, "the state was saved with another tap set");
+    uint64_t taps = e->lp ? long_path_taps_hash(e->lp) : cascade_path_taps_hash(e->cp);
+    if (e->rp) taps = hash_bytes(&taps, sizeof taps, resample_path_taps_hash(e->rp));
+    if (h.taps != taps) return fail(NVX_ERR_ARG, "the state was saved with another tap set");
     if (h.n_channels != e->C) return fail(NVX_ERR_ARG, "the state has %d channels per stream, this engine %d", h.n_channels, e->C);
     if ((h.gen_nco != 0) != gen)
         return fail(NVX_ERR_ARG, "the state was saved %s, this engine runs %s", h.gen_nco ? "with per-stream NCO offsets" : "on the reference NCO table",
@@ -992,14 +1085,14 @@ int nvx_engine_load_streams(nvx_engine* e, const int* streams, int count, const 
     if (e->fmt >= 0 && e->fmt != h.fmt) return fail(NVX_ERR_ARG, "the state holds sample format %d, this engine takes format %d", h.fmt, e->fmt);
     // an engine that has pushed nothing since create or reset adopts the saved position; any other must be on the same grid
     const bool adopt = e->blocks == 0 && !e->adopted;
-    const long long here = adopt ? h.position : e->sb_abs * kSuper;
-    if ((here - h.position) % kStateGrid)
-        return fail(NVX_ERR_ARG, "the state was saved after input sample %lld, this engine is at %lld: the two must agree modulo %lld (567 x 280)",
-                    (long long)h.position, here, kStateGrid);
+    const long long here = adopt ? h.position : in_position(e);
+    if ((here - h.position) % in_grid(e))
+        return fail(NVX_ERR_ARG, "the state was saved after input sample %lld, this engine is at %lld: the two must agree modulo %lld (567 x 280 at 252 kS/s)",
+                    (long long)h.position, here, in_grid(e));
     CU_TRY(cudaSetDevice(e->cfg.device));
     if (e->cp) {      // a fresh engine's tails take the saved format now (it would fill them with its silence at the first push)
         PathReport rep;
-        const int rc = cascade_path_prepare(e->cp, (SampleFmt)h.fmt, e->stream, &rep);
+        const int rc = cascade_path_prepare(e->cp, e->rp ? SampleFmt::F32 : (SampleFmt)h.fmt, e->stream, &rep);
         if (path_report(e, rc, rep)) return rc;
     }
     const CarriedRows rows = e->lp ? long_path_carried(e->lp) : cascade_path_carried(e->cp);
@@ -1009,14 +1102,15 @@ int nvx_engine_load_streams(nvx_engine* e, const int* streams, int count, const 
 
     // accepted: nothing below fails
     if (adopt) {      // its other streams start as streams reset at the saved position
-        e->sb_abs = h.position / kSuper;
+        e->sb_abs = h.position / e->down * e->up / kSuper;
         e->adopted = true;
         for (int s = 0; s < e->S; ++s) nvx_engine_reset_streams(e, &s, 1);
     }
     e->fmt = h.fmt;
-    const StateLayout lay = state_layout(h.words, e->C, gen);
-    const long long d_sb = (here - h.position) / kSuper;                        // epochs: 900 Hz samples
-    const long long d_tick = ((here - h.position) / NVX_D1) % kNcoDen;         // NCO phases: 63 kHz ticks
+    const StateLayout lay = state_layout(h.words, e->C, gen, resampler_words(h.rate));
+    const long long d_out = (here - h.position) / e->down * e->up;             // the same distance at 252 kS/s
+    const long long d_sb = d_out / kSuper;                                      // epochs: 900 Hz samples
+    const long long d_tick = (d_out / NVX_D1) % kNcoDen;                        // NCO phases: 63 kHz ticks
     const uint32_t* recs = reinterpret_cast<const uint32_t*>(static_cast<const uint8_t*>(state) + sizeof(StateHeader));
     for (int k = 0; k < count; ++k) {
         const int s = streams[k];

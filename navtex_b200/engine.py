@@ -26,7 +26,7 @@ class Config(C.Structure):
         ("h1", C.POINTER(C.c_double)), ("h2", C.POINTER(C.c_double)), ("h3", C.POINTER(C.c_double)),
         ("keep_bits", C.c_int), ("first_stream_id", C.c_int),
         ("nco_hz", C.POINTER(C.c_double)), ("stream_freq_tag", C.POINTER(C.c_int)),
-        ("n1", C.c_int), ("n2", C.c_int), ("n3", C.c_int), ("n_channels", C.c_int),
+        ("n1", C.c_int), ("n2", C.c_int), ("n3", C.c_int), ("n_channels", C.c_int), ("input_rate_hz", C.c_int),
     ]
 
 
@@ -38,7 +38,7 @@ class Stats(C.Structure):
     _fields_ = [("cascade_ms", C.c_double), ("demod_ms", C.c_double), ("cascade_launches", C.c_longlong),
                 ("demod_launches", C.c_longlong), ("aux_launches", C.c_longlong), ("samples", C.c_longlong),
                 ("demod_stage_ms", C.c_double * 6), ("long_tc_fallbacks", C.c_longlong), ("messages", C.c_longlong),
-                ("cascade_ms_min", C.c_double), ("cascade_ms_max", C.c_double)]
+                ("cascade_ms_min", C.c_double), ("cascade_ms_max", C.c_double), ("resample_ms", C.c_double)]
 
 
 class SynthDesc(C.Structure):
@@ -48,7 +48,7 @@ class SynthDesc(C.Structure):
 
 
 EXPORTS = (
-    "nvx_default_config", "nvx_last_error", "nvx_engine_create", "nvx_engine_destroy", "nvx_engine_reset",
+    "nvx_default_config", "nvx_last_error", "nvx_resampler_info", "nvx_engine_create", "nvx_engine_destroy", "nvx_engine_reset",
     "nvx_engine_reset_streams", "nvx_engine_retune_stream", "nvx_engine_save_streams", "nvx_engine_load_streams",
     "nvx_stream_state_info",
     "nvx_engine_push_host_f32", "nvx_engine_push_host_s16", "nvx_engine_push_host_u8", "nvx_engine_push_device_f32",
@@ -77,6 +77,8 @@ def load_library():
     L = C.CDLL(LIB_PATH)
     L.nvx_last_error.restype = C.c_char_p
     L.nvx_default_config.argtypes = [C.POINTER(Config)]
+    L.nvx_resampler_info.argtypes = [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_longlong), C.POINTER(C.c_double),
+                                     C.c_size_t, C.POINTER(C.c_size_t)]
     L.nvx_engine_create.argtypes = [C.POINTER(Config), C.POINTER(C.c_void_p)]
     L.nvx_engine_destroy.argtypes = [C.c_void_p]
     L.nvx_engine_destroy.restype = None
@@ -170,6 +172,18 @@ def long_tc_band(decimation: int, h):
     return g, hi.reshape(shape), lo.reshape(shape)
 
 
+def resampler_info(rate: int) -> dict:
+    """The resampler of an engine fed at `rate` S/s (host only, no GPU; nvx_resampler_info): {"up": L, "down": M, "align": input
+    samples every push length must be a multiple of, "taps": float64 prototype h}, with output k = upfirdn(h, x, L, M)[k].
+    Raises NvxError for a rate no engine takes."""
+    L = load_library()
+    up, down, align, n = C.c_int(), C.c_int(), C.c_longlong(), C.c_size_t()
+    _check(L.nvx_resampler_info(rate, C.byref(up), C.byref(down), C.byref(align), None, 0, C.byref(n)))
+    h = np.zeros(n.value, dtype=np.float64)
+    _check(L.nvx_resampler_info(rate, None, None, None, h.ctypes.data_as(C.POINTER(C.c_double)), h.size, C.byref(n)))
+    return {"up": up.value, "down": down.value, "align": align.value, "taps": h}
+
+
 def stream_state_info(state: bytes) -> dict:
     """Validate a saved stream state (host only, no GPU) and return its record count, input position (samples per stream),
     channels per stream and sample format ("f32", "s16" or "u8"); raises NvxError on a corrupt or truncated state."""
@@ -189,7 +203,9 @@ class Engine:
     """One GPU, S streams.  Mirrors the reference's init / per-sample push / add_message flow, batched."""
 
     def __init__(self, n_streams: int, max_block: int, device: int = 0, keep_bits: bool = False, taps=None,
-                 first_stream_id: int = 0, nco_hz=None, stream_freq_tag=None, n_channels: int = 2):
+                 first_stream_id: int = 0, nco_hz=None, stream_freq_tag=None, n_channels: int = 2, input_rate_hz: int = 0):
+        """input_rate_hz: the radio's rate (0 = 252 kS/s); any other accepted rate is resampled on the device, and max_block and
+        every push length then count input samples and are multiples of resampler_info(input_rate_hz)["align"]."""
         L = load_library()
         cfg = Config()
         L.nvx_default_config(C.byref(cfg))
@@ -202,6 +218,7 @@ class Engine:
             # up to 37/47/71 and up to 61/75/111 taps: fused kernel (zero-padded); longer: the long-tap path
             cfg.n1, cfg.n2, cfg.n3 = (len(t) for t in self._taps)
         cfg.n_channels = n_channels
+        cfg.input_rate_hz = input_rate_hz
         if nco_hz is not None:           # [S, n_channels] per-stream channel offsets in Hz
             self._nco = np.ascontiguousarray(nco_hz, dtype=np.float64).reshape(n_streams, n_channels)
             cfg.nco_hz = self._nco.ctypes.data_as(C.POINTER(C.c_double))
@@ -213,6 +230,8 @@ class Engine:
         self.L, self.S, self.max_block, self.device = L, n_streams, max_block, device
         self.C = n_channels
         self.last_n = 0
+        info = resampler_info(input_rate_hz or FS)
+        self.up, self.down, self.align = info["up"], info["down"], info["align"]
 
     def close(self):
         h = getattr(self, "_h", None)
@@ -221,6 +240,15 @@ class Engine:
             h.value = None
 
     __del__ = close
+
+    def resampler_info(self, rate: int) -> dict:
+        """resampler_info(rate): the filter, L / M and alignment of an engine fed at that rate."""
+        return resampler_info(rate)
+
+    @property
+    def last_n_fir(self) -> int:
+        """the last block's length at 252 kS/s (last_n counts input samples)"""
+        return self.last_n // self.down * self.up
 
     def reset(self):
         _check(self.L.nvx_engine_reset(self._h))
@@ -298,7 +326,7 @@ class Engine:
 
     def read_y3(self) -> np.ndarray:
         """[S, n_channels, P] complex64 of the last block."""
-        P = self.last_n // BLOCK_ALIGN
+        P = self.last_n_fir // BLOCK_ALIGN
         out = np.empty((self.S, self.C, P, 2), dtype=np.float32)
         got = C.c_size_t()
         _check(self.L.nvx_engine_read_y3(self._h, out.ctypes.data_as(C.c_void_p), out.size, C.byref(got)))
@@ -306,7 +334,7 @@ class Engine:
         return out.view(np.complex64)[..., 0]
 
     def read_bits(self, stream: int, ch: int):
-        cap = self.last_n // BLOCK_ALIGN // 8 + 4
+        cap = self.last_n_fir // BLOCK_ALIGN // 8 + 4
         bits = np.empty(cap, dtype=np.uint8)
         sums = np.empty((cap, 4), dtype=np.float32)
         got = C.c_size_t()
@@ -314,7 +342,7 @@ class Engine:
         return bits[: got.value].tobytes(), sums[: got.value].copy()
 
     def read_events(self, stream: int, ch: int) -> bytes:
-        cap = self.last_n // BLOCK_ALIGN // 30 + 64
+        cap = self.last_n_fir // BLOCK_ALIGN // 30 + 64
         ev = np.empty(cap, dtype=np.uint8)
         got = C.c_size_t()
         _check(self.L.nvx_engine_read_events(self._h, stream, ch, ev.ctypes.data_as(C.c_void_p), cap, C.byref(got)))
@@ -415,7 +443,8 @@ class Store:
 
 class Capture:
     """Radio front end: per-stream rings fed by radio callbacks, pumped into the engine in blocks.  fmt="s16": SDRplay-format
-    int16 rings (write); fmt="u8": RTL-SDR 8-bit rings (write_u8)."""
+    int16 rings (write); fmt="u8": RTL-SDR 8-bit rings (write_u8).  Rings and max_block count input samples at the engine's
+    input rate; max_block and every pumped block are multiples of the engine's alignment (eng.align)."""
 
     def __init__(self, eng: "Engine", max_block: int, ring_samples: int, fmt: str = "s16"):
         self.L, self.eng = eng.L, eng

@@ -102,32 +102,35 @@ def fsk_iq(
     seed: int = 0,
     fading_hz: float = 0.0,
     idle_carrier: bool = False,
+    rate: int = FS,
 ) -> np.ndarray:
-    """Complex baseband capture (complex128, not yet quantised) of the given emissions.
+    """Complex baseband capture (complex128, not yet quantised) of the given emissions, sampled at `rate` S/s (a multiple of
+    100, so that a bit is a whole number of samples; the engine's own 252 kS/s by default, others for engines that resample).
 
-    snr_db is the signal-to-noise ratio over the full 252 kHz band relative to the
+    snr_db is the signal-to-noise ratio over the full sampled band relative to the
     first emission's amplitude (SURVEY.md 8d: the reference decodes at -20 dB).
     fading_hz > 0 applies a slow Rayleigh-like amplitude (two-pole filtered complex
     Gaussian, unit mean power) to every emission.
     """
-    n = int(round(duration_s * FS))
+    n = int(round(duration_s * rate))
+    spb = rate // BAUD
     rng = np.random.default_rng(seed)
     x = np.zeros(n, dtype=np.complex128)
     for em in emissions:
         bits = message_bits(em.text, em.n_phasing, em.n_tail)
-        start = int(round(em.start_s * FS))
-        span = min(len(bits) * SAMPLES_PER_BIT, max(0, n - start))
+        start = int(round(em.start_s * rate))
+        span = min(len(bits) * spb, max(0, n - start))
         if em.stop_s is not None:
-            span = min(span, int(round(em.stop_s * FS)))
+            span = min(span, int(round(em.stop_s * rate)))
         if span <= 0:
             continue
         tone = np.where(bits == 1, -FSK_SHIFT_HZ, FSK_SHIFT_HZ)       # Y = -85 Hz, B = +85 Hz
-        freq = np.repeat(tone, SAMPLES_PER_BIT)[:span] + em.offset_hz
-        phase = 2.0 * np.pi * np.cumsum(freq) / FS
+        freq = np.repeat(tone, spb)[:span] + em.offset_hz
+        phase = 2.0 * np.pi * np.cumsum(freq) / rate
         sig = em.amplitude * np.exp(1j * phase)
         if fading_hz > 0.0:
             g = rng.standard_normal(span) + 1j * rng.standard_normal(span)
-            a = np.exp(-2.0 * np.pi * fading_hz / FS)
+            a = np.exp(-2.0 * np.pi * fading_hz / rate)
             env = np.empty(span, dtype=np.complex128)
             acc = 0.0 + 0.0j
             # one-pole IIR in blocks (vectorised via cumulative scaling is unstable for long spans)
@@ -142,7 +145,7 @@ def fsk_iq(
             sig = sig * env
         x[start:start + span] += sig
         if idle_carrier and start > 0:
-            x[:start] += em.amplitude * np.exp(2j * np.pi * (em.offset_hz + FSK_SHIFT_HZ) * np.arange(start) / FS)
+            x[:start] += em.amplitude * np.exp(2j * np.pi * (em.offset_hz + FSK_SHIFT_HZ) * np.arange(start) / rate)
     if snr_db is not None and emissions:
         sigma = emissions[0].amplitude / np.sqrt(2.0) * 10.0 ** (-snr_db / 20.0)
         x += sigma * (rng.standard_normal(n) + 1j * rng.standard_normal(n))
